@@ -3,6 +3,7 @@
 through the reference-facing C ABI (tp_prove_dev / tp_prove_inputs).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--log-n L] [--impl reference] [--no-sweep] [--no-north-star]
+                    [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  A "step" is one complete proof (13 G1 MSMs, 5 iNTT + 20 coset NTT + 4 inverse coset
 NTT, grand product, quotient, 6 openings).  `value` = prove ms with the witness resident in HBM; `e2e` = the same
@@ -22,6 +23,11 @@ of the oracle's C++ port on all host threads, no extrapolation.
 
 `--impl reference` times the CPU oracle port (oracle/c, all host threads) on the SAME 2^20 workload: full proves, as
 many of the K requested as fit in ~150 s (at least one); `steps` in its line is the number actually timed.
+
+`--dump-outputs DIR` (rank 0) writes what the last timed step returned to its caller, for the GPU prover and for
+`--impl reference` alike, so that two builds, or the GPU and the CPU port, can be compared output for output on the same
+seeded inputs: DIR/proof.npy, the 1472-byte proof block (TP_PROOF_FIXED_BYTES: 13 G1
+points of 96 B and 7 Fr of 32 B) as float64 values 0..255, so that any changed byte differs by at least 1.
 """
 import argparse
 import json
@@ -156,6 +162,16 @@ def _parity(proof: bytes, log_n: int):
             "vs": "c-oracle golden (tests/golden/mulchain_big.json, all 1472 proof bytes)"}
 
 
+def _dump(args, proof: bytes):
+    """--dump-proof / --dump-outputs: the proof of the last timed step, whichever implementation was timed."""
+    if args.dump_proof:
+        with open(args.dump_proof, "wb") as f:
+            f.write(proof)
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "proof.npy"), np.frombuffer(proof, dtype=np.uint8).astype(np.float64))
+
+
 def _cpu_prove(log_n, budget_s, max_steps):
     """Full proves of the oracle's C++ port on all host threads: (ms per prove, proves timed, threads, proof)."""
     os.environ["OMP_NUM_THREADS"] = str(os.cpu_count() or 1)   # torchrun exports OMP_NUM_THREADS=1
@@ -220,6 +236,7 @@ def run_reference(args):
         "parity": _parity(proof, args.log_n),
         "timed_region_s": round(ms * done / 1e3, 1),
     }
+    _dump(args, proof)
     print(json.dumps(line))
 
 
@@ -239,7 +256,11 @@ def main():
                     help="also time the resident prove with these tp_ctx_set_option settings (repeatable); reported under "
                          "'ab', never as the headline value")
     ap.add_argument("--dump-proof", default=None, help="write the proof bytes of the last timed step to this file (rank 0)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the output of the last timed step as DIR/proof.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -501,7 +522,7 @@ def main():
             f_res()
             ctx.prof_reset()
             ctx.prof_enable(True)
-            ns_steps = 5
+            ns_steps = args.steps
             # every step timed on its own (barrier + events), so that a single stalled upload shows as an outlier in
             # `*_per_step` instead of silently inflating the mean
             res_ms, e2e_ms, pr, pr2 = [], [], None, None
@@ -521,10 +542,10 @@ def main():
                 for k, v in opts.items():
                     ctx.set_option(k, v)
                 f_res()
-                t_ms, pr_ab = timed(f_res, 3)
+                t_ms, pr_ab = timed(f_res, ns_steps)
                 for k in opts:
                     ctx.set_option(k, DEFAULTS.get(k, 0))
-                ns_ab.append({"options": opts, "prove_ms": round(t_ms / 3, 3), "same_bytes": pr_ab == pr})
+                ns_ab.append({"options": opts, "prove_ms": round(t_ms / ns_steps, 3), "same_bytes": pr_ab == pr})
             line["north_star"] = {"workload": "mulchain_prove_n=2^%d" % lg, "gates": (1 << lg) - 3, "n_gpus": world,
                                   "prove_ms": round(sum(res_ms) / ns_steps, 3), "e2e_ms": round(sum(e2e_ms) / ns_steps, 3),
                                   "prove_ms_per_step": res_ms, "e2e_ms_per_step": e2e_ms,
@@ -553,10 +574,8 @@ def main():
             line["b0_as_written"] = _b0_as_written(log_n)
         except Exception as e:  # noqa: BLE001
             line["cpu_baseline"] = {"value": None, "unit": UNIT, "cores": 0, "kind": "port", "sample": "failed: %r" % (e,)}
-    if rank == 0 and args.dump_proof:
-        with open(args.dump_proof, "wb") as f:
-            f.write(proof)
     if rank == 0:
+        _dump(args, proof)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
