@@ -114,6 +114,9 @@ int tp_ctx_group_size(const tp_ctx* ctx, int* ndev, int* uses_nccl);
  *       3: eight elements, 2048-element tiles, two blocks per SM (the round-1 shape);
  *   "msm_acc_staged" (0/1): the accumulation kernel fetches the next table point into shared memory with cp.async
  *       while the current addition runs;
+ *   "msm_fq_lazy" (1 [default] or 0): the MSM's XYZZ addition laws keep Fq values in [0, 2q) -- products without
+ *       their final conditional subtraction, sums and differences modulo 2q -- and normalise the reduction's outputs
+ *       to [0, q) before they leave the device; 0: every value canonical after every operation;
  *   "quotient_all_cosets" (0/1): evaluate the quotient numerator on all four cosets of the 4n domain even when it is
  *       known to vanish on H (gates and copy constraints hold); by default that coset is skipped. */
 int tp_ctx_set_option(tp_ctx* ctx, const char* name, long value);

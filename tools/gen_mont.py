@@ -323,6 +323,78 @@ def check_lazy(mod, n, trials=3000):
     print("%d-limb lazy forms ok" % n)
 
 
+# ---- lazy Fq arithmetic for the MSM's XYZZ addition laws: values stay in [0, 2q) ---------------------------------------
+# q = 0.8126 * 2^381, so 8q < R = 2^384.  A Montgomery product (a b + m q) / R of a, b < 2q is below q (4q / R + 1) <
+# 1.41 q, and a lazy pair a b + c d of operands <= 2q (8 q^2 < q R) below q (8q / R + 1) < 1.82 q: none of the products
+# needs its final conditional subtraction.  Sums and differences are taken modulo 2q (the same cost as modulo q), so
+# every value between a table load and the last store of the reduction lies in [0, 2q); fq_norm2 returns to [0, q).
+# Unreduced sums or differences (up to 4q) would save the correction of a sum or difference too, but a square of such
+# a value is only bounded by q (16q / R + 1) > 2q: the laws square their differences (PP = (U2 - X1)^2, R^2).
+def build_kq_minus(mod, n, k):
+    """r = k p - a for a <= k p (no correction): a negation into [0, k p]"""
+    kl = limbs(k * mod, n)
+    pr = Prog()
+    for i in range(n):
+        op = "sub.cc.u32" if i == 0 else ("subc.cc.u32" if i < n - 1 else "subc.u32")
+        pr.emit(op, "r%d" % i, kl[i], "a%d" % i)
+    return pr
+
+
+def check_lazy_fq(mod, n, trials=2000):
+    R = 1 << (32 * n)
+    assert 8 * mod < R
+    rinv = pow(R, -1, mod)
+    rnd = random.Random(4243)
+    uid = _uid[0]   # the emitted header's temporary names stay what they were before this check existed
+    mul = build_mul(mod, n, reduce_final=False)
+    mul2 = build_mul(mod, n, reduce_final=False, pair2=True)
+    sqr = build_sep(mod, n, "sqr", reduce_final=False)
+    _uid[0] = uid
+    add2 = build_add(2 * mod, n)
+    sub2 = build_sub(2 * mod, n)
+    neg1 = build_kq_minus(mod, n, 1)
+    neg2 = build_kq_minus(mod, n, 2)
+    norm2 = build_condsub(mod, n, (1,))
+
+    def run(pr, **vals):
+        env = {}
+        for nm, v in vals.items():
+            for i, l in enumerate(limbs(v, n)):
+                env["%s%d" % (nm, i)] = l
+        o = pr.run(env)
+        return sum(o["r%d" % i] << (32 * i) for i in range(n))
+
+    # edge operands of the lazy range [0, 2q): values = 0 mod q held as 0 and q, the ends of both halves, all-ones limbs
+    big = [0, 1, mod - 1, mod, mod + 1, 2 * mod - 2, 2 * mod - 1, (1 << 381) - 1, 1 << 380, (R - 1) % (2 * mod),
+           ((1 << (16 * n)) - 1) % (2 * mod), mod // 2, R % mod]
+    lazy = big + [rnd.randrange(2 * mod) for _ in range(trials)]
+    cases = [(x, y) for x in big for y in big] + [(rnd.randrange(2 * mod), rnd.randrange(2 * mod)) for _ in range(trials)]
+    for x, y in cases:
+        # both operand orders: the interleaved form's carry asserts accept any pair below 2q
+        for a, b in ((x, y), (y, x)):
+            t = run(mul, a=a, b=b)
+            assert t < 2 * mod and t % mod == a * b * rinv % mod, ("lazy mul", hex(a), hex(b))
+        t = run(sqr, a=x)
+        assert t < 2 * mod and t % mod == x * x * rinv % mod, ("lazy sqr", hex(x))
+        s = run(add2, a=x, b=y)
+        d = run(sub2, a=x, b=y)
+        assert s < 2 * mod and s % mod == (x + y) % mod, ("add2", hex(x), hex(y))
+        assert d < 2 * mod and d % mod == (x - y) % mod, ("sub2", hex(x), hex(y))
+    # lazy pair: a b + c (2q - d), the subtrahend's negation (0, 2q] included
+    quads = [(x, y, c, d) for x in big[:8] for y in big[:8] for c in big[:8] for d in big[:8]]
+    quads += [tuple(rnd.randrange(2 * mod) for _ in range(4)) for _ in range(trials)]
+    for x, y, c, d in quads:
+        nd = run(neg2, a=d)
+        assert nd == 2 * mod - d
+        t = run(mul2, a=x, b=y, c=c, d=nd)
+        assert t < 2 * mod and t % mod == (x * y - c * d) * rinv % mod, ("lazy pair", hex(x), hex(y), hex(c), hex(d))
+    for u in lazy:
+        assert run(norm2, a=u) == u % mod
+    for u in [0, 1, mod - 1] + [rnd.randrange(mod) for _ in range(trials)]:
+        assert run(neg1, a=u) == mod - u
+    print("%d-limb lazy Fq forms ok" % n)
+
+
 # appended section for tools/gen_mont.py: separated-form (wide product + reduction) builders
 class Cols:
     """Column accumulators in two alignments over absolute limb positions: E holds 64-bit pairs at
@@ -528,9 +600,10 @@ def emit_wide_sqr(pr, a, t, temps):
                 drop_carry=last)
 
 
-def emit_redc(pr, t, out, mod, n, temps, m0=None):
+def emit_redc(pr, t, out, mod, n, temps, m0=None, reduce_final=True):
     """out = t / 2^(32 n) mod p (conditionally subtracted once), t = 2n plain limbs, t < p * 2^(32 n)
-    (or < 2 p^2 for a lazy pair -- the callers' bounds are checked by the simulator's carry asserts)."""
+    (or < 2 p^2 for a lazy pair -- the callers' bounds are checked by the simulator's carry asserts).
+    reduce_final=False: out = (t + m p) / 2^(32 n) < 2 p, without the subtraction."""
     pl = limbs(mod, n)
     if m0 is None:
         m0 = (-pow(mod, -1, 1 << 32)) & MASK
@@ -560,12 +633,17 @@ def emit_redc(pr, t, out, mod, n, temps, m0=None):
         pr.emit("add.cc.u32" if k == 0 else "addc.cc.u32", s[k], s[k], t[n + k])
     pr.emit("addc.u32", s[n], s[n], 0, drop_carry=True)
     # s < 2p (s[n] is zero whenever the inputs respect the bound; asserted through the cond-sub test)
+    if not reduce_final:
+        pr.emit("assert0", None, s[n])
+        for i in range(n):
+            pr.emit("mov.u32", out[i], s[i])
+        return
     d = fresh_names("rd", n)
     temps += d
     cond_sub_p(pr, s[:n], d, out, mod, n)
 
 
-def build_sep(mod, n, kind, karatsuba=False):
+def build_sep(mod, n, kind, karatsuba=False, reduce_final=True):
     """kind: 'mul' (a*b), 'sqr' (a*a), 'mul2' (a*b + c*d)"""
     pr = Prog()
     a = ["a%d" % i for i in range(n)]
@@ -589,7 +667,7 @@ def build_sep(mod, n, kind, karatsuba=False):
             pr.emit("add.cc.u32" if k == 0 else ("addc.cc.u32" if not last else "addc.u32"), t[k], t[k], t2[k],
                     drop_carry=last)
     out = ["r%d" % i for i in range(n)]
-    emit_redc(pr, t, out, mod, n, temps)
+    emit_redc(pr, t, out, mod, n, temps, reduce_final=reduce_final)
     pr.temps = temps
     return pr
 
@@ -724,6 +802,7 @@ def main():
     check_sep(R_MOD, 8)
     check_sep(Q_MOD, 12)
     check_lazy(R_MOD, 8)
+    check_lazy_fq(Q_MOD, 12)
     check("Fr", R_MOD, 8)
     check("Fr(mod in regs)", R_MOD, 8, mod_regs=True)
     check("Fr(m0 in a register)", R_MOD, 8, m0_reg=True)
@@ -768,6 +847,16 @@ def main():
             out.append(emit_fn_ops("fq_mul_sep_ptx", build_sep(mod, n, "mul"), n, ["a", "b"]))
             out.append(emit_fn_ops("fq_mul_kar_ptx", build_sep(mod, n, "mul", True), n, ["a", "b"]))
             out.append(emit_fn_ops("fq_mul2_kar_ptx", build_sep(mod, n, "mul2", True), n, ["a", "b", "c", "d"]))
+            # lazy forms for the MSM's addition laws (see build_kq_minus): values in [0, 2q)
+            out.append(emit_fn("fq_mul_lazy_ptx", build_mul(mod, n, reduce_final=False), n))
+            out.append(emit_fn_ops("fq_mul2_lazy_ptx", build_mul(mod, n, reduce_final=False, pair2=True), n,
+                                   ["a", "b", "c", "d"]))
+            out.append(emit_fn_ops("fq_sqr_lazy_ptx", build_sep(mod, n, "sqr", reduce_final=False), n, ["a"]))
+            out.append(emit_fn("fq_add2_ptx", build_add(2 * mod, n), n))
+            out.append(emit_fn("fq_sub2_ptx", build_sub(2 * mod, n), n))
+            out.append(emit_fn_ops("fq_neg1_ptx", build_kq_minus(mod, n, 1), n, ["a"]))
+            out.append(emit_fn_ops("fq_neg2_ptx", build_kq_minus(mod, n, 2), n, ["a"]))
+            out.append(emit_fn_ops("fq_norm2_ptx", build_condsub(mod, n, (1,)), n, ["a"]))
         out.append(emit_fn("%s_add_ptx" % name, build_add(mod, n), n))
         out.append(emit_fn("%s_sub_ptx" % name, build_sub(mod, n), n))
     dst = Path(__file__).resolve().parent.parent / "typlonk_b200" / "csrc" / "mont_gen.cuh"

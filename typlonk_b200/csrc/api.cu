@@ -168,6 +168,11 @@ int tp_ctx_set_option(tp_ctx* ctx, const char* name, long value) {
     ctx->msm_pipeline = (unsigned)value;
     return TP_OK;
   }
+  if (strcmp(name, "msm_fq_lazy") == 0) {
+    if (value < 0 || value > 1) return fail(ctx, TP_ERR_INVALID_ARG, "set_option: msm_fq_lazy must be 0 or 1");
+    ctx->msm_fq_lazy = (unsigned)value;
+    return TP_OK;
+  }
   if (strcmp(name, "msm_pipe_min_log") == 0) {
     if (value < 0 || value > 27) return fail(ctx, TP_ERR_INVALID_ARG, "set_option: msm_pipe_min_log must be 0..27");
     ctx->msm_pipe_min_log = (unsigned)value;

@@ -61,6 +61,7 @@ struct tp_ctx {
   unsigned msm_pipe_min_log = 15; // ... for inputs of at least 2^this points (tests lower it to reach the path with small circuits)
   unsigned ntt_radix_log = 2;     // butterfly stages per trip through registers: 3 (eight elements per thread) or 2 (four)
   unsigned msm_acc_staged = 0;    // 1: the accumulation stages the next table point in shared memory with cp.async
+  unsigned msm_fq_lazy = 1;       // 1: the MSM's addition laws keep Fq values in [0, 2q) (ec.cuh FqOps<true>); 0: canonical
   // work counters (tp_ctx_get_stat)
   double stat_msm_entries = 0, stat_msm_calls = 0, stat_msm_c = 0, stat_msm_nwin = 0, stat_msm_levels = 0, stat_msm_chunk = 0;
   // profiling

@@ -94,103 +94,143 @@ __device__ __forceinline__ G1Affine affine_pair_finish(const G1Affine& p1, const
   return r;
 }
 
-// 2 * (affine P), P != identity.
+// Field arithmetic of the XYZZ laws.  Canonical (LAZY = false): every value in [0, q), as SRS generation, wire checks
+// and the verifier use them.  Lazy (the MSM, msm.cu): every value in [0, 2q) -- products without their final
+// subtraction, sums and differences modulo 2q (field.cuh) -- and stored so; the MSM brings its outputs to [0, q) with
+// fq_norm2 before they leave the device.  The bounds in the comments of the laws are those of the lazy form.
+template <bool LAZY> struct FqOps;
+template <> struct FqOps<false> {
+  static __device__ __forceinline__ Fq mul(const Fq& a, const Fq& b) { return fq_mul(a, b); }
+  static __device__ __forceinline__ Fq sqr(const Fq& a) { return fq_sqr(a); }
+  static __device__ __forceinline__ Fq mul_sub2(const Fq& a, const Fq& b, const Fq& c, const Fq& d) { return fq_mul_sub2(a, b, c, d); }
+  static __device__ __forceinline__ Fq add(const Fq& a, const Fq& b) { return fq_add(a, b); }
+  static __device__ __forceinline__ Fq sub(const Fq& a, const Fq& b) { return fq_sub(a, b); }
+  static __device__ __forceinline__ Fq dbl(const Fq& a) { return fq_dbl(a); }
+  static __device__ __forceinline__ Fq neg(const Fq& a) { return fq_neg(a); }
+  static __device__ __forceinline__ bool is_zero(const Fq& a) { return fq_is_zero(a); }
+};
+template <> struct FqOps<true> {
+  static __device__ __forceinline__ Fq mul(const Fq& a, const Fq& b) { return fq_mul_lazy(a, b); }
+  static __device__ __forceinline__ Fq sqr(const Fq& a) { return fq_sqr_lazy(a); }
+  static __device__ __forceinline__ Fq mul_sub2(const Fq& a, const Fq& b, const Fq& c, const Fq& d) { return fq_mul_sub2_lazy(a, b, c, d); }
+  static __device__ __forceinline__ Fq add(const Fq& a, const Fq& b) { return fq_add2(a, b); }
+  static __device__ __forceinline__ Fq sub(const Fq& a, const Fq& b) { return fq_sub2(a, b); }
+  static __device__ __forceinline__ Fq dbl(const Fq& a) { return fq_dbl2(a); }
+  static __device__ __forceinline__ Fq neg(const Fq& a) { return fq_neg_lazy(a); }   // a canonical: q - a in [1, q]
+  // exact: zero mod q, i.e. 0 or q in [0, 2q)
+  static __device__ __forceinline__ bool is_zero(const Fq& a) { return fq_is_zero2(a); }
+};
+
+// The identity test ZZ == 0 stays exact on lazy values: ZZ is zeroed only explicitly (xyzz_identity), and every other ZZ
+// is a product of factors that are non-zero mod q (the new ZZ of an addition is ZZ1 (ZZ2) PP with PP != 0 mod q, of a
+// doubling V ZZ1 with V = 4 Y1^2 != 0: G1 has no point of order 2), which lies in [0, 2q) and is neither 0 nor q.
+
+// 2 * (affine P), P != identity.  P canonical, or y lazy in [1, q] (a negated table point).
+template <bool LAZY = false>
 static __device__ __noinline__ void xyzz_mdbl(G1Xyzz& r, const G1Affine p) {
-  Fq u = fq_dbl(p.y);
-  Fq v = fq_sqr(u);
-  Fq w = fq_mul(u, v);
-  Fq s = fq_mul(p.x, v);
-  Fq xx = fq_sqr(p.x);
-  Fq m = fq_add(fq_dbl(xx), xx);
-  Fq x3 = fq_sub(fq_sqr(m), fq_dbl(s));
-  r.y = fq_mul_sub2(m, fq_sub(s, x3), w, p.y);
+  using F = FqOps<LAZY>;
+  Fq u = F::dbl(p.y);                  // < 2q (every value below: < 2q)
+  Fq v = F::sqr(u);
+  Fq w = F::mul(u, v);
+  Fq s = F::mul(p.x, v);
+  Fq xx = F::sqr(p.x);
+  Fq m = F::add(F::dbl(xx), xx);
+  Fq x3 = F::sub(F::sqr(m), F::dbl(s));
+  r.y = F::mul_sub2(m, F::sub(s, x3), w, p.y);   // m (s - x3) + w (2q - y): < 8 q^2 before the reduction
   r.x = x3;
   r.zz = v;
   r.zzz = w;
 }
 
+template <bool LAZY = false>
 static __device__ __noinline__ void xyzz_dbl(G1Xyzz& r) {
+  using F = FqOps<LAZY>;
   if (xyzz_is_identity(r)) return;
-  Fq u = fq_dbl(r.y);
-  Fq v = fq_sqr(u);
-  Fq w = fq_mul(u, v);
-  Fq s = fq_mul(r.x, v);
-  Fq xx = fq_sqr(r.x);
-  Fq m = fq_add(fq_dbl(xx), xx);
-  Fq x3 = fq_sub(fq_sqr(m), fq_dbl(s));
-  Fq y3 = fq_mul_sub2(m, fq_sub(s, x3), w, r.y);
+  Fq u = F::dbl(r.y);                  // < 2q (every value below: < 2q)
+  Fq v = F::sqr(u);
+  Fq w = F::mul(u, v);
+  Fq s = F::mul(r.x, v);
+  Fq xx = F::sqr(r.x);
+  Fq m = F::add(F::dbl(xx), xx);
+  Fq x3 = F::sub(F::sqr(m), F::dbl(s));
+  Fq y3 = F::mul_sub2(m, F::sub(s, x3), w, r.y);
   r.x = x3;
   r.y = y3;
-  r.zz = fq_mul(v, r.zz);
-  r.zzz = fq_mul(w, r.zzz);
+  r.zz = F::mul(v, r.zz);
+  r.zzz = F::mul(w, r.zzz);
 }
 
-// acc += P (affine, not identity); `neg` adds -P.  Handles acc == identity, acc == P, acc == -P.
+// acc += P (affine, not identity, canonical); `neg` adds -P.  Handles acc == identity, acc == P, acc == -P.
+template <bool LAZY = false>
 __device__ __forceinline__ void xyzz_madd(G1Xyzz& acc, const G1Affine& p_in, bool neg) {
+  using F = FqOps<LAZY>;
   G1Affine p = p_in;
-  if (neg) p.y = fq_neg(p.y);
+  if (neg) p.y = F::neg(p.y);          // lazy: q - y in [1, q]
   if (xyzz_is_identity(acc)) {
     acc.x = p.x; acc.y = p.y; acc.zz = fq_one(); acc.zzz = fq_one();
     return;
   }
-  Fq u2 = fq_mul(p.x, acc.zz);
-  Fq s2 = fq_mul(p.y, acc.zzz);
-  Fq pp_ = fq_sub(u2, acc.x);
-  Fq rr = fq_sub(s2, acc.y);
-  if (fq_is_zero(pp_)) {
-    if (fq_is_zero(rr)) {
+  Fq u2 = F::mul(p.x, acc.zz);         // < 2q, as every value below
+  Fq s2 = F::mul(p.y, acc.zzz);
+  Fq pp_ = F::sub(u2, acc.x);
+  Fq rr = F::sub(s2, acc.y);
+  if (F::is_zero(pp_)) {
+    if (F::is_zero(rr)) {
       G1Xyzz d;  // separate object so `acc` itself never has its address taken
-      xyzz_mdbl(d, p);
+      xyzz_mdbl<LAZY>(d, p);
       acc = d;
     } else {
       acc = xyzz_identity();
     }
     return;
   }
-  Fq pp = fq_sqr(pp_);
-  Fq ppp = fq_mul(pp_, pp);
-  Fq q = fq_mul(acc.x, pp);
-  Fq x3 = fq_sub(fq_sub(fq_sqr(rr), ppp), fq_dbl(q));
-  Fq y3 = fq_mul_sub2(rr, fq_sub(q, x3), acc.y, ppp);
+  Fq pp = F::sqr(pp_);
+  Fq ppp = F::mul(pp_, pp);
+  Fq q = F::mul(acc.x, pp);
+  Fq x3 = F::sub(F::sub(F::sqr(rr), ppp), F::dbl(q));
+  Fq y3 = F::mul_sub2(rr, F::sub(q, x3), acc.y, ppp);   // rr (q - x3) + y1 (2q - ppp): < 8 q^2 before the reduction
   acc.x = x3;
   acc.y = y3;
-  acc.zz = fq_mul(acc.zz, pp);
-  acc.zzz = fq_mul(acc.zzz, ppp);
+  acc.zz = F::mul(acc.zz, pp);
+  acc.zzz = F::mul(acc.zzz, ppp);
 }
 
 // acc += b (both XYZZ), all special cases handled.
+template <bool LAZY = false>
 static __device__ __noinline__ void xyzz_add(G1Xyzz& acc, const G1Xyzz& b) {
+  using F = FqOps<LAZY>;
   if (xyzz_is_identity(b)) return;
   if (xyzz_is_identity(acc)) {
     acc = b;
     return;
   }
-  Fq u1 = fq_mul(acc.x, b.zz);
-  Fq u2 = fq_mul(b.x, acc.zz);
-  Fq s1 = fq_mul(acc.y, b.zzz);
-  Fq s2 = fq_mul(b.y, acc.zzz);
-  Fq pp_ = fq_sub(u2, u1);
-  Fq rr = fq_sub(s2, s1);
-  if (fq_is_zero(pp_)) {
-    if (fq_is_zero(rr)) {
-      xyzz_dbl(acc);
+  Fq u1 = F::mul(acc.x, b.zz);         // < 2q, as every value below
+  Fq u2 = F::mul(b.x, acc.zz);
+  Fq s1 = F::mul(acc.y, b.zzz);
+  Fq s2 = F::mul(b.y, acc.zzz);
+  Fq pp_ = F::sub(u2, u1);
+  Fq rr = F::sub(s2, s1);
+  if (F::is_zero(pp_)) {
+    if (F::is_zero(rr)) {
+      xyzz_dbl<LAZY>(acc);
     } else {
       acc = xyzz_identity();
     }
     return;
   }
-  Fq pp = fq_sqr(pp_);
-  Fq ppp = fq_mul(pp_, pp);
-  Fq q = fq_mul(u1, pp);
-  Fq x3 = fq_sub(fq_sub(fq_sqr(rr), ppp), fq_dbl(q));
-  Fq y3 = fq_mul_sub2(rr, fq_sub(q, x3), s1, ppp);
+  Fq pp = F::sqr(pp_);
+  Fq ppp = F::mul(pp_, pp);
+  Fq q = F::mul(u1, pp);
+  Fq x3 = F::sub(F::sub(F::sqr(rr), ppp), F::dbl(q));
+  Fq y3 = F::mul_sub2(rr, F::sub(q, x3), s1, ppp);      // < 8 q^2 before the reduction
   acc.x = x3;
   acc.y = y3;
-  acc.zz = fq_mul(fq_mul(acc.zz, b.zz), pp);
-  acc.zzz = fq_mul(fq_mul(acc.zzz, b.zzz), ppp);
+  acc.zz = F::mul(F::mul(acc.zz, b.zz), pp);
+  acc.zzz = F::mul(F::mul(acc.zzz, b.zzz), ppp);
 }
 
 // acc = k * acc for a small non-negative integer k (double-and-add, MSB first).
+template <bool LAZY = false>
 static __device__ __noinline__ void xyzz_mul_small(G1Xyzz& acc, uint32_t k) {
   if (k == 0 || xyzz_is_identity(acc)) {
     acc = xyzz_identity();
@@ -199,9 +239,16 @@ static __device__ __noinline__ void xyzz_mul_small(G1Xyzz& acc, uint32_t k) {
   G1Xyzz base = acc;
   int top = 31 - __clz(k);
   for (int b = top - 1; b >= 0; b--) {
-    xyzz_dbl(acc);
-    if ((k >> b) & 1) xyzz_add(acc, base);
+    xyzz_dbl<LAZY>(acc);
+    if ((k >> b) & 1) xyzz_add<LAZY>(acc, base);
   }
+}
+
+// [0, 2q) -> [0, q): the last device step of a lazy point before it leaves the device
+__device__ __forceinline__ G1Xyzz xyzz_norm2(const G1Xyzz& a) {
+  G1Xyzz r;
+  r.x = fq_norm2(a.x); r.y = fq_norm2(a.y); r.zz = fq_norm2(a.zz); r.zzz = fq_norm2(a.zzz);
+  return r;
 }
 
 }  // namespace tp

@@ -239,6 +239,62 @@ __device__ __forceinline__ bool fq_eq(const Fq& a, const Fq& b) {
   for (int i = 0; i < 12; i++) o |= a.v[i] ^ b.v[i];
   return o == 0;
 }
+// Lazy forms for the MSM's addition laws (tools/gen_mont.py build_kq_minus): values in [0, 2q), 8q < 2^384.  Products
+// of operands below 2q, and the pair a b - c d with c, d below 2q, come out below 2q without the final subtraction
+// (either operand order: the simulator checks both); sums and differences are taken modulo 2q; fq_norm2 returns to
+// [0, q).  Canonical values are valid lazy inputs.
+__device__ __forceinline__ Fq fq_mul_lazy(const Fq& a, const Fq& b) {
+  Fq r;
+  fq_mul_lazy_ptx(r.v, a.v, b.v);
+  return r;
+}
+__device__ __forceinline__ Fq fq_sqr_lazy(const Fq& a) {
+  Fq r;
+  fq_sqr_lazy_ptx(r.v, a.v);
+  return r;
+}
+// a b - c d = a b + c (2q - d): 2q - d lies in (0, 2q], 4 q^2 + 4 q^2 < q 2^384
+__device__ __forceinline__ Fq fq_mul_sub2_lazy(const Fq& a, const Fq& b, const Fq& c, const Fq& d) {
+  Fq nd, r;
+  fq_neg2_ptx(nd.v, d.v);
+  fq_mul2_lazy_ptx(r.v, a.v, b.v, c.v, nd.v);
+  return r;
+}
+__device__ __forceinline__ Fq fq_add2(const Fq& a, const Fq& b) {
+  Fq r;
+  fq_add2_ptx(r.v, a.v, b.v);
+  return r;
+}
+__device__ __forceinline__ Fq fq_sub2(const Fq& a, const Fq& b) {
+  Fq r;
+  fq_sub2_ptx(r.v, a.v, b.v);
+  return r;
+}
+__device__ __forceinline__ Fq fq_dbl2(const Fq& a) { return fq_add2(a, a); }
+// q - a for a canonical a: in [1, q], no correction
+__device__ __forceinline__ Fq fq_neg_lazy(const Fq& a) {
+  Fq r;
+  fq_neg1_ptx(r.v, a.v);
+  return r;
+}
+__device__ __forceinline__ Fq fq_norm2(const Fq& a) {
+  Fq r;
+  fq_norm2_ptx(r.v, a.v);
+  return r;
+}
+// a = 0 mod q for a in [0, 2q), i.e. a is 0 or q.  The low limb filters: the full compare runs only when it is the low
+// limb of 0 or of q, which a non-zero value almost never has.
+__device__ __forceinline__ bool fq_is_zero2(const Fq& a) {
+  const uint32_t q[12] = TP_FQ_MOD;
+  if (a.v[0] != 0 && a.v[0] != q[0]) return false;
+  uint32_t oz = 0, oq = 0;
+#pragma unroll
+  for (int i = 0; i < 12; i++) {
+    oz |= a.v[i];
+    oq |= a.v[i] ^ q[i];
+  }
+  return oz == 0 || oq == 0;
+}
 static __device__ __noinline__ Fq fq_inv(const Fq& a) {
   const uint32_t e[12] = TP_FQ_MODM2;
   Fq r = fq_one();

@@ -620,8 +620,11 @@ __global__ void __launch_bounds__(AFF_THREADS, 4) k_aff_round(const G1Affine* __
 // stages) while the addition of entry e runs, instead of stalling the addition on a load from a multi-GB table with
 // three warps per scheduler to cover it; costs no registers (a prefetch hint into L1 / L2 measured slower, section 7 of
 // DESIGN.md).
+// LAZY (option msm_fq_lazy, default on): the XYZZ laws on Fq values in [0, 2q) (ec.cuh FqOps<true>) in this kernel and in
+// every later one of the MSM -- buckets, partials and running sums are stored lazy -- until the reduction's outputs are
+// normalised to [0, q) in k_msm_treesum / k_msm_combine.  The same points mod q as the canonical laws, so the same bytes.
 #define ACC_THREADS 128
-template <bool STAGED>
+template <bool STAGED, bool LAZY>
 __global__ void __launch_bounds__(ACC_THREADS, TP_ACC_MIN_BLOCKS) k_msm_accumulate(const G1Affine* __restrict__ bases,
                                                         const G1Affine* __restrict__ scratch, unsigned split,
                                                         const uint2* __restrict__ sorted /* (index | sign, key) */,
@@ -703,7 +706,7 @@ __global__ void __launch_bounds__(ACC_THREADS, TP_ACC_MIN_BLOCKS) k_msm_accumula
 #endif
       p = affine_load(msm_point(bases, scratch, split, idx & 0x7fffffffu));
     }
-    if (!affine_is_identity(p)) xyzz_madd(acc, p, (idx >> 31) != 0);
+    if (!affine_is_identity(p)) xyzz_madd<LAZY>(acc, p, (idx >> 31) != 0);
   }
   if (is_first_run) {
     part_keys[2 * t] = cur;
@@ -895,6 +898,7 @@ __global__ void __launch_bounds__(128, AFC_MIN_BLOCKS) k_msm_accumulate_affine(c
 // PAIR_MAX_SPAN chunks, so the walk is at most PAIR_MAX_SPAN + 1 additions and almost always one;
 // heavier skew goes through the logarithmic merge below.
 #define PAIR_MAX_SPAN 8
+template <bool LAZY>
 __global__ void __launch_bounds__(128) k_msm_pair_fixup(const unsigned* __restrict__ part_keys,
                                                         const G1Xyzz* __restrict__ part_pts, unsigned nchunks,
                                                         G1Xyzz* __restrict__ buckets) {
@@ -914,7 +918,7 @@ __global__ void __launch_bounds__(128) k_msm_pair_fixup(const unsigned* __restri
   G1Xyzz acc = xyzz_load(part_pts + 2 * t + (multi ? 1 : 0));
   for (unsigned j = t + 1; j < nchunks && part_keys[2 * j] == key; j++) {
     G1Xyzz h = xyzz_load(part_pts + 2 * j);
-    xyzz_add(acc, h);
+    xyzz_add<LAZY>(acc, h);
     if (!(part_keys[2 * j + 1] & MSM_IDENT)) break;  // chunk j has further runs: this one ended there
   }
   xyzz_store(buckets + key, acc);
@@ -928,6 +932,7 @@ __global__ void __launch_bounds__(128) k_msm_pair_fixup(const unsigned* __restri
 // extra levels of ~MERGE_B additions, so a bucket holding millions of points (small top window,
 // repeated scalars) is as parallel as a uniform one.  The last level is one thread.
 #define MERGE_B 16
+template <bool LAZY>
 __global__ void __launch_bounds__(128) k_msm_merge_level(const unsigned* __restrict__ keys_in,
                                                          const G1Xyzz* __restrict__ pts_in, unsigned nslots,
                                                          G1Xyzz* __restrict__ buckets, unsigned* __restrict__ keys_out,
@@ -955,7 +960,7 @@ __global__ void __launch_bounds__(128) k_msm_merge_level(const unsigned* __restr
       acc = (kraw & MSM_IDENT) ? xyzz_identity() : xyzz_load(pts_in + e);
     } else if (!(kraw & MSM_IDENT)) {
       G1Xyzz o = xyzz_load(pts_in + e);
-      xyzz_add(acc, o);
+      xyzz_add<LAZY>(acc, o);
     }
   }
   if (final_level) {
@@ -983,6 +988,7 @@ __global__ void __launch_bounds__(128) k_msm_merge_level(const unsigned* __restr
 #ifndef TP_WSUM_MIN_BLOCKS
 #define TP_WSUM_MIN_BLOCKS 3   // 168 registers; 4 blocks (128 registers, 36 bytes of spills): reduce +0.27 ms, 5: +0.7 (profiles r2 J)
 #endif
+template <bool LAZY>
 __global__ void __launch_bounds__(128, TP_WSUM_MIN_BLOCKS) k_msm_wsum_level(const G1Xyzz* __restrict__ in, const unsigned* __restrict__ hist,
                                                         unsigned m_in, unsigned seg, unsigned total_out,
                                                         G1Xyzz* __restrict__ r_out, G1Xyzz* __restrict__ t_out) {
@@ -994,9 +1000,9 @@ __global__ void __launch_bounds__(128, TP_WSUM_MIN_BLOCKS) k_msm_wsum_level(cons
   for (int j = (int)seg - 1; j >= 0; j--) {
     if (!hist || hist[base + j] != 0) {  // first level: empty buckets were never written
       G1Xyzz p = xyzz_load(in + base + j);
-      xyzz_add(running, p);
+      xyzz_add<LAZY>(running, p);
     }
-    if (j > 0) xyzz_add(tot, running);
+    if (j > 0) xyzz_add<LAZY>(tot, running);
   }
   xyzz_store(r_out + t, running);
   xyzz_store(t_out + t, tot);
@@ -1030,6 +1036,8 @@ struct TreeTasks {
   unsigned first[TS_MAX_TASKS + 1];  // block index of each task's job 0
   int ntasks;
 };
+// LAZY: the sums come out normalised to [0, q) -- what the host (or, sharded, k_msm_combine) reads is canonical.
+template <bool LAZY>
 __global__ void __launch_bounds__(TS_THREADS) k_msm_treesum(TreeTasks tasks) {
   __shared__ G1Xyzz sh[TS_THREADS];
   int k = 0;
@@ -1045,7 +1053,7 @@ __global__ void __launch_bounds__(TS_THREADS) k_msm_treesum(TreeTasks tasks) {
     const size_t e = (size_t)i * tk.stride;
     if (h && h[e] == 0) continue;   // raw buckets: empty ones were never written
     G1Xyzz p = xyzz_load(src + e);
-    xyzz_add(acc, p);
+    xyzz_add<LAZY>(acc, p);
   }
   sh[threadIdx.x] = acc;
   __syncthreads();
@@ -1053,12 +1061,12 @@ __global__ void __launch_bounds__(TS_THREADS) k_msm_treesum(TreeTasks tasks) {
     if (threadIdx.x < d) {
       G1Xyzz a = sh[threadIdx.x];
       G1Xyzz b = sh[threadIdx.x + d];
-      xyzz_add(a, b);
+      xyzz_add<LAZY>(a, b);
       sh[threadIdx.x] = a;
     }
     __syncthreads();
   }
-  if (threadIdx.x == 0) xyzz_store(tk.dst + (size_t)set * tk.dst_set_stride + job, sh[0]);
+  if (threadIdx.x == 0) xyzz_store(tk.dst + (size_t)set * tk.dst_set_stride + job, LAZY ? xyzz_norm2(sh[0]) : sh[0]);
 }
 
 // ---- 7. cross-rank combination (sharded MSM) --------------------------------------------------------
@@ -1067,7 +1075,9 @@ __global__ void __launch_bounds__(TS_THREADS) k_msm_treesum(TreeTasks tasks) {
 // host runs per bucket set is linear in the slots and, except for slot 0 (P = sum of the rank's buckets, which enters
 // with the rank-dependent factor rank + 1), the same on every rank: slots >= 1 are therefore summed over ranks here --
 // one warp per (set, slot), lane r holding rank r's point, a shared-memory tree -- and the `world` P points pass
-// through.  out: [sets][(slots - 1) sums | world P points].
+// through.  out: [sets][(slots - 1) sums | world P points].  LAZY: the inputs come canonical from k_msm_treesum, the sums
+// are normalised back to [0, q) before the host reads them.
+template <bool LAZY>
 __global__ void __launch_bounds__(32) k_msm_combine(const G1Xyzz* __restrict__ gathered, unsigned world, unsigned rank_stride,
                                                     unsigned slots, G1Xyzz* __restrict__ out) {
   __shared__ G1Xyzz sh[32];
@@ -1086,12 +1096,12 @@ __global__ void __launch_bounds__(32) k_msm_combine(const G1Xyzz* __restrict__ g
     if (r < d && r + d < world) {
       G1Xyzz a = sh[r];
       G1Xyzz b = sh[r + d];
-      xyzz_add(a, b);
+      xyzz_add<LAZY>(a, b);
       sh[r] = a;
     }
     __syncwarp();
   }
-  if (r == 0) xyzz_store(out + (size_t)set * width + (slot - 1), sh[0]);
+  if (r == 0) xyzz_store(out + (size_t)set * width + (slot - 1), LAZY ? xyzz_norm2(sh[0]) : sh[0]);
 }
 
 // ---- host side ---------------------------------------------------------------------------------
@@ -1184,6 +1194,7 @@ struct MsmJob {
   size_t nkeys = 0;
   unsigned m_total = 0, max_bucket = 0, nchunks = 0;
   bool pair_path = true, empty = false, reduce_queued = false;
+  bool lazy = true;      // option msm_fq_lazy when the job was queued: every kernel of the job uses the same laws
   // reduction plan
   int nl = 0;
   unsigned m_level[WSUM_MAX_LEVELS + 1], seg_level[WSUM_MAX_LEVELS + 1], tcount[WSUM_MAX_LEVELS + 1], tjobs[WSUM_MAX_LEVELS + 1];
@@ -1544,14 +1555,11 @@ static int job_accumulate(tp_ctx* ctx, MsmPipe* p, MsmJob& j) {
             (G1Xyzz*)ln.part_pts.p);
         TP_LAUNCH(ctx, "k_msm_accumulate_affine");
       } else {
-        if (ctx->msm_acc_staged)
-          k_msm_accumulate<true><<<(nchunks + ACC_THREADS - 1) / ACC_THREADS, ACC_THREADS, 0, ctx->stream>>>(
-              bases, scratch, (unsigned)split, final_list, final_m, nchunks, buckets, (unsigned*)ln.part_keys.p,
-              (G1Xyzz*)ln.part_pts.p, chunk);
-        else
-          k_msm_accumulate<false><<<(nchunks + ACC_THREADS - 1) / ACC_THREADS, ACC_THREADS, 0, ctx->stream>>>(
-              bases, scratch, (unsigned)split, final_list, final_m, nchunks, buckets, (unsigned*)ln.part_keys.p,
-              (G1Xyzz*)ln.part_pts.p, chunk);
+        const auto acc_kernel = ctx->msm_acc_staged ? (j.lazy ? k_msm_accumulate<true, true> : k_msm_accumulate<true, false>)
+                                                    : (j.lazy ? k_msm_accumulate<false, true> : k_msm_accumulate<false, false>);
+        acc_kernel<<<(nchunks + ACC_THREADS - 1) / ACC_THREADS, ACC_THREADS, 0, ctx->stream>>>(
+            bases, scratch, (unsigned)split, final_list, final_m, nchunks, buckets, (unsigned*)ln.part_keys.p,
+            (G1Xyzz*)ln.part_pts.p, chunk);
         TP_LAUNCH(ctx, "k_msm_accumulate");
       }
     }
@@ -1562,7 +1570,7 @@ static int job_accumulate(tp_ctx* ctx, MsmPipe* p, MsmJob& j) {
     {
       ProfScope prof(ctx, TP_PHASE_MSM_REDUCE);
       if (j.pair_path) {
-        k_msm_pair_fixup<<<(nchunks + 63) / 64, 64, 0, ctx->stream>>>((const unsigned*)ln.part_keys.p, (const G1Xyzz*)ln.part_pts.p,
+        (j.lazy ? k_msm_pair_fixup<true> : k_msm_pair_fixup<false>)<<<(nchunks + 63) / 64, 64, 0, ctx->stream>>>((const unsigned*)ln.part_keys.p, (const G1Xyzz*)ln.part_pts.p,
                                                                       nchunks, buckets);
         TP_LAUNCH(ctx, "k_msm_pair_fixup");
       } else {
@@ -1571,15 +1579,16 @@ static int job_accumulate(tp_ctx* ctx, MsmPipe* p, MsmJob& j) {
         unsigned* kb = ka + 2 * (size_t)nchunks;
         G1Xyzz* pb = pa + 2 * (size_t)nchunks;
         unsigned nslots = 2 * nchunks;
+        const auto merge = j.lazy ? k_msm_merge_level<true> : k_msm_merge_level<false>;
         while (nslots > 2 * MERGE_B) {
           unsigned nth = (nslots + MERGE_B - 1) / MERGE_B;
-          k_msm_merge_level<<<(nth + 127) / 128, 128, 0, ctx->stream>>>(ka, pa, nslots, buckets, kb, pb, 0);
+          merge<<<(nth + 127) / 128, 128, 0, ctx->stream>>>(ka, pa, nslots, buckets, kb, pb, 0);
           TP_LAUNCH(ctx, "k_msm_merge_level");
           std::swap(ka, kb);
           std::swap(pa, pb);
           nslots = 2 * nth;
         }
-        k_msm_merge_level<<<1, 32, 0, ctx->stream>>>(ka, pa, nslots, buckets, kb, pb, 1);
+        merge<<<1, 32, 0, ctx->stream>>>(ka, pa, nslots, buckets, kb, pb, 1);
         TP_LAUNCH(ctx, "k_msm_merge_level");
       }
     }
@@ -1651,7 +1660,7 @@ static int job_reduce(tp_ctx* ctx, MsmPipe* p, MsmJob& j) {
         G1Xyzz* r_out = cursor;
         G1Xyzz* t_out = cursor + total_out;
         cursor += 2 * (size_t)total_out;
-        k_msm_wsum_level<<<(total_out + 127) / 128, 128, 0, ctx->stream>>>(cur_in, cur_hist, j.m_level[l - 1], j.seg_level[l],
+        (j.lazy ? k_msm_wsum_level<true> : k_msm_wsum_level<false>)<<<(total_out + 127) / 128, 128, 0, ctx->stream>>>(cur_in, cur_hist, j.m_level[l - 1], j.seg_level[l],
                                                                            total_out, r_out, t_out);
         TP_LAUNCH(ctx, "k_msm_wsum_level");
         cur_in = r_out;
@@ -1687,7 +1696,8 @@ static int job_reduce(tp_ctx* ctx, MsmPipe* p, MsmJob& j) {
     add_task(ta, cur_in, cur_hist, D, m_rc, rows, rows, cols, cols, 1, -1);
     add_task(ta, cur_in, cur_hist, C, m_rc, cols, cols, 1, rows, cols, -1);
     for (int l = 1; l <= nl; l++) add_task(ta, t_arr[l], nullptr, TPs[l], j.m_level[l], j.tjobs[l], j.tjobs[l], j.tcount[l], j.tcount[l], 1, -1);
-    k_msm_treesum<<<dim3(ta.first[ta.ntasks], nsets_total), TS_THREADS, 0, ctx->stream>>>(ta);
+    const auto treesum = j.lazy ? k_msm_treesum<true> : k_msm_treesum<false>;
+    treesum<<<dim3(ta.first[ta.ntasks], nsets_total), TS_THREADS, 0, ctx->stream>>>(ta);
     TP_LAUNCH(ctx, "k_msm_treesum");
     // stage B: one slot each -- P, the bit sums of D and of C, the totals of the t arrays
     G1Xyzz* fin = (G1Xyzz*)ctx->msm_winsums.p + j.win_off;
@@ -1702,7 +1712,7 @@ static int job_reduce(tp_ctx* ctx, MsmPipe* p, MsmJob& j) {
       memset(&tb, 0, sizeof(tb));
       for (size_t q = s0; q < slots.size() && q < s0 + TS_MAX_TASKS; q++)
         add_task(tb, slots[q].src, nullptr, fin + q, slots[q].set_stride, total_masks, 1, 0, slots[q].count, 1, slots[q].bit);
-      k_msm_treesum<<<dim3(tb.first[tb.ntasks], nsets_total), TS_THREADS, 0, ctx->stream>>>(tb);
+      treesum<<<dim3(tb.first[tb.ntasks], nsets_total), TS_THREADS, 0, ctx->stream>>>(tb);
       TP_LAUNCH(ctx, "k_msm_treesum");
     }
   }
@@ -1742,6 +1752,7 @@ static int pipe_submit(tp_ctx* ctx, const tp_srs* srs, const Fr* const* scalars,
   j.pl = pl;
   j.nsets_total = pl.nsets * (unsigned)batch;
   j.nkeys = (size_t)j.nsets_total * pl.nbuck;
+  j.lazy = ctx->msm_fq_lazy != 0;
   j.first_result = p->results;
   p->results += batch;
   job_plan_reduce(ctx, j);
@@ -1817,7 +1828,7 @@ static int pipe_finish(tp_ctx* ctx, tph::HG1* results, int count) {
       TP_TRY(comm_allgather(ctx, ctx->msm_winsums.p, gathered, per_rank));
       for (auto& q : p->jobs) {
         if (q.empty) continue;
-        k_msm_combine<<<q.nsets_total * q.total_masks, 32, 0, ctx->stream>>>(gathered + q.win_off, world, (unsigned)p->win_used,
+        (q.lazy ? k_msm_combine<true> : k_msm_combine<false>)<<<q.nsets_total * q.total_masks, 32, 0, ctx->stream>>>(gathered + q.win_off, world, (unsigned)p->win_used,
                                                                              q.total_masks, combined + q.host_off);
         TP_LAUNCH(ctx, "k_msm_combine");
       }

@@ -397,8 +397,9 @@ class Context:
         return v.value
 
     def set_option(self, name, value):
-        """Tunables of the library ("msm_affine_chains": 0/1, "msm_affine_rounds": 0..8); results do not
-        depend on them."""
+        """Tunables of the library ("msm_affine_chains": 0/1, "msm_affine_rounds": 0..8, "msm_reduce_l1": 0..2,
+        "msm_pipeline": 0..2, "msm_pipe_min_log": 0..27, "msm_acc_staged": 0/1, "msm_fq_lazy": 1 [default] / 0,
+        "ntt_radix_log": 2/3, "quotient_all_cosets": 0/1; see the header); results do not depend on them."""
         self._check(lib().tp_ctx_set_option(self._h, name.encode(), C.c_long(int(value))))
 
     def get_stat(self, name) -> float:
