@@ -251,6 +251,23 @@ int tp_circuit_read_poly(tp_ctx* ctx, tp_circuit* c, int which, uint64_t* out, s
  * scalar >= r) is TP_ERR_INVALID_ARG. */
 int tp_verify(tp_ctx* ctx, tp_circuit* c, const uint8_t* proof, size_t proof_len, const uint64_t* public_inputs,
               size_t n_public, int* ok);
+/* Verify `count` proofs of circuit c at once (proof.rs:195-233 for each, folded into one check).
+ * proofs: count x TP_PROOF_FIXED_BYTES, contiguous (the block tp_prove writes).
+ * public_inputs[k] / n_public[k]: proof k's public-input vector as tp_verify takes it (NULL allowed when n_public[k] == 0;
+ * public_inputs itself may be NULL when every n_public[k] is 0).
+ * *all_ok = 1 iff every proof is accepted.  each_ok (count ints, may be NULL): per-proof verdicts.
+ * count == 0 -> *all_ok = 1.  count > 65536, null pointers, n_public[k] > n, unreduced public input
+ * -> TP_ERR_INVALID_ARG.  A proof that tp_verify rejects or reports as malformed gets each_ok[k] = 0; the call still succeeds.
+ * The six KZG equations of every proof are weighted by scalars drawn from a Blake2b-512 hash of the circuit's
+ * commitments and of every proof with its public inputs (so the verdicts are a pure function of the inputs) and summed
+ * into one two-pair pairing product over two MSMs; when that check fails and each_ok is given, the failing set is
+ * halved and re-checked down to sets of 8 proofs, which get tp_verify's own host check.
+ * Stricter than tp_verify: random linear combinations are only sound in the prime-order subgroup, so every proof
+ * point is checked for [r]P = 0 and a proof with a point outside the subgroup is rejected (tp_verify checks only that
+ * the points are on the curve).  For proofs whose points are all in the subgroup, each_ok[k] equals tp_verify's
+ * verdict except with probability about 2^-250.  Device groups: as tp_verify (the MSMs are sharded by bucket). */
+int tp_verify_batch(tp_ctx* ctx, tp_circuit* c, const uint8_t* proofs, size_t count,
+                    const uint64_t* const* public_inputs, const size_t* n_public, int* all_ok, int* each_ok);
 /* The host half of tp_verify with every circuit-dependent value supplied by the caller, for verifiers that hold a
  * verification key instead of the circuit: the eight commitments, the domain size n (power of two), the coset
  * representatives k_i, sigma_1(zeta), sigma_2(zeta) and PI(zeta) for THIS proof's challenge point, [1]G (srs[0]) and

@@ -519,6 +519,24 @@ class CompiledCircuit {
                   "tp_verify", ctx_.get());
     return ok != 0;
   }
+  /// Additive API: every proof checked at once (tp_verify_batch) -> per-proof verdicts.  Stricter than verify() on
+  /// points outside the prime-order subgroup, which it rejects.
+  std::vector<bool> verify_batch(const std::vector<Proof>& proofs) const {
+    std::vector<uint8_t> blob(proofs.size() * TP_PROOF_FIXED_BYTES);
+    std::vector<const uint64_t*> pis(proofs.size());
+    std::vector<size_t> npub(proofs.size());
+    for (size_t k = 0; k < proofs.size(); k++) {
+      std::memcpy(blob.data() + k * TP_PROOF_FIXED_BYTES, proofs[k].fixed.data(), TP_PROOF_FIXED_BYTES);
+      pis[k] = proofs[k].public_inputs.empty() ? nullptr : proofs[k].public_inputs[0].limbs;
+      npub[k] = proofs[k].public_inputs.size();
+    }
+    int all_ok = 0;
+    std::vector<int> each(proofs.size());
+    detail::check(tp_verify_batch(ctx_.get(), circuit_.get(), blob.data(), proofs.size(), pis.data(), npub.data(), &all_ok,
+                                  each.data()),
+                  "tp_verify_batch", ctx_.get());
+    return std::vector<bool>(each.begin(), each.end());
+  }
   const Srs& srs() const { return *srs_; }
   tp_circuit* get() const { return circuit_.get(); }
 

@@ -244,6 +244,21 @@ static __device__ __noinline__ void xyzz_mul_small(G1Xyzz& acc, uint32_t k) {
   }
 }
 
+// [r]P == identity, r = the group order, MSB-first double-and-add in XYZZ (254 doublings + 131 mixed additions).
+static __device__ __noinline__ bool g1_in_subgroup(const G1Affine& p) {
+  const uint32_t r[8] = TP_FR_MOD;
+  G1Xyzz acc;
+  acc.x = p.x;
+  acc.y = p.y;
+  acc.zz = fq_one();
+  acc.zzz = fq_one();
+  for (int bit = 253; bit >= 0; bit--) {  // bit 254 is the leading one
+    xyzz_dbl(acc);
+    if ((r[bit >> 5] >> (bit & 31)) & 1) xyzz_madd(acc, p, false);
+  }
+  return xyzz_is_identity(acc);
+}
+
 // [0, 2q) -> [0, q): the last device step of a lazy point before it leaves the device
 __device__ __forceinline__ G1Xyzz xyzz_norm2(const G1Xyzz& a) {
   G1Xyzz r;

@@ -7,8 +7,7 @@
 // reference re-interpolates all three per call) and the eight circuit commitments (MSM, once per circuit; the
 // reference recomputes the sigma ones per call).  What is left is O(1): two hashes, ~20 G1 scalar multiplications and
 // the pairings (pairing.h), done by the calling thread.
-#include "circuit.h"
-#include "pairing.h"
+#include "verify.h"
 #include "transcript.h"
 
 #include <future>
@@ -16,13 +15,9 @@
 
 using namespace tp;
 using namespace tph;
+using namespace tpv;
 
 namespace {
-
-struct SrsPairing {
-  G2Aff g2, g2s;
-  G2Prepared pg2, pg2s;
-};
 
 // ark-serialize 0.3 uncompressed, unchecked G1 (x | y canonical LE, infinity = bit 6 of the last byte)
 bool read_g1(const uint8_t in[96], G1Aff* out) {
@@ -54,14 +49,10 @@ void abi_g1(const G1Aff& p, uint8_t out[TP_G1_BYTES]) {
   out[96] = p.inf ? 1 : 0;
 }
 
-struct ParsedProof {  // proof.rs:85-95 in the order tp_prove writes it
-  G1Aff com[4];       // a b c z
-  G1Aff wit[6];       // a b c z z-omega r
-  HFr ev[5];          // a b c z z-omega
-  HFr point, r_eval;
-  G1Aff t[3];
-  uint8_t com_abi[4][TP_G1_BYTES];
-};
+}  // namespace
+
+namespace tpv {
+
 bool parse_proof(const uint8_t* p, ParsedProof* o) {
   bool ok = true;
   for (int i = 0; i < 3; i++) {
@@ -96,6 +87,10 @@ void proof_challenges(const ParsedProof& p, HFr* alpha, HFr* beta, HFr* gamma, H
   challenges2({p.com_abi[0], p.com_abi[1], p.com_abi[2], p.com_abi[3]}, alpha, point);
 }
 
+}  // namespace tpv
+
+namespace {
+
 // kzg/src/lib.rs:66-81 as one two-pair product over the prepared SRS points
 bool kzg_check(const SrsPairing& sp, const G1Aff& identity, const G1Aff& com, const G1Aff& w, const HFr& y, const HFr& z) {
   HG1 b = g1_add(g1_from_aff(com), g1_neg(g1_mul_fr(g1_from_aff(identity), y)));  // C - y G
@@ -105,11 +100,9 @@ bool kzg_check(const SrsPairing& sp, const G1Aff& identity, const G1Aff& com, co
   return pairing_product_is_one(ps, qs, 2);
 }
 
-struct VerifierValues {
-  G1Aff fixed[5], sigma[3], identity;
-  HFr k[3], sigma_bar[2], public_eval;
-  uint64_t n;
-};
+}  // namespace
+
+namespace tpv {
 
 // proof.rs:195-233 after the device work.  KzgScheme::verify subtracts y times the prime-subgroup generator (lib.rs:77);
 // linearisation_commitment scales `identity()` = commit(1) = srs[0] (lib.rs:82-85) -- the same point for any SRS made
@@ -144,28 +137,80 @@ bool verify_host(const SrsPairing& sp, const VerifierValues& v, const ParsedProo
     return ok;
   };
   // linearisation_commitment (proof.rs:441-503)
-  const HFr a = p.ev[0], b = p.ev[1], c = p.ev[2], zw = p.ev[4];
-  auto mul = [](const G1Aff& g, const HFr& k) { return g1_mul_fr(g1_from_aff(g), k); };
-  HG1 line1 = mul(v.fixed[0], a);
-  line1 = g1_add(line1, mul(v.fixed[1], b));
-  line1 = g1_add(line1, g1_neg(mul(v.fixed[2], c)));
-  line1 = g1_add(line1, mul(v.fixed[3], a * b));
-  line1 = g1_add(line1, g1_from_aff(v.fixed[4]));
-  HFr l2 = HFr::one();
-  for (int i = 0; i < 3; i++) l2 = l2 * (p.ev[i] + beta * v.k[i] * zeta + gamma);
-  HFr zn = zeta.pow_u64(v.n), zh = zn - HFr::one();
-  HFr l0 = zeta == HFr::one() ? HFr::one() : zh * (HFr::from_u64(v.n) * (zeta - HFr::one())).inv();  // utils.rs:150-159
-  HFr alpha2 = alpha.sqr();
-  HG1 line2 = mul(p.com[3], l2 * alpha + l0 * alpha2);
-  HFr l3 = (a + beta * v.sigma_bar[0] + gamma) * (b + beta * v.sigma_bar[1] + gamma);
-  HG1 line3 = mul(v.sigma[2], l3 * alpha * beta * zw);
-  HG1 quotient = g1_add(g1_from_aff(p.t[0]), g1_add(mul(p.t[1], zn), mul(p.t[2], zn * zn)));  // utils.rs:110-126
-  HG1 line5 = g1_mul_fr(quotient, zh);
-  HFr constant = alpha * (l3 * (c + gamma) * zw) + l0 * alpha2 + v.public_eval;
-  HG1 r = g1_add(g1_add(line1, g1_add(line2, g1_neg(g1_add(line3, mul(v.identity, constant))))), g1_neg(line5));
+  HFr zh = zeta.pow_u64(v.n) - HFr::one();
+  HFr l0 = zeta == HFr::one() ? HFr::one() : zh * l0_denominator(v.n, zeta).inv();  // utils.rs:150-159
+  HFr s[LIN_TERMS];
+  lin_scalars(v, p, alpha, beta, gamma, l0, s);
+  const G1Aff* bases[LIN_TERMS] = {&v.fixed[0], &v.fixed[1], &v.fixed[2], &v.fixed[3], &v.fixed[4], &p.com[3],
+                                   &v.sigma[2], &v.identity, &p.t[0], &p.t[1], &p.t[2]};
+  HG1 r = HG1::identity();
+  for (int j = 0; j < LIN_TERMS; j++)
+    r = g1_add(r, j == LIN_QC ? g1_from_aff(*bases[j]) : g1_mul_fr(g1_from_aff(*bases[j]), s[j]));  // s[LIN_QC] = 1
   bool open_valid = kzg_check(sp, gen, g1_to_aff(r), p.wit[5], p.r_eval, zeta);
   return openings_ok() && open_valid && p.r_eval.is_zero();
 }
+
+HFr l0_denominator(uint64_t n, const HFr& zeta) { return HFr::from_u64(n) * (zeta - HFr::one()); }
+
+// proof.rs:441-503: line1 = a q_l + b q_r - c q_o + ab q_m + q_c, line2 = (l2 alpha + l0 alpha^2) z,
+// line3 = l3 alpha beta zw sigma_3, line5 = zh (t0 + zeta^n t1 + zeta^2n t2) (utils.rs:110-126),
+// r = line1 + line2 - line3 - constant identity - line5
+void lin_scalars(const VerifierValues& v, const ParsedProof& p, const HFr& alpha, const HFr& beta, const HFr& gamma,
+                 const HFr& l0, HFr s[LIN_TERMS]) {
+  const HFr zeta = p.point;
+  const HFr a = p.ev[0], b = p.ev[1], c = p.ev[2], zw = p.ev[4];
+  const HFr zero = HFr::zero();
+  s[LIN_QL] = a;
+  s[LIN_QR] = b;
+  s[LIN_QO] = zero - c;
+  s[LIN_QM] = a * b;
+  s[LIN_QC] = HFr::one();
+  HFr l2 = HFr::one();
+  for (int i = 0; i < 3; i++) l2 = l2 * (p.ev[i] + beta * v.k[i] * zeta + gamma);
+  HFr zn = zeta.pow_u64(v.n), zh = zn - HFr::one();
+  HFr alpha2 = alpha.sqr();
+  s[LIN_Z] = l2 * alpha + l0 * alpha2;
+  HFr l3 = (a + beta * v.sigma_bar[0] + gamma) * (b + beta * v.sigma_bar[1] + gamma);
+  s[LIN_S3] = zero - l3 * alpha * beta * zw;
+  HFr constant = alpha * (l3 * (c + gamma) * zw) + l0 * alpha2 + v.public_eval;
+  s[LIN_ID] = zero - constant;
+  s[LIN_T0] = zero - zh;
+  s[LIN_T1] = zero - zh * zn;
+  s[LIN_T2] = zero - zh * zn * zn;
+}
+
+int circuit_verifier_values(tp_ctx* ctx, tp_circuit* c, VerifierValues* v) {
+  // the circuit's own commitments: one batched MSM the first time
+  if (!c->have_fixed_com || !c->have_sigma_com) {
+    const Fr* sets[8] = {c->sel_coef[0], c->sel_coef[1], c->sel_coef[2], c->sel_coef[3], c->sel_coef[4],
+                         c->sig_coef[0], c->sig_coef[1], c->sig_coef[2]};
+    uint8_t outs[8][TP_G1_BYTES];
+    TP_TRY(msm_batch_dev(ctx, c->srs, sets, 8, c->n, outs));
+    memcpy(c->fixed_com, outs, sizeof(c->fixed_com));
+    memcpy(c->sigma_com, outs + 5, sizeof(c->sigma_com));
+    c->have_fixed_com = c->have_sigma_com = true;
+  }
+  for (int i = 0; i < 5; i++) v->fixed[i] = g1aff_decode(c->fixed_com[i]);
+  for (int i = 0; i < 3; i++) v->sigma[i] = g1aff_decode(c->sigma_com[i]);
+  for (int i = 0; i < 3; i++) v->k[i] = c->k[i];
+  {
+    uint8_t first[96];
+    TP_CUDA_OK(ctx, cudaMemcpyAsync(first, c->srs->g1, 96, cudaMemcpyDeviceToHost, ctx->stream));
+    TP_CUDA_OK(ctx, cudaStreamSynchronize(ctx->stream));
+    bool inf = true;
+    for (int i = 0; i < 96; i++) inf &= first[i] == 0;
+    memcpy(v->identity.x.v, first, 48);
+    memcpy(v->identity.y.v, first + 48, 48);
+    v->identity.inf = inf;
+    if (inf) v->identity = {HFq::zero(), HFq::one(), true};
+  }
+  v->n = c->n;
+  return TP_OK;
+}
+
+}  // namespace tpv
+
+namespace {
 
 int prepare_pairing(const uint8_t g2[TP_G2_BYTES], const uint8_t g2s[TP_G2_BYTES], SrsPairing* sp) {
   sp->g2 = g2_decode(g2);
@@ -318,19 +363,10 @@ int tp_verify(tp_ctx* ctx, tp_circuit* c, const uint8_t* proof, size_t proof_len
   if (!parse_proof(proof, &p)) return fail(ctx, TP_ERR_INVALID_ARG, "verify: non-canonical field element in the proof");
   if (!points_on_curve(p)) return TP_OK;
   const size_t n = c->n;
-  // the circuit's own commitments: one batched MSM the first time
-  if (!c->have_fixed_com || !c->have_sigma_com) {
-    const Fr* sets[8] = {c->sel_coef[0], c->sel_coef[1], c->sel_coef[2], c->sel_coef[3], c->sel_coef[4],
-                         c->sig_coef[0], c->sig_coef[1], c->sig_coef[2]};
-    uint8_t outs[8][TP_G1_BYTES];
-    TP_TRY(msm_batch_dev(ctx, c->srs, sets, 8, n, outs));
-    memcpy(c->fixed_com, outs, sizeof(c->fixed_com));
-    memcpy(c->sigma_com, outs + 5, sizeof(c->sigma_com));
-    c->have_fixed_com = c->have_sigma_com = true;
-  }
+  VerifierValues v;
+  TP_TRY(circuit_verifier_values(ctx, c, &v));
   // public inputs resized to n (proof.rs:204-205), interpolated, evaluated at the proof's point together with sigma_1, sigma_2
   // (the point is checked against the re-derived challenge on the host side; a mismatch rejects before these are used)
-  VerifierValues v;
   {
     size_t take = n_public < n ? n_public : n;
     TP_CUDA_OK(ctx, cudaMemsetAsync(c->pi_eval, 0, n * sizeof(Fr), ctx->stream));
@@ -346,21 +382,6 @@ int tp_verify(tp_ctx* ctx, tp_circuit* c, const uint8_t* proof, size_t proof_len
     v.sigma_bar[0] = ys[1];
     v.sigma_bar[1] = ys[2];
   }
-  for (int i = 0; i < 5; i++) v.fixed[i] = g1aff_decode(c->fixed_com[i]);
-  for (int i = 0; i < 3; i++) v.sigma[i] = g1aff_decode(c->sigma_com[i]);
-  for (int i = 0; i < 3; i++) v.k[i] = c->k[i];
-  {
-    uint8_t first[96];
-    TP_CUDA_OK(ctx, cudaMemcpyAsync(first, c->srs->g1, 96, cudaMemcpyDeviceToHost, ctx->stream));
-    TP_CUDA_OK(ctx, cudaStreamSynchronize(ctx->stream));
-    bool inf = true;
-    for (int i = 0; i < 96; i++) inf &= first[i] == 0;
-    memcpy(v.identity.x.v, first, 48);
-    memcpy(v.identity.y.v, first + 48, 48);
-    v.identity.inf = inf;
-    if (inf) v.identity = {HFq::zero(), HFq::one(), true};
-  }
-  v.n = n;
   *ok = verify_host(*(const SrsPairing*)c->srs->pairing, v, p) ? 1 : 0;
   return TP_OK;
 }

@@ -65,21 +65,6 @@ __global__ void __launch_bounds__(128) k_g1_to_wire(const G1Affine* __restrict__
   }
 }
 
-// [r]P == identity, r = the group order, MSB-first double-and-add in XYZZ (254 doublings + 131 mixed additions).
-static __device__ __noinline__ bool g1_in_subgroup(const G1Affine& p) {
-  const uint32_t r[8] = TP_FR_MOD;
-  G1Xyzz acc;
-  acc.x = p.x;
-  acc.y = p.y;
-  acc.zz = fq_one();
-  acc.zzz = fq_one();
-  for (int bit = 253; bit >= 0; bit--) {  // bit 254 is the leading one
-    xyzz_dbl(acc);
-    if ((r[bit >> 5] >> (bit & 31)) & 1) xyzz_madd(acc, p, false);
-  }
-  return xyzz_is_identity(acc);
-}
-
 // Wire records -> Montgomery SRS records, validated.  check: 0 = canonical encoding only (deserialize_unchecked),
 // 1 = + on the curve, 2 = + in the prime-order subgroup (what ark-ec's checked deserialisation enforces).
 // bad[0] counts rejected records, bad[1] keeps the lowest rejected index + 1.

@@ -31,7 +31,7 @@ SYMBOLS = [
     "tp_commit", "tp_commit_dev", "tp_open", "tp_ntt", "tp_ntt_dev", "tp_perm_prove",
     "tp_circuit_load", "tp_circuit_compile", "tp_circuit_destroy", "tp_circuit_sigma_commitments",
     "tp_prove", "tp_prove_dev", "tp_prove_inputs", "tp_measure_imad_peak", "tp_selftest", "tp_fr_rand_stream", "tp_ctx_set_option", "tp_ctx_get_stat",
-    "tp_srs_g2", "tp_srs_set_g2", "tp_kzg_verify", "tp_pairing_check", "tp_verify", "tp_verify_prepared", "tp_proof_challenges",
+    "tp_srs_g2", "tp_srs_set_g2", "tp_kzg_verify", "tp_pairing_check", "tp_verify", "tp_verify_batch", "tp_verify_prepared", "tp_proof_challenges",
     "tp_trace_create", "tp_trace_destroy", "tp_trace_gate", "tp_trace_gates", "tp_trace_assert_eq", "tp_trace_finish",
     "tp_trace_gate_kinds", "tp_trace_selectors", "tp_trace_permutation", "tp_trace_witness",
     "tp_permutation_builder_create", "tp_permutation_builder_destroy", "tp_permutation_builder_add_row",
@@ -608,6 +608,23 @@ class CircuitHandle:
                                         _buf(public_inputs_mont) if public_inputs_mont else None,
                                         C.c_size_t(len(public_inputs_mont) // 32), C.byref(ok)))
         return bool(ok.value)
+
+    def verify_batch(self, proofs_fixed, public_inputs):
+        """tp_verify_batch: proofs_fixed[k] is proof k's 1472-byte block, public_inputs[k] its public-input vector as
+        Montgomery bytes (b"" = none).  Returns (every proof accepted, per-proof verdicts)."""
+        count = len(proofs_fixed)
+        assert len(public_inputs) == count
+        if any(len(p) != PROOF_FIXED_BYTES for p in proofs_fixed):
+            raise TyplonkError(1, "verify_batch: every proof must be a %d-byte block" % PROOF_FIXED_BYTES)
+        blob = b"".join(proofs_fixed)
+        keep = [(C.c_char * len(b)).from_buffer_copy(b) if b else None for b in public_inputs]
+        pis = (C.c_void_p * max(count, 1))(*[C.cast(b, C.c_void_p) if b is not None else None for b in keep])
+        npub = (C.c_size_t * max(count, 1))(*[len(b) // 32 for b in public_inputs])
+        each = (C.c_int * max(count, 1))()
+        all_ok = C.c_int(0)
+        self.ctx._check(lib().tp_verify_batch(self.ctx._h, self._h, _buf(blob) if count else None, C.c_size_t(count),
+                                              pis, npub, C.byref(all_ok), each))
+        return bool(all_ok.value), [bool(each[k]) for k in range(count)]
 
     POLY_QUOTIENT, POLY_LINEARISATION, POLY_Z_EVALS, POLY_Z, POLY_A, POLY_B, POLY_C = range(7)
 

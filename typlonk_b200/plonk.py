@@ -116,6 +116,11 @@ class CompiledCircuit:
         """CompiledCircuit::verify (proof.rs:59-63, 195-233)."""
         return self.handle.verify(proof.fixed, F.fr_vec_to_bytes(proof.public_inputs))
 
+    def verify_batch(self, proofs: List[Proof]):
+        """Every proof of this circuit checked at once (tp_verify_batch): (all accepted, per-proof verdicts).  Stricter
+        than `verify` on points outside the prime-order subgroup, which it rejects."""
+        return self.handle.verify_batch([p.fixed for p in proofs], [F.fr_vec_to_bytes(p.public_inputs) for p in proofs])
+
 
 class CircuitDescription:
     """description.rs:4-9."""
