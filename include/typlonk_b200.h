@@ -122,7 +122,8 @@ int tp_ctx_group_size(const tp_ctx* ctx, int* ndev, int* uses_nccl);
 int tp_ctx_set_option(tp_ctx* ctx, const char* name, long value);
 /* Work counters since the last tp_prof_reset: "msm_entries" (bucket additions issued by the accumulation
  * kernels), "msm_calls"; and the plan of the last MSM: "msm_window_bits", "msm_windows", "msm_table_levels",
- * "msm_chunk".  Unknown names fail with TP_ERR_INVALID_ARG. */
+ * "msm_chunk"; "prove_batch_wave": the proofs per wave of the last tp_prove_batch.  Unknown names fail with
+ * TP_ERR_INVALID_ARG. */
 int tp_ctx_get_stat(tp_ctx* ctx, const char* name, double* out);
 
 /* Per-phase device timers (CUDA events on the ctx stream).  Phase ids: TP_PHASE_*. */
@@ -232,6 +233,26 @@ int tp_prove_dev(tp_ctx* ctx, tp_circuit* c, const void* const advice_dev[3], co
  * vectors the reference can prove, SURVEY.md App. D.1) the prover skips that polynomial's transforms. */
 int tp_prove_inputs(tp_ctx* ctx, tp_circuit* c, const uint64_t* const advice[3], const uint64_t* public_inputs,
                     size_t n_public, uint8_t* proof_out, size_t proof_cap);
+/* Prove `count` witnesses of circuit c in one call: tp_prove_inputs for each, with the MSMs, NTTs and scans of
+ * all proofs batched and one host round trip per stage for the whole batch.
+ * advice: 3 * count host column pointers, advice[3k + i] = column i of proof k (n Montgomery Fr, blinders in place).
+ * public_inputs[k] / n_public[k]: as tp_prove_inputs takes them (NULL allowed when n_public[k] == 0;
+ *   public_inputs may be NULL when every n_public[k] is 0).
+ * proofs_out: count x TP_PROOF_FIXED_BYTES; block k is byte-identical to what tp_prove_inputs writes for proof k.
+ * status (count ints, may be NULL): status[k] = what tp_prove_inputs returns for proof k (TP_OK,
+ *   TP_ERR_GATE_UNSATISFIED, TP_ERR_ZERO_DENOMINATOR); block k is zero-filled when it is not TP_OK and the call
+ *   still returns TP_OK.  With status == NULL the call returns the lowest-index failure's code (index in
+ *   tp_last_error); the other blocks are written as above.
+ * count == 0 -> TP_OK.  count > 65536, null pointers, n_public[k] > n -> TP_ERR_INVALID_ARG;
+ * proofs_cap < count * TP_PROOF_FIXED_BYTES -> TP_ERR_BUFFER_TOO_SMALL.
+ * The proofs run in waves of W at a time (tp_ctx_get_stat "prove_batch_wave"): W is at most 64 and as many as fit
+ * half of the free device memory, at least 1; each proof of a wave needs 44n + 1 Fr of device buffers, which the
+ * circuit keeps (they only grow) until tp_circuit_destroy.  The circuit's own buffers -- what
+ * tp_circuit_read_poly shows -- are left untouched.  Device groups: every rank runs the batch, the MSMs are sharded
+ * by bucket, everything else is replicated. */
+int tp_prove_batch(tp_ctx* ctx, tp_circuit* c, size_t count, const uint64_t* const* advice,
+                   const uint64_t* const* public_inputs, const size_t* n_public,
+                   uint8_t* proofs_out, size_t proofs_cap, int* status);
 
 /* Inspection: an intermediate polynomial of the LAST proof made with `c`, read from the prover's device buffers
  * (Montgomery Fr): the quotient t as 3n coefficients (quotient_polynomial, proof.rs:292-375; slices t0 | t1 | t2), the

@@ -511,6 +511,36 @@ class CompiledCircuit {
     for (auto& x : blinders) x = Fr::random();
     return prove(inputs, public_inputs, blinders);
   }
+  /// Many proofs in one call (tp_prove_batch): proof k equals prove(inputs[k], public_inputs[k], blinders[k]).  Throws
+  /// what prove() would throw for the first failing proof; tp_last_error names its index.
+  std::vector<Proof> prove_batch(const std::vector<std::array<Fr, INPUTS>>& inputs, const std::vector<std::vector<Fr>>& public_inputs,
+                                 const std::vector<std::array<Fr, 9>>& blinders) const {
+    const size_t count = inputs.size();
+    if (public_inputs.size() != count || blinders.size() != count)
+      throw Error(TP_ERR_INVALID_ARG, "prove_batch: inputs, public inputs and blinders differ in count");
+    std::vector<Fr> cols(3 * count * rows);
+    std::vector<const uint64_t*> adv(3 * count);
+    std::vector<const uint64_t*> pis(count);
+    std::vector<size_t> npub(count);
+    for (size_t k = 0; k < count; k++) {
+      if (public_inputs[k].size() > rows) throw Error(TP_ERR_INVALID_ARG, "prove_batch: more public inputs than rows");
+      uint64_t* a[3];
+      for (int i = 0; i < 3; i++) adv[3 * k + i] = a[i] = cols[(3 * k + i) * rows].limbs;
+      detail::check(tp_trace_witness(trace_.get(), INPUTS ? inputs[k][0].limbs : nullptr, INPUTS, blinders[k][0].limbs, a), "tp_trace_witness");
+      pis[k] = public_inputs[k].empty() ? nullptr : public_inputs[k][0].limbs;
+      npub[k] = public_inputs[k].size();
+    }
+    std::vector<uint8_t> blob(count * TP_PROOF_FIXED_BYTES);
+    detail::check(tp_prove_batch(ctx_.get(), circuit_.get(), count, adv.data(), pis.data(), npub.data(), blob.data(), blob.size(), nullptr),
+                  "tp_prove_batch", ctx_.get());
+    std::vector<Proof> out(count);
+    for (size_t k = 0; k < count; k++) {
+      std::memcpy(out[k].fixed.data(), blob.data() + k * TP_PROOF_FIXED_BYTES, TP_PROOF_FIXED_BYTES);
+      out[k].public_inputs = public_inputs[k];
+      out[k].public_inputs.resize(rows);
+    }
+    return out;
+  }
   /// CompiledCircuit::verify (proof.rs:59-63, 195-233).  A malformed proof throws; a wrong one returns false.
   bool verify(const Proof& proof) const {
     int ok = 0;

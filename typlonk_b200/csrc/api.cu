@@ -4,8 +4,7 @@
 // plonk/src/builder.rs:70-88.  The host only sequences kernels, derives the Fiat-Shamir
 // challenges (transcript.h) and does the O(1) scalar algebra between rounds.
 #include "common.cuh"
-#include "circuit.h"
-#include "transcript.h"
+#include "prove.h"
 
 using namespace tp;
 using tph::HFr;
@@ -124,6 +123,11 @@ int tp_ctx_destroy(tp_ctx* ctx) {
   for (auto* b : bufs) release(*b);
   for (auto& b : ctx->scan_tmp) release(b);
   for (auto& b : ctx->misc) release(b);
+  for (int s = 0; s < TP_PARAM_SLOTS; s++) {
+    release(ctx->param_dev[s]);
+    if (ctx->param_host[s]) cudaFreeHost(ctx->param_host[s]);
+    if (ctx->param_ev[s]) cudaEventDestroy(ctx->param_ev[s]);
+  }
   for (auto e : ctx->event_pool) cudaEventDestroy(e);
   for (auto& p : ctx->pending) {
     cudaEventDestroy(p.a);
@@ -201,7 +205,8 @@ int tp_ctx_get_stat(tp_ctx* ctx, const char* name, double* out) {
   if (is_group(ctx)) return on_rank0(ctx, [&](tp_ctx* c) { return tp_ctx_get_stat(c, name, out); });
   const struct { const char* n; double v; } stats[] = {
       {"msm_entries", ctx->stat_msm_entries}, {"msm_calls", ctx->stat_msm_calls}, {"msm_window_bits", ctx->stat_msm_c},
-      {"msm_windows", ctx->stat_msm_nwin},    {"msm_table_levels", ctx->stat_msm_levels}, {"msm_chunk", ctx->stat_msm_chunk}};
+      {"msm_windows", ctx->stat_msm_nwin},    {"msm_table_levels", ctx->stat_msm_levels}, {"msm_chunk", ctx->stat_msm_chunk},
+      {"prove_batch_wave", ctx->stat_prove_batch_wave}};
   for (auto& st : stats)
     if (strcmp(name, st.n) == 0) {
       *out = st.v;
@@ -559,6 +564,7 @@ int tp_circuit_destroy(tp_ctx* ctx, tp_circuit* c) {
   }
   cudaStreamSynchronize(ctx->stream);
   for (void* p : c->allocs) cudaFree(p);
+  if (c->wave) cudaFree(c->wave);
   delete c;
   return TP_OK;
 }
@@ -694,16 +700,6 @@ int tp_circuit_sigma_commitments(tp_ctx* ctx, tp_circuit* c, uint8_t out[3 * TP_
 }
 
 // ---- prover -----------------------------------------------------------------------------------
-static void put_g1(uint8_t*& w, const uint8_t pt[TP_G1_BYTES]) {
-  tph::serialize_g1_unchecked(pt, w);
-  w += 96;
-}
-static void put_fr(uint8_t*& w, const HFr& x) {
-  HFr c = x.from_mont();
-  memcpy(w, c.v, 32);
-  w += 32;
-}
-
 // The prover's second stream: the forward coset NTTs of the quotient do not depend on any Fiat-Shamir challenge, so they
 // are queued here as soon as their polynomial exists and run underneath the commitment MSMs of the main stream -- above
 // all during the latency-bound tail of each MSM (bucket reduction, host round trip), when most SMs are idle.
@@ -733,7 +729,7 @@ static int prove_resident(tp_ctx* ctx, tp_circuit* c, uint8_t* proof_out, const 
   static const bool no_side_stream = getenv("TP_NO_SIDE_STREAM") && *getenv("TP_NO_SIDE_STREAM") == '1';
   const bool shard = comm_ready(ctx) && !no_coset_shard;
   HFr gens[4];
-  for (unsigned k = 0; k < 4; k++) gens[k] = omega_for_log(c->log_n + 2).pow_u64(k);
+  tpp::coset_gens(c->log_n, gens);
   bool have[4][4] = {{false}};   // have[poly][coset]: evaluations of poly (a, b, c, z) on coset k are in buf4[poly]
   auto queue_cosets = [&](int poly_lo, int poly_hi, unsigned first) -> int {
     const Fr* src[4] = {c->adv_coef[0], c->adv_coef[1], c->adv_coef[2], c->z_coef};
@@ -781,11 +777,12 @@ static int prove_resident(tp_ctx* ctx, tp_circuit* c, uint8_t* proof_out, const 
   // needs nothing but the uploaded columns and also tells whether the public inputs are all zero.
   bool pi_zero = false;
   {
-    bool ok = false;
+    unsigned flags = 0;
     const Fr* sel[5] = {c->sel_eval[0], c->sel_eval[1], c->sel_eval[2], c->sel_eval[3], c->sel_eval[4]};
     const Fr* adv[3] = {c->adv_eval[0], c->adv_eval[1], c->adv_eval[2]};
-    TP_TRY(gate_check_dev(ctx, sel, adv, c->pi_eval, n, &ok, &pi_zero));
-    if (!ok) return fail(ctx, TP_ERR_GATE_UNSATISFIED, "prove: gate constraints do not vanish on the domain");
+    TP_TRY(gate_check_dev(ctx, sel, adv, c->pi_eval, n, 0, 1, &flags));
+    pi_zero = (flags & 2u) == 0;
+    if (flags & 1u) return fail(ctx, TP_ERR_GATE_UNSATISFIED, "prove: gate constraints do not vanish on the domain");
   }
   // A zero public-input vector (the only kind the reference's prover accepts, SURVEY.md App. D.1) interpolates to the
   // zero polynomial: its inverse NTT, its four coset NTTs and its evaluation are skipped and the buffers just hold zeros.
@@ -879,18 +876,20 @@ static int prove_resident(tp_ctx* ctx, tp_circuit* c, uint8_t* proof_out, const 
     for (int i = 0; i < 3; i++) {
       qa.sig4[i] = c->sig4[i];
       qa.adv4[i] = c->buf4[i];
-      qa.k[i] = to_dev(c->k[i]);
+      qa.k[i] = c->k[i];
     }
     qa.z4 = c->buf4[3];
     qa.pi4 = c->buf4[4];
     qa.l0_4 = c->l0_4;
     TP_TRY(ntt_get_twiddles(ctx, c->log_n + 2, &qa.tw4));
-    qa.alpha = to_dev(alpha);
-    qa.beta = to_dev(beta);
-    qa.gamma = to_dev(gamma);
+    qa.count = 1;
+    qa.stride = 0;
+    qa.alpha = &alpha;
+    qa.beta = &beta;
+    qa.gamma = &gamma;
     qa.out = c->buf4[5];
     qa.n = n;
-    TP_TRY(quotient_numerator_dev(ctx, qa, mine, nmine));
+    TP_TRY(quotient_numerator_dev(ctx, qa, mine, nmine));   // proof 0: the items are the cosets themselves
     {
       // out of place into the (now dead) coset slots of buf4[0]; the interpolants are gathered there
       const Fr* ins[4];
@@ -908,7 +907,7 @@ static int prove_resident(tp_ctx* ctx, tp_circuit* c, uint8_t* proof_out, const 
       for (unsigned k = first; k < 4; k++) TP_TRY(comm_bcast(ctx, c->buf4[0] + (size_t)k * n, n * sizeof(Fr), owner(k)));
       TP_TRY(comm_group_end(ctx));
     }
-    TP_TRY(quotient_combine_dev(ctx, c->buf4[0], n, skip0, c->t));
+    TP_TRY(quotient_combine_dev(ctx, c->buf4[0], n, 0, 1, &skip0, c->t));
   }
 
   // The three t commitments (proof.rs:175,181) need nothing that follows: with the MSM pipe they are queued now and
@@ -921,11 +920,10 @@ static int prove_resident(tp_ctx* ctx, tp_circuit* c, uint8_t* proof_out, const 
   }
   // openings (proof.rs:147-163)
   uint8_t wit[6][TP_G1_BYTES];
-  HFr ev[5];
+  tpp::ProofEvals pe;
   HFr omega = omega_for_log(c->log_n);
   // ... together with the three plain evaluations the linearisation needs (proof.rs:416,429): eight
   // recurrences of length n in one batched scan, one read-back.
-  HFr sig_bar[2], pi_bar;
   {
     const Fr* polys[8] = {c->adv_coef[0], c->adv_coef[1], c->adv_coef[2], c->z_coef, c->z_coef,
                           c->sig_coef[0], c->sig_coef[1], c->pi_coef};
@@ -934,43 +932,24 @@ static int prove_resident(tp_ctx* ctx, tp_circuit* c, uint8_t* proof_out, const 
     for (int i = 0; i < 8; i++) points[i] = to_dev(i == 4 ? zeta * omega : zeta);
     HFr ys[8];
     TP_TRY(poly_open_batch_dev(ctx, polys, n, points, quots, pi_zero ? 7 : 8, ys));
-    for (int i = 0; i < 5; i++) ev[i] = ys[i];
-    sig_bar[0] = ys[5];
-    sig_bar[1] = ys[6];
-    pi_bar = pi_zero ? HFr::zero() : ys[7];
+    for (int i = 0; i < 5; i++) pe.ev[i] = ys[i];
+    pe.sig_bar[0] = ys[5];
+    pe.sig_bar[1] = ys[6];
+    pe.pi_bar = pi_zero ? HFr::zero() : ys[7];
   }
   if (piped) {
     const Fr* sets[5] = {c->q[0], c->q[1], c->q[2], c->q[3], c->q[4]};
     TP_TRY(msm_pipe_submit(ctx, srs, sets, 5, n));
   }
   // linearisation (proof.rs:376-439)
-  HFr a = ev[0], b = ev[1], cc = ev[2], zw = ev[4];
-  HFr l2 = HFr::one();
-  for (int i = 0; i < 3; i++) l2 = l2 * (ev[i] + c->k[i] * beta * zeta + gamma);
-  HFr perm_ab = (a + beta * sig_bar[0] + gamma) * (b + beta * sig_bar[1] + gamma);
-  HFr zn = zeta.pow_u64((uint64_t)n);
-  HFr zh = zn - HFr::one();
-  HFr l0;
-  if (zeta == HFr::one()) {
-    l0 = HFr::one();
-  } else {
-    l0 = zh * (HFr::from_u64((uint64_t)n) * (zeta - HFr::one())).inv();
+  {
+    HFr s[tpp::R_TERMS + 1];
+    tpp::lin_scalars(c->k, pe, alpha, beta, gamma, zeta, n, s);
+    const LinTerm terms[tpp::R_TERMS] = {{c->sel_coef[0], 0}, {c->sel_coef[1], 0}, {c->sel_coef[2], 0},
+                                         {c->sel_coef[3], 0}, {c->sel_coef[4], 0}, {c->z_coef, 0},
+                                         {c->sig_coef[2], 0}, {c->t, 0}, {c->t + n, 0}, {c->t + 2 * n, 0}};
+    TP_TRY(lincomb_dev(ctx, terms, tpp::R_TERMS, s, n, 1, c->r, 0));
   }
-  HFr alpha2 = alpha.sqr();
-  HFr ab_zw = alpha * perm_ab * zw;
-  LinTerm terms[10];
-  terms[0] = {c->sel_coef[0], to_dev(a)};
-  terms[1] = {c->sel_coef[1], to_dev(b)};
-  terms[2] = {c->sel_coef[2], to_dev(cc.neg())};
-  terms[3] = {c->sel_coef[3], to_dev(a * b)};
-  terms[4] = {c->sel_coef[4], to_dev(HFr::one())};
-  terms[5] = {c->z_coef, to_dev(alpha * l2 + alpha2 * l0)};
-  terms[6] = {c->sig_coef[2], to_dev((ab_zw * beta).neg())};
-  terms[7] = {c->t, to_dev(zh.neg())};
-  terms[8] = {c->t + n, to_dev((zh * zn).neg())};
-  terms[9] = {c->t + 2 * n, to_dev((zh * zn * zn).neg())};
-  HFr constant = pi_bar - ab_zw * (gamma + cc) - alpha2 * l0;
-  TP_TRY(lincomb_dev(ctx, terms, 10, to_dev(constant), n, c->r));
   HFr r_bar;
   TP_TRY(poly_open_dev(ctx, c->r, n, to_dev(zeta), c->q[5], &r_bar));
   // the six opening witnesses and the three t commitments (proof.rs:149,162,163,175,181) are
@@ -991,21 +970,7 @@ static int prove_resident(tp_ctx* ctx, tp_circuit* c, uint8_t* proof_out, const 
     for (int i = 0; i < 3; i++) memcpy(tcom[i], outs[6 + i], TP_G1_BYTES);
   }
 
-  uint8_t* w = proof_out;
-  for (int i = 0; i < 3; i++) {
-    put_g1(w, com[i]);
-    put_g1(w, wit[i]);
-    put_fr(w, ev[i]);
-  }
-  put_g1(w, com[3]);
-  put_g1(w, wit[3]);
-  put_fr(w, ev[3]);
-  put_g1(w, wit[4]);
-  put_fr(w, ev[4]);
-  put_fr(w, zeta);
-  for (int i = 0; i < 3; i++) put_g1(w, tcom[i]);
-  put_g1(w, wit[5]);
-  put_fr(w, r_bar);
+  tpp::write_proof(proof_out, com, wit, tcom, pe.ev, zeta, r_bar);
   return TP_OK;
 }
 

@@ -32,6 +32,9 @@ struct tp_circuit {
   // skips that polynomial's six transforms
   bool pi_buffers_zero = false;
   std::vector<void*> allocs;
+  // tp_prove_batch (prove_batch.cu): the per-proof buffers of `wave_cap` proofs, grown on demand, freed with the circuit
+  tp::Fr* wave = nullptr;
+  size_t wave_cap = 0;
   std::vector<tp_circuit*> parts;  // circuit of a device group: one per rank (n and log_n are set, nothing else)
   // verifier state (verify.cu): the eight commitments of the circuit itself, computed on first use and kept
   // (the reference recomputes the sigma commitments in every verify, permutation/src/lib.rs:180-194)

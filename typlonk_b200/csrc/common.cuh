@@ -36,6 +36,8 @@ struct CosetTable {
 
 }  // namespace tp
 
+#define TP_PARAM_SLOTS 8
+
 struct tp_ctx {
   int device = 0;
   cudaStream_t stream = nullptr;
@@ -97,6 +99,14 @@ struct tp_ctx {
   cudaEvent_t side_ev[4] = {nullptr, nullptr, nullptr, nullptr};
   cudaStream_t copy_stream = nullptr;
   cudaEvent_t copy_ev[4] = {nullptr, nullptr, nullptr, nullptr};  // [0..2] column landed, [3] compute stream reached the upload
+  // kernel parameter blocks (poly.cu params_upload): pinned staging, device copy and copy-done event per ring slot
+  void* param_host[TP_PARAM_SLOTS] = {nullptr};
+  size_t param_host_cap[TP_PARAM_SLOTS] = {0};
+  tp::DevBuf param_dev[TP_PARAM_SLOTS];
+  cudaEvent_t param_ev[TP_PARAM_SLOTS] = {nullptr};
+  unsigned param_next = 0;
+  // last tp_prove_batch: proofs per wave (tp_ctx_get_stat "prove_batch_wave")
+  double stat_prove_batch_wave = 0;
 };
 
 struct tp_srs {
@@ -241,39 +251,55 @@ int msm_pipe_finish(tp_ctx* ctx, uint8_t (*out)[TP_G1_BYTES], int count);
 bool msm_pipe_overlaps(const tp_ctx* ctx, size_t len);
 void msm_pipe_destroy(tp_ctx* ctx);
 // poly.cu
+// `bytes` of kernel parameters copied to the device in stream order; *dev stays valid for the launches queued next
+int params_upload(tp_ctx* ctx, const void* src, size_t bytes, const void** dev);
+// Several device entry points below work on `count` proofs at once: proof p's per-proof arrays sit at the given base
+// pointer + p * stride (in Fr), circuit arrays are shared.  tp_prove calls them with count 1.
 int perm_grand_product_dev(tp_ctx* ctx, const Fr* const values[3], const Fr* const id[3], const Fr* const sigma[3],
                            size_t n, const Fr& beta, const Fr& gamma, Fr* out /* n+1 */, bool* closes = nullptr);
 // *closes (may be null): out[n] == 1, i.e. the copy constraints hold on the witness
+// zero_den[p]: proof p has a zero denominator (its out is left undefined); closes[p] (may be null) as above
+int perm_grand_product_batch_dev(tp_ctx* ctx, const Fr* const values[3], size_t vstride, const Fr* const id[3],
+                                 const Fr* const sigma[3], size_t n, int count, const tph::HFr* beta,
+                                 const tph::HFr* gamma, Fr* out, size_t ostride, bool* zero_den, bool* closes);
 // q[k-1] = p[k] + z q[k]; writes q (len-1 coeffs, then a zero at [len-1]) and returns y = p(z)
 int poly_open_dev(tp_ctx* ctx, const Fr* p, size_t len, const Fr& z, Fr* q_out /* len, may be null */, tph::HFr* y);
-// up to 8 polynomials of the same length at once (own point each; q_out[b] may be null = evaluation only)
+// any number of polynomials of the same length at once (own point each; q_out[b] may be null = evaluation only)
 int poly_open_batch_dev(tp_ctx* ctx, const Fr* const* p, size_t len, const Fr* z, Fr* const* q_out, int batch, tph::HFr* y);
-// *ok: the gate equation holds on every row; *pi_is_zero (may be null): every public input is zero
+// flags[p] bit 0: the gate equation fails on some row of proof p; bit 1: some public input of proof p is non-zero
 int gate_check_dev(tp_ctx* ctx, const Fr* const sel_evals[5], const Fr* const adv[3], const Fr* pi, size_t n,
-                   bool* ok, bool* pi_is_zero);
+                   size_t stride, int count, unsigned* flags);
 struct QuotientArgs {   // every 4n-sized array is coset-major: slot k * n + i <-> omega_4n^(4i + k)
   const Fr* sel4[5];   // 4n evaluations
   const Fr* sig4[3];
-  const Fr* adv4[3];
-  const Fr* z4;
-  const Fr* pi4;
   const Fr* l0_4;      // L0 on the 4n domain
   const Fr* tw4;       // omega_4n^i, i in [0, 2n]
-  Fr alpha, beta, gamma;
-  Fr k[3];
+  const Fr* adv4[3];   // per proof (+ p * stride)
+  const Fr* z4;
+  const Fr* pi4;
   Fr* out;             // 4n numerator evaluations
+  size_t stride;
+  int count;
+  const tph::HFr* alpha;   // host, count each
+  const tph::HFr* beta;
+  const tph::HFr* gamma;
+  tph::HFr k[3];
   size_t n;
 };
-int quotient_numerator_dev(tp_ctx* ctx, const QuotientArgs& a, const unsigned* cosets, int ncosets);
+// items[j] = proof << 2 | coset: one launch over every listed (proof, coset) pair
+int quotient_numerator_dev(tp_ctx* ctx, const QuotientArgs& a, const unsigned* items, int nitems);
 // t = floor(N / (X^n - 1)) (3n coefficients) from the four per-coset interpolants of N (coset-major, 4n)
-// c0_is_zero: coset 0 (H itself) was skipped because the numerator is known to vanish there
-int quotient_combine_dev(tp_ctx* ctx, const Fr* c4, size_t n, bool c0_is_zero, Fr* t /* 3n */);
+// c0_is_zero[p]: coset 0 (H itself) of proof p was skipped because its numerator is known to vanish there
+int quotient_combine_dev(tp_ctx* ctx, const Fr* c4, size_t n, size_t stride, int count, const bool* c0_is_zero,
+                         Fr* t /* 3n */);
 int l0_evals_4n_dev(tp_ctx* ctx, const Fr* tw4, size_t n, Fr* out /* 4n */);
 struct LinTerm {
   const Fr* p;
-  Fr s;
+  size_t stride;   // 0: shared by every proof
 };
-int lincomb_dev(tp_ctx* ctx, const LinTerm* terms, int nterms, const Fr& constant, size_t n, Fr* out);
+// out + p * ostride = scalars[p * (nterms + 1) + nterms] (at coefficient 0) + sum_t scalars[p * (nterms + 1) + t] * term t
+int lincomb_dev(tp_ctx* ctx, const LinTerm* terms, int nterms, const tph::HFr* scalars, size_t n, int count, Fr* out,
+                size_t ostride);
 int sigma_tables_dev(tp_ctx* ctx, const uint64_t* perm_dev, size_t n, const Fr* tw, const Fr k[3], Fr* id[3],
                      Fr* sigma[3]);
 int pad_copy_dev(tp_ctx* ctx, const Fr* in, size_t len, Fr* out, size_t out_len);

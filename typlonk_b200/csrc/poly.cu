@@ -22,6 +22,29 @@ __device__ __forceinline__ Fr pmul(const Fr& a, const Fr& b) { return fr_mul(a, 
 #endif
 
 
+// Small per-launch parameter blocks (per-proof scalars, item lists, pointer tables) go through a ring of pinned staging
+// blocks, each copied in stream order to a device block of its own.  A staging block is written again only after the
+// copy out of it has run, which the stream has long done by then (every stage of a proof ends in a host read-back).
+int params_upload(tp_ctx* ctx, const void* src, size_t bytes, const void** dev) {
+  const unsigned s = ctx->param_next++ % TP_PARAM_SLOTS;
+  if (!ctx->param_ev[s]) TP_CUDA_OK(ctx, cudaEventCreateWithFlags(&ctx->param_ev[s], cudaEventDisableTiming));
+  TP_CUDA_OK(ctx, cudaEventSynchronize(ctx->param_ev[s]));
+  if (ctx->param_host_cap[s] < bytes) {
+    if (ctx->param_host[s]) cudaFreeHost(ctx->param_host[s]);
+    ctx->param_host[s] = nullptr;
+    ctx->param_host_cap[s] = 0;
+    const size_t want = bytes < 4096 ? 4096 : bytes;
+    TP_CUDA_OK(ctx, cudaMallocHost(&ctx->param_host[s], want));
+    ctx->param_host_cap[s] = want;
+  }
+  TP_TRY(ensure(ctx, ctx->param_dev[s], bytes));
+  memcpy(ctx->param_host[s], src, bytes);
+  TP_CUDA_OK(ctx, cudaMemcpyAsync(ctx->param_dev[s].p, ctx->param_host[s], bytes, cudaMemcpyHostToDevice, ctx->stream));
+  TP_CUDA_OK(ctx, cudaEventRecord(ctx->param_ev[s], ctx->stream));
+  *dev = ctx->param_dev[s].p;
+  return TP_OK;
+}
+
 #define EW_THREADS 256
 static inline unsigned ew_grid(size_t n) { return (unsigned)((n + EW_THREADS - 1) / EW_THREADS); }
 
@@ -31,15 +54,19 @@ static inline unsigned ew_grid(size_t n) { return (unsigned)((n + EW_THREADS - 1
 #define SCAN_CH 32
 #define SCAN_BASE 64
 
-// two independent scans of the same length side by side (blockIdx.y picks the array): the upper levels of a scan are
-// chains of small launches, so two cost what one costs
+// 2 * count independent scans of the same length side by side (blockIdx.y = 2 * proof + which): the upper levels of a
+// scan are chains of small launches, so the two scans of every proof of a batch cost what one costs.  Scan (proof p,
+// which w) runs over a[w] + p * stride; its chunk totals go to tot[w] + p * tot_stride.
 struct ScanPair {
   Fr* a[2];
   Fr* tot[2];
+  size_t stride, tot_stride;
+  __device__ __forceinline__ Fr* arr(unsigned y) const { return ((y & 1) ? a[1] : a[0]) + (size_t)(y >> 1) * stride; }
+  __device__ __forceinline__ Fr* tots(unsigned y) const { return ((y & 1) ? tot[1] : tot[0]) + (size_t)(y >> 1) * tot_stride; }
 };
 __global__ void k_mulscan2_serial(ScanPair p, size_t n) {   // exclusive
   if (threadIdx.x != 0) return;
-  Fr* a = p.a[blockIdx.x];
+  Fr* a = p.arr(blockIdx.x);
   Fr acc = fr_one();
   for (size_t i = 0; i < n; i++) {
     Fr x = fr_load(a + i);
@@ -51,7 +78,7 @@ __global__ void k_mulscan2_chunk(ScanPair p, size_t n) {    // exclusive
   size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   size_t lo = t * SCAN_CH;
   if (lo >= n) return;
-  Fr* a = p.a[blockIdx.y];
+  Fr* a = p.arr(blockIdx.y);
   size_t hi = lo + SCAN_CH < n ? lo + SCAN_CH : n;
   Fr acc = fr_one();
   for (size_t i = lo; i < hi; i++) {
@@ -59,35 +86,38 @@ __global__ void k_mulscan2_chunk(ScanPair p, size_t n) {    // exclusive
     fr_store(a + i, acc);
     acc = fr_mul(acc, x);
   }
-  fr_store(p.tot[blockIdx.y] + t, acc);
+  fr_store(p.tots(blockIdx.y) + t, acc);
 }
 __global__ void k_mulscan2_apply(ScanPair p, size_t n) {
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   size_t ch = i / SCAN_CH;
   if (ch == 0) return;
-  Fr* a = p.a[blockIdx.y];
-  fr_store(a + i, fr_mul(fr_load(a + i), fr_load(p.tot[blockIdx.y] + ch)));
+  Fr* a = p.arr(blockIdx.y);
+  fr_store(a + i, fr_mul(fr_load(a + i), fr_load(p.tots(blockIdx.y) + ch)));
 }
-// exclusive prefix products of a0[0..n) and a1[0..n), in place
-static int mulscan2_exclusive(tp_ctx* ctx, Fr* a0, Fr* a1, size_t n, int level) {
+// exclusive prefix products of a0 + p * stride and a1 + p * stride over [0, n), p < count, in place
+static int mulscan2_exclusive(tp_ctx* ctx, Fr* a0, Fr* a1, size_t stride, int count, size_t n, int level) {
   ScanPair p;
   p.a[0] = a0;
   p.a[1] = a1;
+  p.stride = stride;
   p.tot[0] = p.tot[1] = nullptr;
+  p.tot_stride = 0;
   if (n <= SCAN_BASE) {
-    k_mulscan2_serial<<<2, 32, 0, ctx->stream>>>(p, n);
+    k_mulscan2_serial<<<2 * count, 32, 0, ctx->stream>>>(p, n);
     TP_LAUNCH(ctx, "k_mulscan2_serial");
     return TP_OK;
   }
   size_t nch = (n + SCAN_CH - 1) / SCAN_CH;
-  TP_TRY(ensure(ctx, ctx->scan_tmp[level], 2 * nch * sizeof(Fr)));
+  TP_TRY(ensure(ctx, ctx->scan_tmp[level], 2 * nch * (size_t)count * sizeof(Fr)));
   p.tot[0] = (Fr*)ctx->scan_tmp[level].p;
   p.tot[1] = p.tot[0] + nch;
-  k_mulscan2_chunk<<<dim3(ew_grid(nch), 2), EW_THREADS, 0, ctx->stream>>>(p, n);
+  p.tot_stride = 2 * nch;
+  k_mulscan2_chunk<<<dim3(ew_grid(nch), 2 * count), EW_THREADS, 0, ctx->stream>>>(p, n);
   TP_LAUNCH(ctx, "k_mulscan2_chunk");
-  TP_TRY(mulscan2_exclusive(ctx, p.tot[0], p.tot[1], nch, level + 1));
-  k_mulscan2_apply<<<dim3(ew_grid(n), 2), EW_THREADS, 0, ctx->stream>>>(p, n);
+  TP_TRY(mulscan2_exclusive(ctx, p.tot[0], p.tot[1], p.tot_stride, count, nch, level + 1));
+  k_mulscan2_apply<<<dim3(ew_grid(n), 2 * count), EW_THREADS, 0, ctx->stream>>>(p, n);
   TP_LAUNCH(ctx, "k_mulscan2_apply");
   return TP_OK;
 }
@@ -101,27 +131,41 @@ static int mulscan2_exclusive(tp_ctx* ctx, Fr* a0, Fr* a1, size_t n, int level) 
 // so z[j+1] = (prefix product of num up to j) * (suffix product of den after j) * Dtot^-1 -- two product scans that
 // share their launches and ONE inversion per proof, done by the host between the up- and the down-sweep (it also
 // replaces the zero-denominator flag: a zero denominator makes Dtot zero).  About 15 field products per row in all.
+// The grand products of `count` proofs run in the same launches, proof p in blockIdx.y, and the host inverts their
+// Dtot values with one batch inversion.
 #define PERM_CH 16   // rows per thread
 struct PermArgs {
-  const Fr* v[3];
+  const Fr* v[3];   // proof p's witness column i: v[i] + p * vstride
+  size_t vstride;
   const Fr* id[3];
   const Fr* sg[3];
-  Fr beta, gamma;
+  const Fr* bg;     // per proof: beta, gamma
+  const Fr* dinv;   // per proof: Dtot^-1 (k_perm_finish)
   size_t n;
-  Fr* pre;     // n: prefix product of num inside the row's chunk (inclusive)
-  Fr* den;     // n: den of the row
-  Fr* tot_num; // nch + 1: chunk totals of num, then a trailing one
-  Fr* tot_den; // nch + 1: chunk totals of den in REVERSE chunk order, then a trailing one
+  Fr* pre;     // n per proof: prefix product of num inside the row's chunk (inclusive)
+  Fr* den;     // n per proof: den of the row
+  Fr* tot;     // 2 (nch + 1) per proof: chunk totals of num, then a trailing one; chunk totals of den in REVERSE chunk
+               // order, then a trailing one
   size_t nch;
 };
 __global__ void __launch_bounds__(128) k_perm_chunks(PermArgs a) {
+  // the proof's beta and gamma are read from shared memory at each use: held in registers they would push the row
+  // loop past its register budget
+  __shared__ Fr bg[2];
+  const size_t p = blockIdx.y;
+  if (threadIdx.x < 2) bg[threadIdx.x] = fr_load(a.bg + 2 * p + threadIdx.x);
+  __syncthreads();
   size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (t > a.nch) return;
   if (t == a.nch) {   // the trailing ones: the exclusive scans then leave the grand totals there
-    fr_store(a.tot_num + a.nch, fr_one());
-    fr_store(a.tot_den + a.nch, fr_one());
+    Fr* tot_num = a.tot + p * 2 * (a.nch + 1);
+    fr_store(tot_num + a.nch, fr_one());
+    fr_store(tot_num + (a.nch + 1) + a.nch, fr_one());
     return;
   }
+  const size_t vo = p * a.vstride;
+  Fr* const pre = a.pre + p * a.n;
+  Fr* const den_out = a.den + p * a.n;
   const size_t lo = t * PERM_CH;
   const size_t hi = lo + PERM_CH < a.n ? lo + PERM_CH : a.n;
   Fr pn = fr_one(), pd = fr_one();
@@ -129,71 +173,125 @@ __global__ void __launch_bounds__(128) k_perm_chunks(PermArgs a) {
     Fr num, den;
 #pragma unroll
     for (int i = 0; i < 3; i++) {
-      Fr v = fr_add(fr_load(a.v[i] + j), a.gamma);
-      Fr nu = fr_add(v, pmul(a.beta, fr_load(a.id[i] + j)));
-      Fr de = fr_add(v, pmul(a.beta, fr_load(a.sg[i] + j)));
+      Fr v = fr_add(fr_load(a.v[i] + vo + j), fr_load(&bg[1]));
+      Fr nu = fr_add(v, pmul(fr_load(&bg[0]), fr_load(a.id[i] + j)));
+      Fr de = fr_add(v, pmul(fr_load(&bg[0]), fr_load(a.sg[i] + j)));
       num = i == 0 ? nu : pmul(num, nu);
       den = i == 0 ? de : pmul(den, de);
     }
     pn = j == lo ? num : pmul(pn, num);
     pd = j == lo ? den : pmul(pd, den);
-    fr_store(a.pre + j, pn);
-    fr_store(a.den + j, den);
+    fr_store(pre + j, pn);
+    fr_store(den_out + j, den);
   }
-  fr_store(a.tot_num + t, pn);
-  fr_store(a.tot_den + (a.nch - 1 - t), pd);
+  Fr* tot_num = a.tot + p * 2 * (a.nch + 1);
+  fr_store(tot_num + t, pn);
+  fr_store(tot_num + (a.nch + 1) + (a.nch - 1 - t), pd);
 }
 // carry_num[t] = product of num over the chunks before t; carry_den[nch-1-t] = product of den over the chunks after t
-__global__ void __launch_bounds__(128) k_perm_finish(PermArgs a, Fr dtot_inv, Fr* __restrict__ z /* n + 1 */) {
+__global__ void __launch_bounds__(128) k_perm_finish(PermArgs a, Fr* __restrict__ z /* n + 1 per proof */, size_t zstride) {
   size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= a.nch) return;
+  const size_t p = blockIdx.y;
+  const Fr* tot_num = a.tot + p * 2 * (a.nch + 1);
+  const Fr* tot_den = tot_num + (a.nch + 1);
+  const Fr* pre = a.pre + p * a.n;
+  const Fr* den = a.den + p * a.n;
+  z += p * zstride;
   const size_t lo = t * PERM_CH;
   const size_t hi = lo + PERM_CH < a.n ? lo + PERM_CH : a.n;
   if (t == 0) fr_store(z, fr_one());
-  Fr k = pmul(pmul(fr_load(a.tot_num + t), fr_load(a.tot_den + (a.nch - 1 - t))), dtot_inv);
+  Fr k = pmul(pmul(fr_load(tot_num + t), fr_load(tot_den + (a.nch - 1 - t))), fr_load(a.dinv + p));
   // walk the chunk backwards: k = (carries) * Dtot^-1 * product of the chunk's den after row j
   for (size_t j = hi; j-- > lo;) {
-    fr_store(z + j + 1, pmul(fr_load(a.pre + j), k));
-    if (j > lo) k = pmul(k, fr_load(a.den + j));
+    fr_store(z + j + 1, pmul(fr_load(pre + j), k));
+    if (j > lo) k = pmul(k, fr_load(den + j));
   }
 }
 
-int perm_grand_product_dev(tp_ctx* ctx, const Fr* const values[3], const Fr* const id[3], const Fr* const sigma[3],
-                           size_t n, const Fr& beta, const Fr& gamma, Fr* out, bool* closes) {
+int perm_grand_product_batch_dev(tp_ctx* ctx, const Fr* const values[3], size_t vstride, const Fr* const id[3],
+                                 const Fr* const sigma[3], size_t n, int count, const tph::HFr* beta,
+                                 const tph::HFr* gamma, Fr* out, size_t ostride, bool* zero_den, bool* closes) {
   ProfScope prof(ctx, TP_PHASE_PERM);
   const size_t nch = (n + PERM_CH - 1) / PERM_CH;
-  TP_TRY(ensure(ctx, ctx->misc[0], n * sizeof(Fr)));
-  TP_TRY(ensure(ctx, ctx->misc[1], n * sizeof(Fr)));
-  TP_TRY(ensure(ctx, ctx->misc[2], 2 * (nch + 1) * sizeof(Fr)));
+  const size_t cnt = (size_t)count;
+  if (2 * cnt * sizeof(Fr) > ctx->pinned_cap) return fail(ctx, TP_ERR_INVALID_ARG, "permutation prove: batch too large");
+  TP_TRY(ensure(ctx, ctx->misc[0], cnt * n * sizeof(Fr)));
+  TP_TRY(ensure(ctx, ctx->misc[1], cnt * n * sizeof(Fr)));
+  TP_TRY(ensure(ctx, ctx->misc[2], cnt * 2 * (nch + 1) * sizeof(Fr)));
+  std::vector<Fr> bg(2 * cnt);
+  for (size_t p = 0; p < cnt; p++) {
+    bg[2 * p] = to_dev(beta[p]);
+    bg[2 * p + 1] = to_dev(gamma[p]);
+  }
   PermArgs a;
   for (int i = 0; i < 3; i++) {
     a.v[i] = values[i];
     a.id[i] = id[i];
     a.sg[i] = sigma[i];
   }
-  a.beta = beta;
-  a.gamma = gamma;
+  a.vstride = vstride;
+  TP_TRY(params_upload(ctx, bg.data(), bg.size() * sizeof(Fr), (const void**)&a.bg));
+  a.dinv = nullptr;
   a.n = n;
   a.nch = nch;
   a.pre = (Fr*)ctx->misc[0].p;
   a.den = (Fr*)ctx->misc[1].p;
-  a.tot_num = (Fr*)ctx->misc[2].p;
-  a.tot_den = a.tot_num + (nch + 1);
-  k_perm_chunks<<<(unsigned)((nch + 1 + 127) / 128), 128, 0, ctx->stream>>>(a);
+  a.tot = (Fr*)ctx->misc[2].p;
+  k_perm_chunks<<<dim3((unsigned)((nch + 1 + 127) / 128), count), 128, 0, ctx->stream>>>(a);
   TP_LAUNCH(ctx, "k_perm_chunks");
-  TP_TRY(mulscan2_exclusive(ctx, a.tot_num, a.tot_den, nch + 1, 0));
-  // the one inversion: Dtot = product of every denominator (the last slot of the reversed den scan)
-  TP_CUDA_OK(ctx, cudaMemcpyAsync(ctx->pinned, a.tot_den + nch, sizeof(Fr), cudaMemcpyDeviceToHost, ctx->stream));
-  TP_CUDA_OK(ctx, cudaMemcpyAsync((uint8_t*)ctx->pinned + 32, a.tot_num + nch, sizeof(Fr), cudaMemcpyDeviceToHost, ctx->stream));
+  TP_TRY(mulscan2_exclusive(ctx, a.tot, a.tot + (nch + 1), 2 * (nch + 1), count, nch + 1, 0));
+  // the one inversion per proof: Dtot = product of every denominator (the last slot of the reversed den scan); Ntot
+  // the product of every numerator.  Both for every proof in one read-back.
+  const size_t pitch = 2 * (nch + 1) * sizeof(Fr);
+  uint8_t* host = (uint8_t*)ctx->pinned;
+  TP_CUDA_OK(ctx, cudaMemcpy2DAsync(host, sizeof(Fr), a.tot + (2 * nch + 1), pitch, sizeof(Fr), cnt, cudaMemcpyDeviceToHost, ctx->stream));
+  TP_CUDA_OK(ctx, cudaMemcpy2DAsync(host + cnt * sizeof(Fr), sizeof(Fr), a.tot + nch, pitch, sizeof(Fr), cnt, cudaMemcpyDeviceToHost, ctx->stream));
   TP_CUDA_OK(ctx, cudaStreamSynchronize(ctx->stream));
-  tph::HFr dtot, ntot;
-  memcpy(dtot.v, ctx->pinned, 32);
-  memcpy(ntot.v, (uint8_t*)ctx->pinned + 32, 32);
-  if (dtot.is_zero()) return fail(ctx, TP_ERR_ZERO_DENOMINATOR, "permutation prove: zero denominator");
-  const tph::HFr dinv = dtot.inv();
-  if (closes) *closes = ntot * dinv == tph::HFr::one();   // out[n], the value the caller pops (proof.rs:120)
-  k_perm_finish<<<(unsigned)((nch + 127) / 128), 128, 0, ctx->stream>>>(a, to_dev(dinv), out);
+  std::vector<tph::HFr> dtot(cnt), ntot(cnt), dinv(cnt);
+  for (size_t p = 0; p < cnt; p++) {
+    memcpy(dtot[p].v, host + p * sizeof(Fr), 32);
+    memcpy(ntot[p].v, host + (cnt + p) * sizeof(Fr), 32);
+  }
+  // Montgomery batch inversion over the non-zero Dtot; a zero one leaves its proof with Dtot^-1 = 0
+  {
+    tph::HFr acc = tph::HFr::one();
+    std::vector<tph::HFr> pre(cnt);
+    for (size_t p = 0; p < cnt; p++) {
+      pre[p] = acc;
+      if (!dtot[p].is_zero()) acc = acc * dtot[p];
+    }
+    tph::HFr inv = acc.inv();
+    for (size_t p = cnt; p-- > 0;) {
+      if (dtot[p].is_zero()) {
+        dinv[p] = tph::HFr::zero();
+        continue;
+      }
+      dinv[p] = inv * pre[p];
+      inv = inv * dtot[p];
+    }
+  }
+  std::vector<Fr> dv(cnt);
+  for (size_t p = 0; p < cnt; p++) {
+    zero_den[p] = dtot[p].is_zero();
+    if (closes) closes[p] = !zero_den[p] && ntot[p] * dinv[p] == tph::HFr::one();   // out[n], the value the caller pops (proof.rs:120)
+    dv[p] = to_dev(dinv[p]);
+  }
+  bool any = false;
+  for (size_t p = 0; p < cnt; p++) any = any || !zero_den[p];
+  if (!any) return TP_OK;
+  TP_TRY(params_upload(ctx, dv.data(), cnt * sizeof(Fr), (const void**)&a.dinv));
+  k_perm_finish<<<dim3((unsigned)((nch + 127) / 128), count), 128, 0, ctx->stream>>>(a, out, ostride);
   TP_LAUNCH(ctx, "k_perm_finish");
+  return TP_OK;
+}
+int perm_grand_product_dev(tp_ctx* ctx, const Fr* const values[3], const Fr* const id[3], const Fr* const sigma[3],
+                           size_t n, const Fr& beta, const Fr& gamma, Fr* out, bool* closes) {
+  const tph::HFr b = to_host(beta), g = to_host(gamma);
+  bool zero = false, cl = false;
+  TP_TRY(perm_grand_product_batch_dev(ctx, values, 0, id, sigma, n, 1, &b, &g, out, 0, &zero, &cl));
+  if (zero) return fail(ctx, TP_ERR_ZERO_DENOMINATOR, "permutation prove: zero denominator");
+  if (closes) *closes = cl;
   return TP_OK;
 }
 
@@ -202,37 +300,42 @@ int perm_grand_product_dev(tp_ctx* ctx, const Fr* const values[3], const Fr* con
 // =====================================================================================
 #define LIN_CH 32
 #define LIN_BASE 64
-#define LIN_MAX_BATCH 8
-// Up to LIN_MAX_BATCH independent recurrences of the same length run side by side (blockIdx.y):
-// the scans are latency-bound chains of small launches, so the prover's eight evaluations /
-// openings at one Fiat-Shamir point cost what one costs.
-struct LinBatch {
-  const Fr* p[LIN_MAX_BATCH];
-  Fr* q[LIN_MAX_BATCH];       // may be null: evaluation only
-  Fr z[LIN_MAX_BATCH];
+// Any number of independent recurrences of the same length run side by side (blockIdx.y): the scans are latency-bound
+// chains of small launches, so the eight evaluations / openings of a proof at its Fiat-Shamir points -- or those of
+// every proof of a batch -- cost what one costs.  One level of the hierarchy:
+struct LinLevel {
+  const Fr* const* p;   // level 0: device table of the inputs (null above level 0)
+  Fr* const* q;         // level 0: device table of the quotients (entries may be null: evaluation only)
+  const Fr* pbase;      // above level 0: recurrence b's input at pbase + b * stride ...
+  Fr* qbase;            // ... and its quotient at qbase + b * stride, where wantq[b]
+  size_t stride;
+  const unsigned* wantq;
+  const Fr* z;          // per recurrence: its point raised to LIN_CH^level
+  __device__ __forceinline__ const Fr* in(unsigned b) const { return p ? p[b] : pbase + b * stride; }
+  __device__ __forceinline__ Fr* out(unsigned b) const { return q ? q[b] : (wantq[b] ? qbase + b * stride : nullptr); }
 };
 
 // h[t] = sum_{k in chunk t} p[k] z^(k - lo)
-__global__ void k_linrec_reduce(LinBatch a, size_t n, Fr* h, size_t h_stride) {
+__global__ void k_linrec_reduce(LinLevel a, size_t n, Fr* h, size_t h_stride) {
   size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   size_t lo = t * LIN_CH;
   if (lo >= n) return;
-  const Fr* p = a.p[blockIdx.y];
-  const Fr z = a.z[blockIdx.y];
+  const Fr* p = a.in(blockIdx.y);
+  const Fr z = fr_load(a.z + blockIdx.y);
   size_t hi = lo + LIN_CH < n ? lo + LIN_CH : n;
   Fr acc = fr_zero();
   for (size_t k = hi; k-- > lo;) acc = fr_add(fr_load(p + k), fr_mul(z, acc));
   fr_store(h + blockIdx.y * h_stride + t, acc);
 }
 // q[k-1] = p[k] + z q[k] inside chunk t, starting from carry = qprime[t] (q at index hi-1)
-__global__ void k_linrec_apply(LinBatch a, size_t n, const Fr* qprime, size_t qp_stride) {
+__global__ void k_linrec_apply(LinLevel a, size_t n, const Fr* qprime, size_t qp_stride) {
   size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   size_t lo = t * LIN_CH;
   if (lo >= n) return;
-  Fr* q = a.q[blockIdx.y];
+  Fr* q = a.out(blockIdx.y);
   if (!q) return;
-  const Fr* p = a.p[blockIdx.y];
-  const Fr z = a.z[blockIdx.y];
+  const Fr* p = a.in(blockIdx.y);
+  const Fr z = fr_load(a.z + blockIdx.y);
   size_t hi = lo + LIN_CH < n ? lo + LIN_CH : n;
   Fr acc = fr_load(qprime + blockIdx.y * qp_stride + t);
   if (hi == n) fr_store(q + n - 1, fr_zero());
@@ -242,13 +345,12 @@ __global__ void k_linrec_apply(LinBatch a, size_t n, const Fr* qprime, size_t qp
   }
 }
 // serial base case (one thread per recurrence): q and y = p(z) -> yout[b]
-__global__ void k_linrec_serial(LinBatch a, size_t n, Fr* yout) {
-  const unsigned b = threadIdx.x;
-  if (b >= LIN_MAX_BATCH) return;
-  const Fr* p = a.p[b];
-  if (!p) return;
-  Fr* q = a.q[b];
-  const Fr z = a.z[b];
+__global__ void k_linrec_serial(LinLevel a, size_t n, unsigned batch, Fr* yout) {
+  const unsigned b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= batch) return;
+  const Fr* p = a.in(b);
+  Fr* q = a.out(b);
+  const Fr z = fr_load(a.z + b);
   Fr acc = fr_zero();
   if (q) fr_store(q + n - 1, fr_zero());
   for (size_t k = n; k-- > 0;) {
@@ -259,31 +361,27 @@ __global__ void k_linrec_serial(LinBatch a, size_t n, Fr* yout) {
 }
 
 // y[b] is written to the device words yout[b].
-static int linrec(tp_ctx* ctx, const LinBatch& in, int batch, size_t n, Fr* yout, int level) {
+static int linrec(tp_ctx* ctx, const LinLevel& in, int batch, bool any_q, size_t n, Fr* yout, int level) {
   if (n <= LIN_BASE) {
-    LinBatch a = in;
-    for (int b = batch; b < LIN_MAX_BATCH; b++) a.p[b] = nullptr;
-    k_linrec_serial<<<1, LIN_MAX_BATCH, 0, ctx->stream>>>(a, n, yout);
+    k_linrec_serial<<<(unsigned)((batch + 63) / 64), 64, 0, ctx->stream>>>(in, n, (unsigned)batch, yout);
     TP_LAUNCH(ctx, "k_linrec_serial");
     return TP_OK;
   }
   size_t nch = (n + LIN_CH - 1) / LIN_CH;
   // level buffers: h (nch per recurrence) and qprime (nch per recurrence)
-  TP_TRY(ensure(ctx, ctx->scan_tmp[level], 2 * nch * LIN_MAX_BATCH * sizeof(Fr)));
+  TP_TRY(ensure(ctx, ctx->scan_tmp[level], 2 * nch * (size_t)batch * sizeof(Fr)));
   Fr* h = (Fr*)ctx->scan_tmp[level].p;
-  Fr* qp = h + nch * LIN_MAX_BATCH;
+  Fr* qp = h + nch * batch;
   k_linrec_reduce<<<dim3(ew_grid(nch), (unsigned)batch), EW_THREADS, 0, ctx->stream>>>(in, n, h, nch);
   TP_LAUNCH(ctx, "k_linrec_reduce");
-  LinBatch next;
-  bool any_q = false;
-  for (int b = 0; b < LIN_MAX_BATCH; b++) {
-    const int s = b < batch ? b : 0;
-    next.p[b] = h + (size_t)s * nch;
-    next.q[b] = in.q[s] ? qp + (size_t)s * nch : nullptr;
-    next.z[b] = to_dev(to_host(in.z[s]).pow_u64(LIN_CH));
-    any_q = any_q || (b < batch && in.q[b]);
-  }
-  TP_TRY(linrec(ctx, next, batch, nch, yout, level + 1));
+  LinLevel next = in;
+  next.p = nullptr;
+  next.q = nullptr;
+  next.pbase = h;
+  next.qbase = qp;
+  next.stride = nch;
+  next.z = in.z + batch;
+  TP_TRY(linrec(ctx, next, batch, any_q, nch, yout, level + 1));
   if (any_q) {
     k_linrec_apply<<<dim3(ew_grid(nch), (unsigned)batch), EW_THREADS, 0, ctx->stream>>>(in, n, qp, nch);
     TP_LAUNCH(ctx, "k_linrec_apply");
@@ -295,21 +393,47 @@ static int linrec(tp_ctx* ctx, const LinBatch& in, int batch, size_t n, Fr* yout
 int poly_open_batch_dev(tp_ctx* ctx, const Fr* const* p, size_t len, const Fr* z, Fr* const* q_out, int batch,
                         tph::HFr* y) {
   if (len == 0) return fail(ctx, TP_ERR_EMPTY_POLY, "open: empty polynomial");
-  if (batch < 1 || batch > LIN_MAX_BATCH) return fail(ctx, TP_ERR_INVALID_ARG, "open: bad batch size");
+  if (batch < 1 || batch > 65535 || (size_t)batch * sizeof(Fr) > ctx->pinned_cap)
+    return fail(ctx, TP_ERR_INVALID_ARG, "open: bad batch size");
   ProfScope prof(ctx, TP_PHASE_SCAN);
-  TP_TRY(ensure(ctx, ctx->misc[2], LIN_MAX_BATCH * sizeof(Fr)));
+  const size_t nb = (size_t)batch;
+  TP_TRY(ensure(ctx, ctx->misc[2], nb * sizeof(Fr)));
   Fr* yd = (Fr*)ctx->misc[2].p;
-  LinBatch in;
-  for (int b = 0; b < LIN_MAX_BATCH; b++) {
-    const int s = b < batch ? b : 0;
-    in.p[b] = p[s];
-    in.q[b] = q_out ? q_out[s] : nullptr;
-    in.z[b] = z[s];
+  // one parameter block: the points of every level, the input and quotient tables, the wanted-quotient flags
+  int levels = 1;
+  for (size_t m = len; m > LIN_BASE; m = (m + LIN_CH - 1) / LIN_CH) levels++;
+  const size_t zbytes = (size_t)levels * nb * sizeof(Fr), pbytes = nb * sizeof(void*);
+  std::vector<uint8_t> blk(zbytes + 2 * pbytes + nb * sizeof(unsigned));
+  Fr* zs = (Fr*)blk.data();
+  const Fr** ps = (const Fr**)(blk.data() + zbytes);
+  Fr** qs = (Fr**)(blk.data() + zbytes + pbytes);
+  unsigned* wq = (unsigned*)(blk.data() + zbytes + 2 * pbytes);
+  bool any_q = false;
+  for (size_t b = 0; b < nb; b++) {
+    tph::HFr zl = to_host(z[b]);
+    for (int l = 0; l < levels; l++) {
+      zs[(size_t)l * nb + b] = to_dev(zl);
+      zl = zl.pow_u64(LIN_CH);
+    }
+    ps[b] = p[b];
+    qs[b] = q_out ? q_out[b] : nullptr;
+    wq[b] = qs[b] ? 1u : 0u;
+    any_q = any_q || qs[b];
   }
-  TP_TRY(linrec(ctx, in, batch, len, yd, 0));
-  TP_CUDA_OK(ctx, cudaMemcpyAsync(ctx->pinned, yd, batch * sizeof(Fr), cudaMemcpyDeviceToHost, ctx->stream));
+  const uint8_t* dev = nullptr;
+  TP_TRY(params_upload(ctx, blk.data(), blk.size(), (const void**)&dev));
+  LinLevel in;
+  in.z = (const Fr*)dev;
+  in.p = (const Fr* const*)(dev + zbytes);
+  in.q = (Fr* const*)(dev + zbytes + pbytes);
+  in.wantq = (const unsigned*)(dev + zbytes + 2 * pbytes);
+  in.pbase = nullptr;
+  in.qbase = nullptr;
+  in.stride = 0;
+  TP_TRY(linrec(ctx, in, batch, any_q, len, yd, 0));
+  TP_CUDA_OK(ctx, cudaMemcpyAsync(ctx->pinned, yd, nb * sizeof(Fr), cudaMemcpyDeviceToHost, ctx->stream));
   TP_CUDA_OK(ctx, cudaStreamSynchronize(ctx->stream));
-  for (int b = 0; b < batch; b++) memcpy(y[b].v, (const uint8_t*)ctx->pinned + 32 * b, 32);
+  for (size_t b = 0; b < nb; b++) memcpy(y[b].v, (const uint8_t*)ctx->pinned + 32 * b, 32);
   return TP_OK;
 }
 int poly_open_dev(tp_ctx* ctx, const Fr* p, size_t len, const Fr& z, Fr* q_out, tph::HFr* y) {
@@ -323,43 +447,45 @@ int poly_open_dev(tp_ctx* ctx, const Fr* p, size_t len, const Fr& z, Fr* q_out, 
 // =====================================================================================
 struct GateArgs {
   const Fr* sel[5];
-  const Fr* adv[3];
+  const Fr* adv[3];   // proof p (blockIdx.y): adv[i] + p * stride, pi + p * stride
   const Fr* pi;
-  size_t n;
-  unsigned* flag;
+  size_t n, stride;
+  unsigned* flag;     // one per proof
 };
 __global__ void k_gate_check(GateArgs g) {
   size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= g.n) return;
-  Fr a = fr_load(g.adv[0] + j), b = fr_load(g.adv[1] + j), c = fr_load(g.adv[2] + j);
+  const size_t o = (size_t)blockIdx.y * g.stride + j;
+  Fr a = fr_load(g.adv[0] + o), b = fr_load(g.adv[1] + o), c = fr_load(g.adv[2] + o);
   Fr acc = fr_mul(fr_load(g.sel[0] + j), a);
   acc = fr_add(acc, fr_mul(fr_load(g.sel[1] + j), b));
   acc = fr_sub(acc, fr_mul(fr_load(g.sel[2] + j), c));
   acc = fr_add(acc, fr_mul(fr_mul(fr_load(g.sel[3] + j), a), b));
   acc = fr_add(acc, fr_load(g.sel[4] + j));
-  const Fr pi = fr_load(g.pi + j);
+  const Fr pi = fr_load(g.pi + o);
   acc = fr_add(acc, pi);
   // bit 0: the gate equation fails on some row; bit 1: some public input is non-zero
   const unsigned f = (fr_is_zero(acc) ? 0u : 1u) | (fr_is_zero(pi) ? 0u : 2u);
-  if (f) atomicOr(g.flag, f);
+  if (f) atomicOr(g.flag + blockIdx.y, f);
 }
 int gate_check_dev(tp_ctx* ctx, const Fr* const sel_evals[5], const Fr* const adv[3], const Fr* pi, size_t n,
-                   bool* ok, bool* pi_is_zero) {
-  TP_TRY(ensure(ctx, ctx->flag, sizeof(unsigned)));
+                   size_t stride, int count, unsigned* flags) {
+  const size_t bytes = (size_t)count * sizeof(unsigned);
+  if (bytes > ctx->pinned_cap) return fail(ctx, TP_ERR_INVALID_ARG, "gate check: batch too large");
+  TP_TRY(ensure(ctx, ctx->flag, bytes));
   GateArgs g;
   for (int i = 0; i < 5; i++) g.sel[i] = sel_evals[i];
   for (int i = 0; i < 3; i++) g.adv[i] = adv[i];
   g.pi = pi;
   g.n = n;
+  g.stride = stride;
   g.flag = (unsigned*)ctx->flag.p;
-  TP_CUDA_OK(ctx, cudaMemsetAsync(g.flag, 0, sizeof(unsigned), ctx->stream));
-  k_gate_check<<<ew_grid(n), EW_THREADS, 0, ctx->stream>>>(g);
+  TP_CUDA_OK(ctx, cudaMemsetAsync(g.flag, 0, bytes, ctx->stream));
+  k_gate_check<<<dim3(ew_grid(n), count), EW_THREADS, 0, ctx->stream>>>(g);
   TP_LAUNCH(ctx, "k_gate_check");
-  TP_CUDA_OK(ctx, cudaMemcpyAsync(ctx->pinned, g.flag, sizeof(unsigned), cudaMemcpyDeviceToHost, ctx->stream));
+  TP_CUDA_OK(ctx, cudaMemcpyAsync(ctx->pinned, g.flag, bytes, cudaMemcpyDeviceToHost, ctx->stream));
   TP_CUDA_OK(ctx, cudaStreamSynchronize(ctx->stream));
-  const unsigned f = *(unsigned*)ctx->pinned;
-  *ok = (f & 1u) == 0;
-  if (pi_is_zero) *pi_is_zero = (f & 2u) == 0;
+  memcpy(flags, ctx->pinned, bytes);
   return TP_OK;
 }
 
@@ -370,54 +496,63 @@ int gate_check_dev(tp_ctx* ctx, const Fr* const sel_evals[5], const Fr* const ad
 // 4n-sized table here is COSET-MAJOR: entry k * n + i belongs to the point omega_4n^(4i + k).  A
 // coset is a self-contained unit of work (five size-n coset NTTs, this kernel, one inverse coset
 // NTT), which is what lets the quotient be sharded over GPUs by coset (api.cu).
+struct QuotScalars {   // per proof
+  Fr alpha, alpha2, beta, gamma;
+  Fr bk[3];  // beta * k_i
+};
 struct QuotKernelArgs {
   const Fr* sel4[5];
   const Fr* sig4[3];
-  const Fr* adv4[3];
-  const Fr* z4;
-  const Fr* pi4;
   const Fr* l0_4;
   const Fr* tw4;
-  Fr alpha, alpha2, beta, gamma;
-  Fr bk[3];  // beta * k_i
+  const Fr* adv4[3];   // proof p: + p * stride, likewise z4, pi4 and out
+  const Fr* z4;
+  const Fr* pi4;
   Fr* out;
+  size_t stride;
+  const QuotScalars* sc;
+  const unsigned* items;   // blockIdx.y selects the item: proof << 2 | coset
   size_t n;
-  unsigned cosets[4];  // blockIdx.y selects the coset
 };
 __global__ void __launch_bounds__(EW_THREADS) k_quotient_numerator(QuotKernelArgs q) {
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= q.n) return;
-  const unsigned k = q.cosets[blockIdx.y];
+  const unsigned item = q.items[blockIdx.y];
+  const unsigned k = item & 3u;
+  const size_t po = (size_t)(item >> 2) * q.stride;
+  const QuotScalars* sc = q.sc + (item >> 2);
   const size_t half = q.n * 2;
   const size_t i4 = 4 * i + k;               // exponent of omega_4n at this point
   const size_t o = (size_t)k * q.n + i;      // coset-major slot
   Fr x = i4 < half ? fr_load(q.tw4 + i4) : fr_neg(fr_load(q.tw4 + (i4 - half)));
-  Fr a = fr_load(q.adv4[0] + o), b = fr_load(q.adv4[1] + o), c = fr_load(q.adv4[2] + o);
-  Fr z = fr_load(q.z4 + o);
-  Fr zw = fr_load(q.z4 + (size_t)k * q.n + (i + 1 < q.n ? i + 1 : 0));   // z(omega x): next point of the same coset
+  Fr a = fr_load(q.adv4[0] + po + o), b = fr_load(q.adv4[1] + po + o), c = fr_load(q.adv4[2] + po + o);
+  Fr z = fr_load(q.z4 + po + o);
+  Fr zw = fr_load(q.z4 + po + (size_t)k * q.n + (i + 1 < q.n ? i + 1 : 0));   // z(omega x): next point of the same coset
   // gate line (proof.rs:317-320)
   Fr acc = pmul(fr_load(q.sel4[0] + o), a);
   acc = fr_add(acc, pmul(fr_load(q.sel4[1] + o), b));
   acc = fr_sub(acc, pmul(fr_load(q.sel4[2] + o), c));
   acc = fr_add(acc, pmul(pmul(fr_load(q.sel4[3] + o), a), b));
   acc = fr_add(acc, fr_load(q.sel4[4] + o));
-  acc = fr_add(acc, fr_load(q.pi4 + o));
+  acc = fr_add(acc, fr_load(q.pi4 + po + o));
   // permutation lines (proof.rs:323-354)
-  Fr ag = fr_add(a, q.gamma), bg = fr_add(b, q.gamma), cg = fr_add(c, q.gamma);
-  Fr l2 = pmul(fr_add(ag, pmul(q.bk[0], x)), fr_add(bg, pmul(q.bk[1], x)));
-  l2 = pmul(l2, fr_add(cg, pmul(q.bk[2], x)));
+  const Fr gamma = fr_load(&sc->gamma), beta = fr_load(&sc->beta);
+  Fr ag = fr_add(a, gamma), bg = fr_add(b, gamma), cg = fr_add(c, gamma);
+  Fr l2 = pmul(fr_add(ag, pmul(fr_load(&sc->bk[0]), x)), fr_add(bg, pmul(fr_load(&sc->bk[1]), x)));
+  l2 = pmul(l2, fr_add(cg, pmul(fr_load(&sc->bk[2]), x)));
   l2 = pmul(l2, z);
-  Fr l3 = pmul(fr_add(ag, pmul(q.beta, fr_load(q.sig4[0] + o))), fr_add(bg, pmul(q.beta, fr_load(q.sig4[1] + o))));
-  l3 = pmul(l3, fr_add(cg, pmul(q.beta, fr_load(q.sig4[2] + o))));
+  Fr l3 = pmul(fr_add(ag, pmul(beta, fr_load(q.sig4[0] + o))), fr_add(bg, pmul(beta, fr_load(q.sig4[1] + o))));
+  l3 = pmul(l3, fr_add(cg, pmul(beta, fr_load(q.sig4[2] + o))));
   l3 = pmul(l3, zw);
-  acc = fr_add(acc, pmul(q.alpha, fr_sub(l2, l3)));
+  acc = fr_add(acc, pmul(fr_load(&sc->alpha), fr_sub(l2, l3)));
   // L0 line (proof.rs:355-360)
   Fr l4 = pmul(fr_sub(z, fr_one()), fr_load(q.l0_4 + o));
-  acc = fr_add(acc, pmul(q.alpha2, l4));
-  fr_store(q.out + o, acc);
+  acc = fr_add(acc, pmul(fr_load(&sc->alpha2), l4));
+  fr_store(q.out + po + o, acc);
 }
-int quotient_numerator_dev(tp_ctx* ctx, const QuotientArgs& a, const unsigned* cosets, int ncosets) {
-  if (ncosets <= 0) return TP_OK;
+int quotient_numerator_dev(tp_ctx* ctx, const QuotientArgs& a, const unsigned* items, int nitems) {
+  if (nitems <= 0) return TP_OK;
+  if (nitems > 65535) return fail(ctx, TP_ERR_INVALID_ARG, "quotient: too many cosets in one launch");
   ProfScope prof(ctx, TP_PHASE_QUOTIENT);
   QuotKernelArgs q;
   for (int i = 0; i < 5; i++) q.sel4[i] = a.sel4[i];
@@ -429,16 +564,26 @@ int quotient_numerator_dev(tp_ctx* ctx, const QuotientArgs& a, const unsigned* c
   q.pi4 = a.pi4;
   q.l0_4 = a.l0_4;
   q.tw4 = a.tw4;
-  tph::HFr al = to_host(a.alpha), be = to_host(a.beta);
-  q.alpha = a.alpha;
-  q.alpha2 = to_dev(al.sqr());
-  q.beta = a.beta;
-  q.gamma = a.gamma;
-  for (int i = 0; i < 3; i++) q.bk[i] = to_dev(be * to_host(a.k[i]));
   q.out = a.out;
+  q.stride = a.stride;
   q.n = a.n;
-  for (int i = 0; i < 4; i++) q.cosets[i] = cosets[i < ncosets ? i : 0];
-  k_quotient_numerator<<<dim3(ew_grid(a.n), (unsigned)ncosets), EW_THREADS, 0, ctx->stream>>>(q);
+  // one parameter block: the per-proof scalars, then the items
+  const size_t sbytes = (size_t)a.count * sizeof(QuotScalars);
+  std::vector<uint8_t> blk(sbytes + (size_t)nitems * sizeof(unsigned));
+  QuotScalars* sc = (QuotScalars*)blk.data();
+  for (int p = 0; p < a.count; p++) {
+    sc[p].alpha = to_dev(a.alpha[p]);
+    sc[p].alpha2 = to_dev(a.alpha[p].sqr());
+    sc[p].beta = to_dev(a.beta[p]);
+    sc[p].gamma = to_dev(a.gamma[p]);
+    for (int i = 0; i < 3; i++) sc[p].bk[i] = to_dev(a.beta[p] * a.k[i]);
+  }
+  memcpy(blk.data() + sbytes, items, (size_t)nitems * sizeof(unsigned));
+  const uint8_t* dev = nullptr;
+  TP_TRY(params_upload(ctx, blk.data(), blk.size(), (const void**)&dev));
+  q.sc = (const QuotScalars*)dev;
+  q.items = (const unsigned*)(dev + sbytes);
+  k_quotient_numerator<<<dim3(ew_grid(a.n), (unsigned)nitems), EW_THREADS, 0, ctx->stream>>>(q);
   TP_LAUNCH(ctx, "k_quotient_numerator");
   return TP_OK;
 }
@@ -450,11 +595,14 @@ int quotient_numerator_dev(tp_ctx* ctx, const QuotientArgs& a, const unsigned* c
 // Then t_2 = N_3, t_1 = N_2 + t_2, t_0 = N_1 + t_1.
 // c0_is_zero: the numerator vanishes on H itself (always, for a witness that satisfies the copy constraints), so
 // coset 0 was never evaluated and its slot holds nothing.
-__global__ void k_quotient_combine(const Fr* __restrict__ c4, size_t n, Fr iota_inv, Fr quarter, int c0_is_zero,
-                                   Fr* __restrict__ t) {
+// Proof p (blockIdx.y) reads c4 + p * stride and writes t + p * stride.
+__global__ void k_quotient_combine(const Fr* __restrict__ c4, size_t n, size_t stride, Fr iota_inv, Fr quarter,
+                                   const unsigned* __restrict__ c0_is_zero, Fr* __restrict__ t) {
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  const Fr c0 = c0_is_zero ? fr_zero() : fr_load(c4 + i);
+  c4 += blockIdx.y * stride;
+  t += blockIdx.y * stride;
+  const Fr c0 = c0_is_zero[blockIdx.y] ? fr_zero() : fr_load(c4 + i);
   const Fr c1 = fr_load(c4 + n + i), c2 = fr_load(c4 + 2 * n + i), c3 = fr_load(c4 + 3 * n + i);
   const Fr e = fr_add(c0, c2), f = fr_sub(c0, c2), g = fr_add(c1, c3);
   const Fr h = fr_mul(iota_inv, fr_sub(c1, c3));
@@ -466,14 +614,18 @@ __global__ void k_quotient_combine(const Fr* __restrict__ c4, size_t n, Fr iota_
   fr_store(t + n + i, t1);
   fr_store(t + i, fr_add(n1, t1));
 }
-int quotient_combine_dev(tp_ctx* ctx, const Fr* c4, size_t n, bool c0_is_zero, Fr* t) {
+int quotient_combine_dev(tp_ctx* ctx, const Fr* c4, size_t n, size_t stride, int count, const bool* c0_is_zero, Fr* t) {
   ProfScope prof(ctx, TP_PHASE_QUOTIENT);
   // iota = omega_4n^n is a primitive fourth root of unity: iota^-1 = -iota; quarter = 4^-1
   unsigned log_n = 0;
   while (((size_t)1 << log_n) < n) log_n++;
   tph::HFr iota_inv = omega_for_log(log_n + 2).pow_u64((uint64_t)n).neg();
   tph::HFr quarter = tph::HFr::from_u64(4).inv();
-  k_quotient_combine<<<ew_grid(n), EW_THREADS, 0, ctx->stream>>>(c4, n, to_dev(iota_inv), to_dev(quarter), c0_is_zero ? 1 : 0, t);
+  std::vector<unsigned> flags(count);
+  for (int p = 0; p < count; p++) flags[p] = c0_is_zero[p] ? 1u : 0u;
+  const unsigned* fd = nullptr;
+  TP_TRY(params_upload(ctx, flags.data(), flags.size() * sizeof(unsigned), (const void**)&fd));
+  k_quotient_combine<<<dim3(ew_grid(n), count), EW_THREADS, 0, ctx->stream>>>(c4, n, stride, to_dev(iota_inv), to_dev(quarter), fd, t);
   TP_LAUNCH(ctx, "k_quotient_combine");
   return TP_OK;
 }
@@ -530,31 +682,37 @@ int l0_evals_4n_dev(tp_ctx* ctx, const Fr* tw4, size_t n, Fr* out) {
 #define LIN_MAX_TERMS 12
 struct LinArgs {
   const Fr* p[LIN_MAX_TERMS];
-  Fr s[LIN_MAX_TERMS];
+  size_t pstride[LIN_MAX_TERMS];   // proof p reads term t at p[t] + p * pstride[t] (0: shared by every proof)
   int nterms;
-  Fr constant;
-  size_t n;
-  Fr* out;
+  const Fr* s;                     // per proof: nterms scalars, then the constant
+  size_t n, ostride;
+  Fr* out;                         // proof p: out + p * ostride
 };
 __global__ void k_lincomb(LinArgs a) {
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= a.n) return;
-  Fr acc = i == 0 ? a.constant : fr_zero();
-  for (int t = 0; t < a.nterms; t++) acc = fr_add(acc, fr_mul(a.s[t], fr_load(a.p[t] + i)));
-  fr_store(a.out + i, acc);
+  const size_t pr = blockIdx.y;
+  const Fr* s = a.s + pr * (a.nterms + 1);
+  Fr acc = i == 0 ? fr_load(s + a.nterms) : fr_zero();
+  for (int t = 0; t < a.nterms; t++) acc = fr_add(acc, fr_mul(fr_load(s + t), fr_load(a.p[t] + pr * a.pstride[t] + i)));
+  fr_store(a.out + pr * a.ostride + i, acc);
 }
-int lincomb_dev(tp_ctx* ctx, const LinTerm* terms, int nterms, const Fr& constant, size_t n, Fr* out) {
+int lincomb_dev(tp_ctx* ctx, const LinTerm* terms, int nterms, const tph::HFr* scalars, size_t n, int count, Fr* out,
+                size_t ostride) {
   if (nterms > LIN_MAX_TERMS) return fail(ctx, TP_ERR_INVALID_ARG, "lincomb: too many terms");
   LinArgs a;
   for (int t = 0; t < nterms; t++) {
     a.p[t] = terms[t].p;
-    a.s[t] = terms[t].s;
+    a.pstride[t] = terms[t].stride;
   }
+  std::vector<Fr> s((size_t)count * (nterms + 1));
+  for (size_t i = 0; i < s.size(); i++) s[i] = to_dev(scalars[i]);
+  TP_TRY(params_upload(ctx, s.data(), s.size() * sizeof(Fr), (const void**)&a.s));
   a.nterms = nterms;
-  a.constant = constant;
   a.n = n;
   a.out = out;
-  k_lincomb<<<ew_grid(n), EW_THREADS, 0, ctx->stream>>>(a);
+  a.ostride = ostride;
+  k_lincomb<<<dim3(ew_grid(n), count), EW_THREADS, 0, ctx->stream>>>(a);
   TP_LAUNCH(ctx, "k_lincomb");
   return TP_OK;
 }

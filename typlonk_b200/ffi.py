@@ -31,7 +31,7 @@ SYMBOLS = [
     "tp_commit", "tp_commit_dev", "tp_open", "tp_ntt", "tp_ntt_dev", "tp_perm_prove",
     "tp_circuit_load", "tp_circuit_compile", "tp_circuit_destroy", "tp_circuit_sigma_commitments",
     "tp_prove", "tp_prove_dev", "tp_prove_inputs", "tp_measure_imad_peak", "tp_selftest", "tp_fr_rand_stream", "tp_ctx_set_option", "tp_ctx_get_stat",
-    "tp_srs_g2", "tp_srs_set_g2", "tp_kzg_verify", "tp_pairing_check", "tp_verify", "tp_verify_batch", "tp_verify_prepared", "tp_proof_challenges",
+    "tp_srs_g2", "tp_srs_set_g2", "tp_kzg_verify", "tp_pairing_check", "tp_verify", "tp_verify_batch", "tp_prove_batch", "tp_verify_prepared", "tp_proof_challenges",
     "tp_trace_create", "tp_trace_destroy", "tp_trace_gate", "tp_trace_gates", "tp_trace_assert_eq", "tp_trace_finish",
     "tp_trace_gate_kinds", "tp_trace_selectors", "tp_trace_permutation", "tp_trace_witness",
     "tp_permutation_builder_create", "tp_permutation_builder_destroy", "tp_permutation_builder_add_row",
@@ -594,6 +594,25 @@ class CircuitHandle:
         self.ctx._check(lib().tp_prove_inputs(self.ctx._h, self._h, adv, _buf(public_inputs_mont) if n_public else None,
                                               C.c_size_t(n_public), out, C.c_size_t(PROOF_FIXED_BYTES)))
         return bytes(out)
+
+    def prove_batch(self, advice_list, public_inputs_list):
+        """tp_prove_batch: advice_list[k] is proof k's three witness columns, public_inputs_list[k] its public-input
+        vector as prove_inputs takes it (Montgomery bytes, any length <= n; b"" = none).  Returns (proof blocks,
+        statuses): status 0 is a proof, 6 (gate unsatisfied) or 5 (zero denominator) a zero-filled block."""
+        count = len(advice_list)
+        assert len(public_inputs_list) == count
+        keep = [(C.c_char * len(b)).from_buffer_copy(b) for cols in advice_list for b in cols]
+        adv = (C.c_void_p * max(3 * count, 1))(*[C.cast(b, C.c_void_p) for b in keep])
+        pkeep = [(C.c_char * len(b)).from_buffer_copy(b) if b else None for b in public_inputs_list]
+        pis = (C.c_void_p * max(count, 1))(*[C.cast(b, C.c_void_p) if b is not None else None for b in pkeep])
+        npub = (C.c_size_t * max(count, 1))(*[len(b) // 32 for b in public_inputs_list])
+        out = (C.c_char * max(count * PROOF_FIXED_BYTES, 1))()
+        status = (C.c_int * max(count, 1))()
+        self.ctx._check(lib().tp_prove_batch(self.ctx._h, self._h, C.c_size_t(count), adv, pis, npub, out,
+                                             C.c_size_t(count * PROOF_FIXED_BYTES), status))
+        raw = bytes(out)
+        return ([raw[k * PROOF_FIXED_BYTES:(k + 1) * PROOF_FIXED_BYTES] for k in range(count)],
+                [status[k] for k in range(count)])
 
     def prove_dev(self, advice_dptrs, pi_dptr) -> bytes:
         adv = (C.c_void_p * 3)(*[C.c_void_p(p) for p in advice_dptrs])

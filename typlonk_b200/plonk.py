@@ -28,7 +28,7 @@ from dataclasses import dataclass
 from typing import List
 
 from . import field as F
-from .ffi import (Context, GateUnsatisfied, PROOF_FIXED_BYTES, GATE_ADD, GATE_MUL, Trace,  # noqa: F401
+from .ffi import (Context, GateUnsatisfied, TyplonkError, PROOF_FIXED_BYTES, GATE_ADD, GATE_MUL, Trace,  # noqa: F401
                   proof_decode, proof_encode)
 from .kzg import Srs
 from .permutation import Permutation
@@ -111,6 +111,22 @@ class CompiledCircuit:
         pis = (given + [0] * self.rows)[: self.rows]          # what Proof.public_inputs carries (proof.rs:52-53, 190)
         fixed = self.handle.prove_inputs(cols, F.fr_vec_to_bytes(given))
         return Proof(fixed, pis)
+
+    def prove_batch(self, inputs_list, public_inputs_list, blinders_list) -> List[Proof]:
+        """Many proofs of this circuit in one call (tp_prove_batch); proof k equals prove(inputs_list[k],
+        public_inputs_list[k], blinders_list[k]).  Raises what prove would raise for the first failing proof, naming
+        its index."""
+        count = len(inputs_list)
+        assert len(public_inputs_list) == count and len(blinders_list) == count
+        cols = [self.witness_bytes(i, b) for i, b in zip(inputs_list, blinders_list)]
+        given = [[v % F.R_MOD for v in pi][: self.rows] for pi in public_inputs_list]
+        fixed, status = self.handle.prove_batch(cols, [F.fr_vec_to_bytes(g) for g in given])
+        for k, st in enumerate(status):
+            if st == 6:
+                raise GateUnsatisfied(st, "prove_batch: proof %d: gate constraints do not vanish on the domain" % k)
+            if st != 0:
+                raise TyplonkError(st, "prove_batch: proof %d: permutation prove: zero denominator" % k)
+        return [Proof(f, (g + [0] * self.rows)[: self.rows]) for f, g in zip(fixed, given)]
 
     def verify(self, proof: Proof) -> bool:
         """CompiledCircuit::verify (proof.rs:59-63, 195-233)."""
