@@ -403,6 +403,47 @@ int tp_srs_serialized_size(const tp_srs* srs, size_t* bytes);
 int tp_srs_serialize(tp_ctx* ctx, const tp_srs* srs, uint8_t* out, size_t cap, size_t* written);
 int tp_srs_deserialize(tp_ctx* ctx, const uint8_t* bytes, size_t len, int check, tp_srs** out);
 
+/* Compressed encodings (ark-serialize 0.3 `serialize`, what CanonicalSerialize writes by default): a G1 point is its
+ * canonical x, 48 B LE, with bit 7 of the last byte set iff y > -y (canonical integers) and bit 6 for infinity
+ * (written as x = 0, sign bit clear; both bits set is invalid); a G2 point is x.c0 | x.c1 with the flags in the last
+ * byte of x.c1, y > -y comparing c1 first, then c0.  Decoding recovers y = (x^3 + b)^((q+1)/4): an x without a root is
+ * rejected at every check level.  A proof block is the same fields in the same order as the TP_PROOF_FIXED_BYTES
+ * block: 13 x 48 + 7 x 32 bytes.  The Fiat-Shamir transcript still hashes uncompressed points, so challenges do not
+ * depend on the wire form. */
+#define TP_WIRE_G1_COMPRESSED_BYTES 48
+#define TP_WIRE_G2_COMPRESSED_BYTES 96
+#define TP_PROOF_COMPRESSED_FIXED_BYTES 848
+/* TP_PROOF_FIXED_BYTES block -> compressed block (host only).  len != TP_PROOF_FIXED_BYTES, or anything
+ * tp_proof_decode rejects in the block -> TP_ERR_MALFORMED; cap < TP_PROOF_COMPRESSED_FIXED_BYTES ->
+ * TP_ERR_BUFFER_TOO_SMALL. */
+int tp_proof_compress(const uint8_t* fixed, size_t len, uint8_t* out, size_t cap);
+/* Compressed block -> TP_PROOF_FIXED_BYTES block (host only, checked: what tp_verify and tp_verify_prepared take).
+ * len != TP_PROOF_COMPRESSED_FIXED_BYTES, a scalar >= r, x >= q, an x without a root or invalid flags ->
+ * TP_ERR_MALFORMED; cap < TP_PROOF_FIXED_BYTES -> TP_ERR_BUFFER_TOO_SMALL.  fixed_out is untouched on failure. */
+int tp_proof_decompress(const uint8_t* in, size_t len, uint8_t* fixed_out, size_t cap);
+/* The Proof framing of tp_proof_encode / tp_proof_decode with the compressed block: block | Vec<Fr>.  Encoding takes
+ * and decoding returns the uncompressed TP_PROOF_FIXED_BYTES block, so everything downstream is unchanged. */
+int tp_proof_encoded_size_compressed(size_t n_public, size_t* bytes);
+int tp_proof_encode_compressed(const uint8_t* fixed, const uint64_t* public_inputs, size_t n_public, uint8_t* out,
+                               size_t cap, size_t* written);
+int tp_proof_decode_compressed(const uint8_t* bytes, size_t len, uint8_t fixed_out[TP_PROOF_FIXED_BYTES],
+                               uint64_t* public_inputs_out, size_t cap_public, size_t* n_public);
+/* tp_proof_decompress for `count` contiguous compressed blocks at once, the square roots on the device (one point per
+ * thread): fixed_out gets count x TP_PROOF_FIXED_BYTES, ready for tp_verify_batch.
+ * status (count ints, may be NULL): status[k] = tp_proof_decompress's verdict on block k (TP_OK or TP_ERR_MALFORMED);
+ *   a failed block is zero-filled and the call still returns TP_OK.  With status == NULL the call returns
+ *   TP_ERR_MALFORMED for the lowest failing index (named in tp_last_error); the other blocks are written as above.
+ * count == 0 -> TP_OK.  count > 65536, null pointers -> TP_ERR_INVALID_ARG; cap < count * TP_PROOF_FIXED_BYTES ->
+ * TP_ERR_BUFFER_TOO_SMALL.  Device groups: rank 0 does the work. */
+int tp_proofs_decompress(tp_ctx* ctx, const uint8_t* in, size_t count, uint8_t* fixed_out, size_t cap, int* status);
+/* Srs with compressed points: u64 count | count x 48 B G1 | G2 | tau G2 (96 B each), half the size of the
+ * uncompressed form.  check as tp_srs_deserialize: 0 and 1 recover y (on the curve by construction), 2 adds the
+ * prime-order subgroup check; a rejected point -> TP_ERR_MALFORMED with the count and the first index in
+ * tp_last_error.  Device groups: serialisation reads rank 0's copy, every rank decodes its own. */
+int tp_srs_serialized_size_compressed(const tp_srs* srs, size_t* bytes);
+int tp_srs_serialize_compressed(tp_ctx* ctx, const tp_srs* srs, uint8_t* out, size_t cap, size_t* written);
+int tp_srs_deserialize_compressed(tp_ctx* ctx, const uint8_t* bytes, size_t len, int check, tp_srs** out);
+
 /* ---- helpers ---------------------------------------------------------------------------- */
 /* Measured dependent-free IMAD throughput of this device (instructions/s), for rooflines. */
 int tp_measure_imad_peak(tp_ctx* ctx, double* imad_per_s, double* imad_wide_per_s);

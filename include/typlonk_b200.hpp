@@ -214,14 +214,26 @@ class Srs {
   }
   /// Srs::random (srs.rs:36-41).
   static Srs random(const Context& ctx, size_t gates) { return from_secret(ctx, Fr::random(), gates); }
-  /// Additive API (SURVEY.md 8 f4): ark-serialize 0.3 uncompressed Vec<G1> | G2 | tau G2.
-  static Srs from_bytes(const Context& ctx, const std::vector<uint8_t>& raw, int check = 2) {
+  /// Additive API (SURVEY.md 8 f4): ark-serialize 0.3 uncompressed Vec<G1> | G2 | tau G2, or with compressed points
+  /// (48 B per G1, 96 B per G2; decompressed and checked on the device).
+  static Srs from_bytes(const Context& ctx, const std::vector<uint8_t>& raw, int check = 2, bool compressed = false) {
     tp_srs* h = nullptr;
-    detail::check(tp_srs_deserialize(ctx.get(), raw.data(), raw.size(), check, &h), "tp_srs_deserialize", ctx.get());
+    if (compressed)
+      detail::check(tp_srs_deserialize_compressed(ctx.get(), raw.data(), raw.size(), check, &h),
+                    "tp_srs_deserialize_compressed", ctx.get());
+    else
+      detail::check(tp_srs_deserialize(ctx.get(), raw.data(), raw.size(), check, &h), "tp_srs_deserialize", ctx.get());
     return Srs(ctx, h);
   }
-  std::vector<uint8_t> to_bytes() const {
+  std::vector<uint8_t> to_bytes(bool compressed = false) const {
     size_t need = 0;
+    if (compressed) {
+      detail::check(tp_srs_serialized_size_compressed(get(), &need), "tp_srs_serialized_size_compressed");
+      std::vector<uint8_t> out(need);
+      detail::check(tp_srs_serialize_compressed(ctx_.get(), get(), out.data(), out.size(), nullptr),
+                    "tp_srs_serialize_compressed", ctx_.get());
+      return out;
+    }
     detail::check(tp_srs_serialized_size(get(), &need), "tp_srs_serialized_size");
     std::vector<uint8_t> out(need);
     detail::check(tp_srs_serialize(ctx_.get(), get(), out.data(), out.size(), nullptr), "tp_srs_serialize", ctx_.get());
@@ -436,24 +448,48 @@ class Var {
 struct Proof {
   std::array<uint8_t, TP_PROOF_FIXED_BYTES> fixed{};
   std::vector<Fr> public_inputs;  // padded to `rows` (proof.rs:52-53, 190)
-  /// Additive API (SURVEY.md 8 f4).
-  std::vector<uint8_t> to_bytes() const {
+  /// Additive API (SURVEY.md 8 f4).  compressed: the same framing with an 848-byte block of compressed points.
+  std::vector<uint8_t> to_bytes(bool compressed = false) const {
     size_t need = 0;
+    const uint64_t* pis = public_inputs.empty() ? nullptr : public_inputs[0].limbs;
+    if (compressed) {
+      tp_proof_encoded_size_compressed(public_inputs.size(), &need);
+      std::vector<uint8_t> out(need);
+      detail::check(tp_proof_encode_compressed(fixed.data(), pis, public_inputs.size(), out.data(), out.size(), nullptr),
+                    "tp_proof_encode_compressed");
+      return out;
+    }
     tp_proof_encoded_size(public_inputs.size(), &need);
     std::vector<uint8_t> out(need);
-    detail::check(tp_proof_encode(fixed.data(), public_inputs.empty() ? nullptr : public_inputs[0].limbs, public_inputs.size(),
-                                  out.data(), out.size(), nullptr),
+    detail::check(tp_proof_encode(fixed.data(), pis, public_inputs.size(), out.data(), out.size(), nullptr),
                   "tp_proof_encode");
     return out;
   }
-  static Proof from_bytes(const std::vector<uint8_t>& raw) {
+  /// `fixed` is the uncompressed block either way.
+  static Proof from_bytes(const std::vector<uint8_t>& raw, bool compressed = false) {
+    auto decode = compressed ? tp_proof_decode_compressed : tp_proof_decode;
+    const char* what = compressed ? "tp_proof_decode_compressed" : "tp_proof_decode";
     Proof p;
     size_t n = 0;
-    detail::check(tp_proof_decode(raw.data(), raw.size(), nullptr, nullptr, 0, &n), "tp_proof_decode");
+    detail::check(decode(raw.data(), raw.size(), nullptr, nullptr, 0, &n), what);
     p.public_inputs.resize(n);
-    detail::check(tp_proof_decode(raw.data(), raw.size(), p.fixed.data(), n ? p.public_inputs[0].limbs : nullptr, n, &n),
-                  "tp_proof_decode");
+    detail::check(decode(raw.data(), raw.size(), p.fixed.data(), n ? p.public_inputs[0].limbs : nullptr, n, &n), what);
     return p;
+  }
+  /// tp_proofs_decompress: `count` contiguous compressed blocks -> uncompressed blocks, the square roots on the device.
+  /// status[k] is TP_OK or TP_ERR_MALFORMED (block zero-filled); without `status` a malformed block throws.
+  static std::vector<std::array<uint8_t, TP_PROOF_FIXED_BYTES>> decompress_blocks(const Context& ctx,
+                                                                                 const std::vector<uint8_t>& blocks,
+                                                                                 std::vector<int>* status = nullptr) {
+    const size_t count = blocks.size() / TP_PROOF_COMPRESSED_FIXED_BYTES;
+    if (count * TP_PROOF_COMPRESSED_FIXED_BYTES != blocks.size())
+      throw Malformed(TP_ERR_MALFORMED, "decompress_blocks: not a whole number of compressed proof blocks");
+    std::vector<std::array<uint8_t, TP_PROOF_FIXED_BYTES>> out(count);
+    if (status) status->assign(count, TP_OK);
+    detail::check(tp_proofs_decompress(ctx.get(), blocks.data(), count, count ? out[0].data() : nullptr,
+                                       count * TP_PROOF_FIXED_BYTES, status ? status->data() : nullptr),
+                  "tp_proofs_decompress", ctx.get());
+    return out;
   }
 };
 

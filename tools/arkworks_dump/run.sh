@@ -41,6 +41,29 @@ impl Proof {
         self.public_inputs.serialize_uncompressed(&mut v).unwrap();
         v
     }
+    // the same items with `serialize`: compressed points (x and the y-sign flag), scalars unchanged
+    pub fn dump_compressed(&self) -> Vec<u8> {
+        use ark_serialize::CanonicalSerialize;
+        let mut v = vec![];
+        for p in [&self.a, &self.b, &self.c] {
+            p.commitment.0.serialize(&mut v).unwrap();
+            p.opening.0.serialize(&mut v).unwrap();
+            p.opening.1.serialize(&mut v).unwrap();
+        }
+        self.permutation.commitment.0.serialize(&mut v).unwrap();
+        self.permutation.z.0.serialize(&mut v).unwrap();
+        self.permutation.z.1.serialize(&mut v).unwrap();
+        self.permutation.zw.0.serialize(&mut v).unwrap();
+        self.permutation.zw.1.serialize(&mut v).unwrap();
+        self.evaluation_point.serialize(&mut v).unwrap();
+        for t in self.t.iter() {
+            t.0.serialize(&mut v).unwrap();
+        }
+        self.r.0.serialize(&mut v).unwrap();
+        self.r.1.serialize(&mut v).unwrap();
+        self.public_inputs.serialize(&mut v).unwrap();
+        v
+    }
 }
 RS
 grep -q 'seed_from_u64(1)' "$here/ref/kzg/src/srs.rs" && grep -q 'seed_from_u64(2)' "$here/ref/plonk/src/proof.rs"

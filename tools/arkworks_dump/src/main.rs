@@ -1,8 +1,8 @@
 //! Writes arkworks-generated known answers for everything the oracle restates from memory (SURVEY.md App. A.4 - A.6):
 //! `serialize_unchecked` of G1 points, `StdRng::seed_from_u64`, `Fr::rand`, the challenge chain of
-//! plonk/src/proof/challenges.rs, domain elements, and whole proofs of the reference's own circuits under the fixed
-//! randomness run.sh patches in.  Output: one JSON object (hex strings are little-endian bytes as arkworks writes them).
-use ark_bls12_381::{Fr, G1Affine};
+//! plonk/src/proof/challenges.rs, domain elements, whole proofs of the reference's own circuits under the fixed
+//! randomness run.sh patches in, and the compressed encoding (`serialize`) of G1 / G2 points and of one proof.  Output: one JSON object (hex strings are little-endian bytes as arkworks writes them).
+use ark_bls12_381::{Fr, G1Affine, G2Affine};
 use ark_ec::AffineCurve;
 use ark_ff::{BigInteger, FftField, PrimeField, UniformRand, Zero};
 use ark_poly::{EvaluationDomain, GeneralEvaluationDomain};
@@ -35,6 +35,16 @@ fn g1_unchecked(p: &G1Affine) -> String {
     p.serialize_unchecked(&mut v).unwrap();
     hex(&v)
 }
+fn g1_compressed(p: &G1Affine) -> String {
+    let mut v = vec![];
+    p.serialize(&mut v).unwrap();
+    hex(&v)
+}
+fn g2_compressed(p: &G2Affine) -> String {
+    let mut v = vec![];
+    p.serialize(&mut v).unwrap();
+    hex(&v)
+}
 
 struct Pythagoras;
 impl CircuitDescription<3> for Pythagoras {
@@ -65,6 +75,18 @@ fn main() {
     writeln!(j, "  \"g1_generator_unchecked\": \"{}\",", g1_unchecked(&g)).unwrap();
     writeln!(j, "  \"g1_17_unchecked\": \"{}\",", g1_unchecked(&g17)).unwrap();
     writeln!(j, "  \"g1_zero_unchecked\": \"{}\",", g1_unchecked(&G1Affine::zero())).unwrap();
+    // compressed (`serialize`): x with the PositiveY / infinity flags in the top bits of the last byte
+    writeln!(j, "  \"g1_generator_compressed\": \"{}\",", g1_compressed(&g)).unwrap();
+    writeln!(j, "  \"g1_17_compressed\": \"{}\",", g1_compressed(&g17)).unwrap();
+    writeln!(j, "  \"g1_minus_17_compressed\": \"{}\",", g1_compressed(&-g17)).unwrap();
+    writeln!(j, "  \"g1_zero_compressed\": \"{}\",", g1_compressed(&G1Affine::zero())).unwrap();
+    {
+        let h = G2Affine::prime_subgroup_generator();
+        let tau = Fr::rand(&mut StdRng::seed_from_u64(1));
+        let htau: G2Affine = h.mul(tau).into();
+        writeln!(j, "  \"g2_generator_compressed\": \"{}\",", g2_compressed(&h)).unwrap();
+        writeln!(j, "  \"g2_tau_seed_1_compressed\": \"{}\",", g2_compressed(&htau)).unwrap();
+    }
     // StdRng::seed_from_u64(k): first four u64 draws
     for k in [0u64, 1, 2, 13037422643194131432] {
         let mut rng = StdRng::seed_from_u64(k);
@@ -106,6 +128,7 @@ fn main() {
     let circuit = Pythagoras::build();
     let proof = circuit.prove([3, 4, 5], vec![0]);
     writeln!(j, "  \"readme_pythagoras_3_4_5_proof\": \"{}\",", hex(&proof.dump_uncompressed())).unwrap();
+    writeln!(j, "  \"readme_pythagoras_3_4_5_proof_compressed\": \"{}\",", hex(&proof.dump_compressed())).unwrap();
     assert!(circuit.verify(proof));
     let circuit = MulChain13::build();
     let proof = circuit.prove([3, 5], vec![0]);

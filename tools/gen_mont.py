@@ -822,6 +822,10 @@ def main():
         out.append("#define TP_%s_ONE %s   // R mod p" % (nm, carr(R, n)))
         out.append("#define TP_%s_R2 %s   // R^2 mod p" % (nm, carr(R * R % mod, n)))
         out.append("#define TP_%s_MODM2 %s   // p - 2 (Fermat inversion exponent)" % (nm, carr(mod - 2, n)))
+        if nm == "FQ":
+            assert mod % 4 == 3
+            out.append("#define TP_FQ_SQRT_EXP %s   // (q + 1) / 4 (square-root exponent, q = 3 mod 4)"
+                       % carr((mod + 1) // 4, n))
     # Fr has -r^-1 mod 2^32 = 0xffffffff.  When ptxas sees that immediate it rewrites mi = -t0 and
     # then splits every reduction product mi * r_j into IMAD.X + IMAD.HI.U32.X (6.6 clk on the
     # FMA-heavy pipe instead of 4 for the fused IMAD.WIDE.U32.X) -- about half of all products of

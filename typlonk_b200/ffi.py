@@ -13,6 +13,7 @@ _LIB_PATH = Path(os.environ.get("TYPLONK_B200_LIB") or
 G1_BYTES = 97
 G2_BYTES = 193
 PROOF_FIXED_BYTES = 1472
+PROOF_COMPRESSED_FIXED_BYTES = 848
 PHASES = ["msm_total", "msm_sort", "msm_accum", "msm_reduce", "ntt", "quotient", "perm", "scan"]
 
 ERRORS = {
@@ -39,6 +40,9 @@ SYMBOLS = [
     "tp_permutation_compile", "tp_fr_from_i64", "tp_fr_from_canonical", "tp_fr_to_canonical",
     "tp_proof_encoded_size", "tp_proof_encode", "tp_proof_decode",
     "tp_srs_serialized_size", "tp_srs_serialize", "tp_srs_deserialize", "tp_build_stamp", "tp_stdrng_words", "tp_circuit_read_poly", "tp_proof_points_in_subgroup",
+    "tp_proof_compress", "tp_proof_decompress", "tp_proof_encoded_size_compressed", "tp_proof_encode_compressed",
+    "tp_proof_decode_compressed", "tp_proofs_decompress",
+    "tp_srs_serialized_size_compressed", "tp_srs_serialize_compressed", "tp_srs_deserialize_compressed",
 ]
 
 COMM_ID_BYTES = 128
@@ -179,6 +183,59 @@ def proof_decode(raw: bytes):
     rc = lib().tp_proof_decode(_buf(raw), C.c_size_t(len(raw)), fixed, pis, C.c_size_t(n.value), C.byref(n))
     if rc != 0:
         raise TyplonkError(rc, "tp_proof_decode")
+    return bytes(fixed), bytes(pis)[: 32 * n.value]
+
+
+def proof_compress(fixed: bytes) -> bytes:
+    """tp_proof_compress: 1472-byte block -> 848-byte block with compressed points.  Host only; raises Malformed."""
+    out = (C.c_char * PROOF_COMPRESSED_FIXED_BYTES)()
+    rc = lib().tp_proof_compress(_buf(fixed), C.c_size_t(len(fixed)), out, C.c_size_t(PROOF_COMPRESSED_FIXED_BYTES))
+    if rc == 12:
+        raise Malformed(rc, "tp_proof_compress: malformed proof block")
+    if rc != 0:
+        raise TyplonkError(rc, "tp_proof_compress")
+    return bytes(out)
+
+
+def proof_decompress(block: bytes) -> bytes:
+    """tp_proof_decompress (checked): 848-byte block -> 1472-byte block.  Host only; raises Malformed."""
+    out = (C.c_char * PROOF_FIXED_BYTES)()
+    rc = lib().tp_proof_decompress(_buf(block), C.c_size_t(len(block)), out, C.c_size_t(PROOF_FIXED_BYTES))
+    if rc == 12:
+        raise Malformed(rc, "tp_proof_decompress: malformed compressed proof block")
+    if rc != 0:
+        raise TyplonkError(rc, "tp_proof_decompress")
+    return bytes(out)
+
+
+def proof_encode_compressed(fixed: bytes, public_inputs_mont: bytes) -> bytes:
+    """tp_proof_encode_compressed: the 848-byte compressed block + Vec<Fr> of public inputs.  Host only."""
+    n = len(public_inputs_mont) // 32
+    need = C.c_size_t(0)
+    lib().tp_proof_encoded_size_compressed(C.c_size_t(n), C.byref(need))
+    out = (C.c_char * need.value)()
+    rc = lib().tp_proof_encode_compressed(_buf(fixed), _buf(public_inputs_mont) if n else None, C.c_size_t(n), out,
+                                          C.c_size_t(need.value), None)
+    if rc == 12:
+        raise Malformed(rc, "tp_proof_encode_compressed: malformed proof block")
+    if rc != 0:
+        raise TyplonkError(rc, "tp_proof_encode_compressed")
+    return bytes(out)
+
+
+def proof_decode_compressed(raw: bytes):
+    """tp_proof_decode_compressed (checked): -> (uncompressed 1472-byte block, public inputs as Montgomery bytes)."""
+    n = C.c_size_t(0)
+    rc = lib().tp_proof_decode_compressed(_buf(raw), C.c_size_t(len(raw)), None, None, C.c_size_t(0), C.byref(n))
+    if rc == 12:
+        raise Malformed(rc, "tp_proof_decode_compressed: malformed proof encoding")
+    if rc != 0:
+        raise TyplonkError(rc, "tp_proof_decode_compressed")
+    fixed = (C.c_char * PROOF_FIXED_BYTES)()
+    pis = (C.c_char * (32 * n.value or 1))()
+    rc = lib().tp_proof_decode_compressed(_buf(raw), C.c_size_t(len(raw)), fixed, pis, C.c_size_t(n.value), C.byref(n))
+    if rc != 0:
+        raise TyplonkError(rc, "tp_proof_decode_compressed")
     return bytes(fixed), bytes(pis)[: 32 * n.value]
 
 
@@ -517,6 +574,26 @@ class Context:
         self._check(rc)
         return SrsHandle(self, h)
 
+    def srs_deserialize_compressed(self, raw, check=2):
+        """tp_srs_deserialize_compressed: u64 count | count x 48 B G1 | G2 | tau G2 (96 B each) -> device SRS; the
+        square roots and checks run on the device.  check: 0 / 1 recover y, 2 + prime-order subgroup.  Raises
+        Malformed."""
+        h = C.c_void_p()
+        rc = lib().tp_srs_deserialize_compressed(self._h, _buf(raw), C.c_size_t(len(raw)), C.c_int(check), C.byref(h))
+        if rc == 12:
+            raise Malformed(rc, lib().tp_last_error(self._h).decode())
+        self._check(rc)
+        return SrsHandle(self, h)
+
+    def proofs_decompress(self, blocks: bytes, count: int):
+        """tp_proofs_decompress: `count` contiguous 848-byte blocks -> (count x 1472-byte blocks as one bytes object,
+        per-block statuses: 0 = TP_OK, 12 = TP_ERR_MALFORMED with the block zero-filled)."""
+        out = (C.c_char * max(count * PROOF_FIXED_BYTES, 1))()
+        status = (C.c_int * max(count, 1))()
+        self._check(lib().tp_proofs_decompress(self._h, _buf(blocks) if count else None, C.c_size_t(count), out,
+                                               C.c_size_t(count * PROOF_FIXED_BYTES), status))
+        return bytes(out)[: count * PROOF_FIXED_BYTES], [status[k] for k in range(count)]
+
     def circuit_compile(self, srs, selector_evals, perm_u64: bytes, n):
         keep = [_buf(b) for b in selector_evals]
         sel = (C.c_void_p * 5)(*[C.cast(x, C.c_void_p) for x in keep])
@@ -543,6 +620,14 @@ class SrsHandle:
         lib().tp_srs_serialized_size(self._h, C.byref(need))
         out = bytearray(need.value)
         self.ctx._check(lib().tp_srs_serialize(self.ctx._h, self._h, _buf(out), C.c_size_t(len(out)), None))
+        return out
+
+    def serialize_compressed(self) -> bytearray:
+        """tp_srs_serialize_compressed: u64 count | count x 48 B G1 | G2 | tau G2 (96 B each), compressed points."""
+        need = C.c_size_t(0)
+        lib().tp_srs_serialized_size_compressed(self._h, C.byref(need))
+        out = bytearray(need.value)
+        self.ctx._check(lib().tp_srs_serialize_compressed(self.ctx._h, self._h, _buf(out), C.c_size_t(len(out)), None))
         return out
 
     def download(self, offset=0, count=None) -> bytes:

@@ -23,13 +23,17 @@ class Srs:
     def from_points(cls, ctx: Context, points) -> "Srs":
         return cls(ctx, ctx.srs_upload(b"".join(F.g1_to_packed(p) for p in points)))
 
-    def to_bytes(self) -> bytes:
-        """Vec<G1> | G2 | tau G2 in ark-serialize 0.3 uncompressed encoding (tp_srs_serialize; SURVEY.md 8 f4)."""
-        return bytes(self.handle.serialize())
+    def to_bytes(self, compressed=False) -> bytes:
+        """Vec<G1> | G2 | tau G2 in ark-serialize 0.3 uncompressed encoding (tp_srs_serialize; SURVEY.md 8 f4), or
+        with compressed points (tp_srs_serialize_compressed: 48 B per G1 point, 96 B per G2 point)."""
+        return bytes(self.handle.serialize_compressed() if compressed else self.handle.serialize())
 
     @classmethod
-    def from_bytes(cls, ctx: Context, raw, check=2) -> "Srs":
-        """tp_srs_deserialize: validated on the device (check = 2: on the curve and in the prime-order subgroup)."""
+    def from_bytes(cls, ctx: Context, raw, check=2, compressed=False) -> "Srs":
+        """tp_srs_deserialize / tp_srs_deserialize_compressed: validated on the device (check = 2: on the curve and in
+        the prime-order subgroup; compressed points are decompressed there too)."""
+        if compressed:
+            return cls(ctx, ctx.srs_deserialize_compressed(raw, check))
         return cls(ctx, ctx.srs_deserialize(raw, check))
 
     def g1_ref(self, offset=0, count=None):

@@ -29,7 +29,7 @@ from typing import List
 
 from . import field as F
 from .ffi import (Context, GateUnsatisfied, TyplonkError, PROOF_FIXED_BYTES, GATE_ADD, GATE_MUL, Trace,  # noqa: F401
-                  proof_decode, proof_encode)
+                  proof_decode, proof_decode_compressed, proof_encode, proof_encode_compressed)
 from .kzg import Srs
 from .permutation import Permutation
 
@@ -75,15 +75,18 @@ class Proof:
     fixed: bytes
     public_inputs: List[int]
 
-    def to_bytes(self) -> bytes:
-        """tp_proof_encode (the additive `Proof::to_bytes` of SURVEY.md 8 f4)."""
-        return proof_encode(self.fixed, F.fr_vec_to_bytes(self.public_inputs))
+    def to_bytes(self, compressed=False) -> bytes:
+        """tp_proof_encode (the additive `Proof::to_bytes` of SURVEY.md 8 f4), or tp_proof_encode_compressed: the
+        same framing with compressed points (an 848-byte block instead of 1472)."""
+        encode = proof_encode_compressed if compressed else proof_encode
+        return encode(self.fixed, F.fr_vec_to_bytes(self.public_inputs))
 
     @classmethod
-    def from_bytes(cls, raw: bytes) -> "Proof":
+    def from_bytes(cls, raw: bytes, compressed=False) -> "Proof":
         """tp_proof_decode: checked (canonical scalars and coordinates, points on the curve, exact length);
-        raises ffi.Malformed otherwise."""
-        fixed, pis = proof_decode(raw)
+        raises ffi.Malformed otherwise.  compressed=True: tp_proof_decode_compressed, which recovers every y (an x
+        without a root is malformed); `fixed` is the uncompressed block either way."""
+        fixed, pis = (proof_decode_compressed if compressed else proof_decode)(raw)
         return cls(fixed, F.fr_vec_from_bytes(pis))
 
 
