@@ -161,6 +161,25 @@ int tp_srs_destroy(tp_ctx* ctx, tp_srs* srs);
 int tp_srs_g2(const tp_srs* srs, uint8_t g2[TP_G2_BYTES], uint8_t g2s[TP_G2_BYTES]);
 int tp_srs_set_g2(tp_srs* srs, const uint8_t g2[TP_G2_BYTES], const uint8_t g2s[TP_G2_BYTES]);
 
+/* ---- SRS ceremony (additive API: a powers-of-tau setup that no single party's secret controls) ------------------ */
+
+/* One ceremony contribution: *out = a new SRS with g1[i] = s^i * srs.g1[i], g2 unchanged, g2s = s * srs.g2s;
+ * pubkey = [s]G2 (TP_G2_BYTES, ABI encoding as tp_srs_g2), which proves the link (tp_srs_update_check).
+ * s: Montgomery limbs like tp_srs_from_secret's tau; s == 0 or s >= r -> TP_ERR_INVALID_ARG; an SRS without G2
+ * points -> TP_ERR_INVALID_ARG.  srs is left untouched (destroy it once the link is checked).  Device groups: every
+ * rank scales its own copy. */
+int tp_srs_contribute(tp_ctx* ctx, const tp_srs* srs, const uint64_t s[4], tp_srs** out, uint8_t pubkey[TP_G2_BYTES]);
+/* *ok = 1 iff the SRS is the powers of one secret: g1[0] = G, g2 = the G2 generator, every g1[i] in G1 and not
+ * infinity, g2s in G2 and not infinity, and g1[i+1] = t g1[i] for all i where g2s = [t]G2 (a pairing check of a
+ * combination with random weights rho^i, rho drawn inside the call from the operating system; a wrong SRS passes
+ * with probability at most (len - 1) / (r - 1)).  len < 2, no G2 points -> TP_ERR_INVALID_ARG.  A bad point is
+ * *ok = 0, not an error.  Device groups: one rho for every rank, the verdict is rank 0's. */
+int tp_srs_verify(tp_ctx* ctx, const tp_srs* srs, int* ok);
+/* One ceremony link, host only: *ok = 1 iff e(next_tau_g1, G2) == e(prev_tau_g1, pubkey), with both G1 points
+ * on the curve, in G1, not infinity, and pubkey in G2, not infinity.  (tau_g1 = g1[1] of each SRS.) */
+int tp_srs_update_check(const uint8_t prev_tau_g1[TP_G1_BYTES], const uint8_t next_tau_g1[TP_G1_BYTES],
+                        const uint8_t pubkey[TP_G2_BYTES], int* ok);
+
 /* ---- KZG  (kzg/src/lib.rs) ------------------------------------------------------------- */
 
 /* KzgScheme::commit (lib.rs:37-54): sum_i coeffs[i] * srs[i].  len == 0 -> infinity.

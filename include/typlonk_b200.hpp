@@ -5,6 +5,7 @@
 // so that a program written against fabrizio-m/TyPLONK reads the same here:
 //
 //   kzg          Srs::{from_secret, random, g1_ref, g2_ref, g2s_ref}            kzg/src/srs.rs:8-52
+//                (additive: Srs::{contribute, verify, verify_update}, a powers-of-tau ceremony)
 //                KzgScheme::{commit, open, verify, identity}                    kzg/src/lib.rs:33-86
 //   permutation  Tag, PermutationBuilder::{with_rows, add_row, add_constrain,
 //                add_constrains, build}, Permutation::compile,
@@ -266,6 +267,29 @@ class Srs {
   }
   G2Affine g2_ref() const { return g2_pair().first; }    // srs.rs:46-48
   G2Affine g2s_ref() const { return g2_pair().second; }  // srs.rs:49-51
+  /// Additive API, one powers-of-tau contribution (tp_srs_contribute): a new SRS with g1[i] * s^i and g2s * s, and the
+  /// pubkey [s]G2 that links it to this one (verify_update).  This SRS is unchanged.
+  std::pair<Srs, G2Affine> contribute(const Fr& s) const {
+    tp_srs* h = nullptr;
+    G2Affine pub;
+    detail::check(tp_srs_contribute(ctx_.get(), get(), s.limbs, &h, pub.bytes.data()), "tp_srs_contribute", ctx_.get());
+    return {Srs(ctx_, h), pub};
+  }
+  /// ... with s drawn from the operating system's CSPRNG and forgotten.
+  std::pair<Srs, G2Affine> contribute() const { return contribute(Fr::random()); }
+  /// Is this SRS the powers of one secret (tp_srs_verify: subgroup checks and a randomised pairing check)?
+  bool verify() const {
+    int ok = 0;
+    detail::check(tp_srs_verify(ctx_.get(), get(), &ok), "tp_srs_verify", ctx_.get());
+    return ok != 0;
+  }
+  /// Was this SRS made from `prev` by the contribution with this pubkey (tp_srs_update_check on g1[1] of both)?
+  bool verify_update(const Srs& prev, const G2Affine& pubkey) const {
+    int ok = 0;
+    detail::check(tp_srs_update_check(prev.g1_ref(1, 1)[0].bytes.data(), g1_ref(1, 1)[0].bytes.data(), pubkey.bytes.data(), &ok),
+                  "tp_srs_update_check");
+    return ok != 0;
+  }
   tp_srs* get() const { return h_.get(); }
   const Context& context() const { return ctx_; }
 
@@ -504,25 +528,13 @@ class CompiledCircuit {
 
   /// CircuitBuilder::compile (builder.rs:60-113) with the SRS secret as an input.
   CompiledCircuit(const Context& ctx, const Fr& tau) : ctx_(ctx) {
-    tp_trace* t = nullptr;
-    detail::check(tp_trace_create(INPUTS, &t), "tp_trace_create");
-    trace_ = std::shared_ptr<tp_trace>(t, [](tp_trace* p) { tp_trace_destroy(p); });
-    DESC::template run<Var>(make_inputs(std::make_index_sequence<INPUTS>{}));
-    size_t gates = 0;
-    detail::check(tp_trace_finish(t, &rows, &gates), "tp_trace_finish (an asserted variable never entered a gate?)");
-    srs_ = std::make_unique<Srs>(Srs::from_secret(ctx, tau, rows));
-    std::vector<Fr> sel(5 * rows);
-    detail::check(tp_trace_selectors(t, sel[0].limbs), "tp_trace_selectors");
-    std::vector<uint64_t> perm(3 * rows);
-    detail::check(tp_trace_permutation(t, perm.data()), "tp_trace_permutation");
-    const uint64_t* cols[5];
-    for (int k = 0; k < 5; k++) cols[k] = sel[k * rows].limbs;
-    uint8_t fixed[5 * TP_G1_BYTES];
-    tp_circuit* c = nullptr;
-    detail::check(tp_circuit_compile(ctx.get(), srs_->get(), cols, perm.data(), rows, &c, fixed), "tp_circuit_compile", ctx.get());
-    Context keep = ctx;
-    circuit_ = std::shared_ptr<tp_circuit>(c, [keep](tp_circuit* p) { tp_circuit_destroy(keep.get(), p); });
-    for (int k = 0; k < 5; k++) std::memcpy(fixed_commitments[k].point.bytes.data(), fixed + k * TP_G1_BYTES, TP_G1_BYTES);
+    trace();
+    compile(Srs::from_secret(ctx, tau, rows));
+  }
+  /// Additive API: compiled against an existing SRS (e.g. the outcome of a ceremony) of at least `rows` points.
+  CompiledCircuit(const Context& ctx, const Srs& srs) : ctx_(ctx) {
+    trace();
+    compile(srs);
   }
 
   /// CompiledCircuit::prove (proof.rs:26-57) with the nine blinders a0 a1 a2 b0 b1 b2 c0 c1 c2 (proof.rs:43-48)
@@ -611,6 +623,29 @@ class CompiledCircuit {
   std::array<Var, INPUTS> make_inputs(std::index_sequence<K...>) const {
     return {Var(trace_, (uint64_t)K)...};
   }
+  void trace() {
+    tp_trace* t = nullptr;
+    detail::check(tp_trace_create(INPUTS, &t), "tp_trace_create");
+    trace_ = std::shared_ptr<tp_trace>(t, [](tp_trace* p) { tp_trace_destroy(p); });
+    DESC::template run<Var>(make_inputs(std::make_index_sequence<INPUTS>{}));
+    size_t gates = 0;
+    detail::check(tp_trace_finish(t, &rows, &gates), "tp_trace_finish (an asserted variable never entered a gate?)");
+  }
+  void compile(const Srs& srs) {
+    srs_ = std::make_unique<Srs>(srs);
+    std::vector<Fr> sel(5 * rows);
+    detail::check(tp_trace_selectors(trace_.get(), sel[0].limbs), "tp_trace_selectors");
+    std::vector<uint64_t> perm(3 * rows);
+    detail::check(tp_trace_permutation(trace_.get(), perm.data()), "tp_trace_permutation");
+    const uint64_t* cols[5];
+    for (int k = 0; k < 5; k++) cols[k] = sel[k * rows].limbs;
+    uint8_t fixed[5 * TP_G1_BYTES];
+    tp_circuit* c = nullptr;
+    detail::check(tp_circuit_compile(ctx_.get(), srs_->get(), cols, perm.data(), rows, &c, fixed), "tp_circuit_compile", ctx_.get());
+    Context keep = ctx_;
+    circuit_ = std::shared_ptr<tp_circuit>(c, [keep](tp_circuit* p) { tp_circuit_destroy(keep.get(), p); });
+    for (int k = 0; k < 5; k++) std::memcpy(fixed_commitments[k].point.bytes.data(), fixed + k * TP_G1_BYTES, TP_G1_BYTES);
+  }
   Context ctx_;
   std::shared_ptr<tp_trace> trace_;
   std::unique_ptr<Srs> srs_;
@@ -626,6 +661,11 @@ CompiledCircuit<DESC> build(const Context& ctx) {
 template <class DESC>
 CompiledCircuit<DESC> build(const Context& ctx, const Fr& tau) {
   return CompiledCircuit<DESC>(ctx, tau);
+}
+/// ... or on an SRS the caller made, e.g. by a ceremony (Srs::contribute, Srs::verify).
+template <class DESC>
+CompiledCircuit<DESC> build(const Context& ctx, const Srs& srs) {
+  return CompiledCircuit<DESC>(ctx, srs);
 }
 
 }  // namespace typlonk

@@ -288,11 +288,9 @@ int srs_alloc(tp_ctx* ctx, size_t len, tp_srs** out) {
   delete s;
   return fail(ctx, TP_ERR_CUDA, "srs: out of device memory");
 }
-}  // namespace tp
-}  // extern "C++"
 
 // group front of an SRS: `make(rank context, &part)` on every rank
-static int srs_group_new(tp_ctx* g, tp_srs** out, const std::function<int(tp_ctx*, tp_srs**)>& make) {
+int srs_group_new(tp_ctx* g, tp_srs** out, const std::function<int(tp_ctx*, tp_srs**)>& make) {
   tp_srs* front = new tp_srs();
   front->parts.assign(g->children.size(), nullptr);
   int rc = group_run(g, [&](tp_ctx* c, int r) { return make(c, &front->parts[r]); });
@@ -307,6 +305,8 @@ static int srs_group_new(tp_ctx* g, tp_srs** out, const std::function<int(tp_ctx
   *out = front;
   return TP_OK;
 }
+}  // namespace tp
+}  // extern "C++"
 
 int tp_srs_from_secret(tp_ctx* ctx, const uint64_t tau[4], size_t gates, tp_srs** out) {
   if (!ctx) return TP_ERR_INVALID_ARG;

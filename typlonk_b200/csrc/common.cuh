@@ -237,6 +237,7 @@ int ntt_batch_dev(tp_ctx* ctx, const Fr* const* in, Fr* const* out, const uint64
                   unsigned log_n, bool inverse);
 int ntt_get_twiddles(tp_ctx* ctx, unsigned log_n, const Fr** tw);
 tph::HFr omega_for_log(unsigned log_n);  // generator of the 2^log_n-th roots of unity (ark-poly Radix2EvaluationDomain)
+int pow_table_dev(tp_ctx* ctx, Fr* out, const tph::HFr& base, size_t count);  // out[i] = base^i, i < count
 // msm.cu : result as host Jacobian (this rank's shard only when sharded = false, else combined)
 int msm_dev(tp_ctx* ctx, const tp_srs* srs, const Fr* scalars_dev, size_t len, uint8_t out[TP_G1_BYTES]);
 // `batch` MSMs over the same bases in one pipeline (out[b] = sum_i scalars[b][i] * srs[i])
@@ -307,6 +308,8 @@ int rotate_copy_dev(tp_ctx* ctx, const Fr* in, size_t n, size_t shift, Fr* out);
 void msm_choose_tables(size_t len, size_t table_len, size_t budget_bytes, unsigned world, unsigned* c_out, unsigned* levels_out);
 // api.cu: device allocation of an SRS with the fixed-base table levels the MSM plan wants
 int srs_alloc(tp_ctx* ctx, size_t len, tp_srs** out);
+// api.cu: group front of an SRS, `make(rank context, &part)` on every rank (the rank is the context's `rank`)
+int srs_group_new(tp_ctx* group, tp_srs** out, const std::function<int(tp_ctx*, tp_srs**)>& make);
 // wire.cu: Montgomery SRS records <-> ark-serialize 0.3 uncompressed records, on the device
 int g1_to_wire_dev(tp_ctx* ctx, const G1Affine* in, size_t len, void* out_dev);
 int g1_from_wire_dev(tp_ctx* ctx, const void* in_dev, size_t len, int check, G1Affine* out, size_t* rejected,
@@ -314,6 +317,10 @@ int g1_from_wire_dev(tp_ctx* ctx, const void* in_dev, size_t len, int check, G1A
 // srs.cu
 int srs_generate_dev(tp_ctx* ctx, const tph::HFr& tau, size_t len, G1Affine* out);
 int srs_build_levels_dev(tp_ctx* ctx, tp_srs* srs);
+// out[i] = [s^i] in[i], i < len (level 0 only; the caller rebuilds the table levels)
+int srs_contribute_dev(tp_ctx* ctx, const G1Affine* in, const tph::HFr& s, size_t len, G1Affine* out);
+// verify_batch.cu: ok[i] = 1 iff [r] pts[i] is the identity (an all-zero record gets 0)
+int subgroup_flags_dev(tp_ctx* ctx, const G1Affine* pts, size_t len, uint8_t* ok_dev);
 // selftest.cu
 int selftest_dev(tp_ctx* ctx, int* failures);
 int measure_imad_dev(tp_ctx* ctx, double* imad, double* wide);

@@ -44,6 +44,14 @@ __global__ void k_pow_table(Fr* out, Fr base, size_t count, Fr scale) {
   }
 }
 
+int pow_table_dev(tp_ctx* ctx, Fr* out, const tph::HFr& base, size_t count) {
+  if (count == 0) return TP_OK;
+  k_pow_table<<<(unsigned)(((count + 15) / 16 + 127) / 128), 128, 0, ctx->stream>>>(out, to_dev(base), count,
+                                                                                   to_dev(tph::HFr::one()));
+  TP_LAUNCH(ctx, "k_pow_table");
+  return TP_OK;
+}
+
 __device__ __forceinline__ unsigned bitrev(unsigned x, unsigned bits) { return bits == 0 ? 0u : (__brev(x) >> (32 - bits)); }
 
 // Up to NTT_MAX_BATCH transforms of the same size and direction run in one launch (blockIdx.y):

@@ -2,7 +2,8 @@
 // reference computes as `length` serial double-and-add multiplications).  Here: every thread
 // takes 8 consecutive powers of tau (one pow, then a multiply chain), multiplies the generator
 // by each with a fixed-base table of 32 windows x 255 affine multiples (32 mixed additions per
-// point, no doublings), and normalises its 8 results to affine with one shared inversion.
+// point, no doublings), and normalises its 8 results to affine with one shared inversion.  A ceremony contribution
+// (k_srs_contribute, srs_ceremony.cu) rescales an existing SRS by the powers of a new secret in the same shape.
 #include "common.cuh"
 
 namespace tp {
@@ -56,6 +57,34 @@ static int build_fixed_base(tp_ctx* ctx) {
   return TP_OK;
 }
 
+// The tail every kernel below shares: a thread's `cnt` XYZZ results to packed affine records out[0 .. cnt), with one
+// shared inversion of the product of their zz * zzz (the identity stays the all-zero record).
+__device__ __forceinline__ void store_affine(const G1Xyzz (&pts)[SRS_PER], int cnt, G1Affine* __restrict__ out) {
+  Fq pre[SRS_PER];
+  Fq acc = fq_one();
+  for (int i = 0; i < cnt; i++) {
+    pre[i] = acc;
+    Fq d = xyzz_is_identity(pts[i]) ? fq_one() : fq_mul(pts[i].zz, pts[i].zzz);
+    acc = fq_mul(acc, d);
+  }
+  Fq inv = fq_inv(acc);
+  for (int i = cnt - 1; i >= 0; i--) {
+    G1Affine r;
+    if (xyzz_is_identity(pts[i])) {
+      r.x = fq_zero();
+      r.y = fq_zero();
+    } else {
+      Fq d = fq_mul(pts[i].zz, pts[i].zzz);
+      Fq di = fq_mul(inv, pre[i]);  // 1 / (zz zzz)
+      inv = fq_mul(inv, d);
+      r.x = fq_mul(pts[i].x, fq_mul(di, pts[i].zzz));  // X / ZZ
+      r.y = fq_mul(pts[i].y, fq_mul(di, pts[i].zz));   // Y / ZZZ
+    }
+    fq_store(&out[i].x, r.x);
+    fq_store(&out[i].y, r.y);
+  }
+}
+
 __global__ void __launch_bounds__(64) k_srs_generate(const G1Affine* __restrict__ table, Fr tau, size_t len,
                                                      G1Affine* __restrict__ out) {
   size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -77,30 +106,7 @@ __global__ void __launch_bounds__(64) k_srs_generate(const G1Affine* __restrict_
     pts[i] = acc;
     power = fr_mul(power, tau);
   }
-  // shared inversion of zz*zzz
-  Fq pre[SRS_PER];
-  Fq acc = fq_one();
-  for (int i = 0; i < cnt; i++) {
-    pre[i] = acc;
-    Fq d = xyzz_is_identity(pts[i]) ? fq_one() : fq_mul(pts[i].zz, pts[i].zzz);
-    acc = fq_mul(acc, d);
-  }
-  Fq inv = fq_inv(acc);
-  for (int i = cnt - 1; i >= 0; i--) {
-    G1Affine r;
-    if (xyzz_is_identity(pts[i])) {
-      r.x = fq_zero();
-      r.y = fq_zero();
-    } else {
-      Fq d = fq_mul(pts[i].zz, pts[i].zzz);
-      Fq di = fq_mul(inv, pre[i]);  // 1 / (zz zzz)
-      inv = fq_mul(inv, d);
-      r.x = fq_mul(pts[i].x, fq_mul(di, pts[i].zzz));  // X / ZZ
-      r.y = fq_mul(pts[i].y, fq_mul(di, pts[i].zz));   // Y / ZZZ
-    }
-    fq_store(&out[lo + i].x, r.x);
-    fq_store(&out[lo + i].y, r.y);
-  }
+  store_affine(pts, cnt, out + lo);
 }
 
 // Fixed-base window tables: level k+1 = 2^c * level k.  Every thread doubles SRS_PER consecutive
@@ -121,29 +127,41 @@ __global__ void __launch_bounds__(64) k_srs_next_level(const G1Affine* __restric
     }
     pts[i] = acc;
   }
-  Fq pre[SRS_PER];
-  Fq acc = fq_one();
+  store_affine(pts, cnt, out + lo);
+}
+
+// One powers-of-tau contribution: out[i] = [s^i] in[i].  Every thread takes SRS_PER consecutive points (one pow, then a
+// multiply chain for the scalars), runs an MSB-first XYZZ double-and-add from each affine point -- the ladder of
+// g1_in_subgroup, ~254 doublings and ~127 mixed additions for a random scalar -- and normalises its results with one
+// shared inversion.  An input identity stays the identity; s^0 = 1 leaves in[0] as it is.
+__global__ void __launch_bounds__(64) k_srs_contribute(const G1Affine* __restrict__ in, Fr s, size_t len,
+                                                       G1Affine* __restrict__ out) {
+  size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  size_t lo = t * SRS_PER;
+  if (lo >= len) return;
+  int cnt = (int)(lo + SRS_PER < len ? SRS_PER : len - lo);
+  G1Xyzz pts[SRS_PER];
+  Fr power = fr_pow_u64(s, (unsigned long long)lo);
   for (int i = 0; i < cnt; i++) {
-    pre[i] = acc;
-    Fq d = xyzz_is_identity(pts[i]) ? fq_one() : fq_mul(pts[i].zz, pts[i].zzz);
-    acc = fq_mul(acc, d);
-  }
-  Fq inv = fq_inv(acc);
-  for (int i = cnt - 1; i >= 0; i--) {
-    G1Affine r;
-    if (xyzz_is_identity(pts[i])) {
-      r.x = fq_zero();
-      r.y = fq_zero();
-    } else {
-      Fq d = fq_mul(pts[i].zz, pts[i].zzz);
-      Fq di = fq_mul(inv, pre[i]);  // 1 / (zz zzz)
-      inv = fq_mul(inv, d);
-      r.x = fq_mul(pts[i].x, fq_mul(di, pts[i].zzz));  // X / ZZ
-      r.y = fq_mul(pts[i].y, fq_mul(di, pts[i].zz));   // Y / ZZZ
+    Fr k = fr_from_mont(power);
+    power = fr_mul(power, s);
+    G1Affine p = affine_load(in + lo + i);
+    G1Xyzz acc = xyzz_identity();
+    int top = 7;
+    while (top >= 0 && k.v[top] == 0) top--;
+    if (top >= 0 && !affine_is_identity(p)) {
+      acc.x = p.x;
+      acc.y = p.y;
+      acc.zz = fq_one();
+      acc.zzz = fq_one();
+      for (int bit = top * 32 + 30 - __clz(k.v[top]); bit >= 0; bit--) {   // below the leading one
+        xyzz_dbl(acc);
+        if ((k.v[bit >> 5] >> (bit & 31)) & 1) xyzz_madd(acc, p, false);
+      }
     }
-    fq_store(&out[lo + i].x, r.x);
-    fq_store(&out[lo + i].y, r.y);
+    pts[i] = acc;
   }
+  store_affine(pts, cnt, out + lo);
 }
 
 int srs_build_levels_dev(tp_ctx* ctx, tp_srs* srs) {
@@ -163,6 +181,14 @@ int srs_generate_dev(tp_ctx* ctx, const tph::HFr& tau, size_t len, G1Affine* out
   k_srs_generate<<<(unsigned)((nth + 63) / 64), 64, 0, ctx->stream>>>((const G1Affine*)ctx->fixed_base, to_dev(tau), len,
                                                                     out);
   TP_LAUNCH(ctx, "k_srs_generate");
+  return TP_OK;
+}
+
+int srs_contribute_dev(tp_ctx* ctx, const G1Affine* in, const tph::HFr& s, size_t len, G1Affine* out) {
+  if (len == 0) return TP_OK;
+  size_t nth = (len + SRS_PER - 1) / SRS_PER;
+  k_srs_contribute<<<(unsigned)((nth + 63) / 64), 64, 0, ctx->stream>>>(in, to_dev(s), len, out);
+  TP_LAUNCH(ctx, "k_srs_contribute");
   return TP_OK;
 }
 

@@ -102,6 +102,20 @@ __global__ void __launch_bounds__(128) k_subgroup_flags(const G1Affine* __restri
     ok[i] = g1_in_subgroup(affine_load(pts + i)) ? 1 : 0;
 }
 
+}  // namespace
+
+// An all-zero record (the device's infinity) gets 0: from (0, 0, 1, 1) every doubling gives the identity and every
+// mixed addition (0, 0, 1, 1) again, and the ladder of the odd r ends with an addition.
+int tp::subgroup_flags_dev(tp_ctx* ctx, const G1Affine* pts, size_t len, uint8_t* ok_dev) {
+  if (len == 0) return TP_OK;
+  const size_t blocks = std::min((len + 127) / 128, (size_t)ctx->sm_count * 16);
+  k_subgroup_flags<<<(unsigned)blocks, 128, 0, ctx->stream>>>(pts, len, ok_dev);
+  TP_LAUNCH(ctx, "k_subgroup_flags");
+  return TP_OK;
+}
+
+namespace {
+
 // device scratch of one call
 struct DevMem {
   void* p = nullptr;
@@ -223,9 +237,7 @@ int verify_batch_one(tp_ctx* ctx, tp_circuit* c, const uint8_t* proofs, size_t c
       TP_TRY(dev_alloc(ctx, dpts, pts.size() * sizeof(G1Affine)));
       TP_TRY(dev_alloc(ctx, dok, pts.size()));
       TP_CUDA_OK(ctx, cudaMemcpyAsync(dpts.p, pts.data(), pts.size() * sizeof(G1Affine), cudaMemcpyHostToDevice, ctx->stream));
-      const size_t blocks = std::min((pts.size() + 127) / 128, (size_t)ctx->sm_count * 16);
-      k_subgroup_flags<<<(unsigned)blocks, 128, 0, ctx->stream>>>((const G1Affine*)dpts.p, pts.size(), (uint8_t*)dok.p);
-      TP_LAUNCH(ctx, "k_subgroup_flags");
+      TP_TRY(subgroup_flags_dev(ctx, (const G1Affine*)dpts.p, pts.size(), (uint8_t*)dok.p));
       std::vector<uint8_t> ok(pts.size());
       TP_TRY(d2h_sync(ctx, ok.data(), dok.p, ok.size()));
       std::vector<char> bad(count, 0);

@@ -43,6 +43,7 @@ SYMBOLS = [
     "tp_proof_compress", "tp_proof_decompress", "tp_proof_encoded_size_compressed", "tp_proof_encode_compressed",
     "tp_proof_decode_compressed", "tp_proofs_decompress",
     "tp_srs_serialized_size_compressed", "tp_srs_serialize_compressed", "tp_srs_deserialize_compressed",
+    "tp_srs_contribute", "tp_srs_verify", "tp_srs_update_check",
 ]
 
 COMM_ID_BYTES = 128
@@ -141,6 +142,16 @@ def pairing_check(g1s, g2s) -> bool:
     rc = lib().tp_pairing_check(_buf(b"".join(g1s)), _buf(b"".join(g2s)), C.c_size_t(len(g1s)), C.byref(ok))
     if rc != 0:
         raise TyplonkError(rc, "tp_pairing_check")
+    return bool(ok.value)
+
+
+def srs_update_check(prev_tau_g1: bytes, next_tau_g1: bytes, pubkey: bytes) -> bool:
+    """tp_srs_update_check: e(next, G2) == e(prev, pubkey) on 97-byte G1 / 193-byte G2 ABI records, with every point in
+    its prime-order group and not infinity (host only)."""
+    ok = C.c_int(0)
+    rc = lib().tp_srs_update_check(_buf(prev_tau_g1), _buf(next_tau_g1), _buf(pubkey), C.byref(ok))
+    if rc != 0:
+        raise TyplonkError(rc, "tp_srs_update_check")
     return bool(ok.value)
 
 
@@ -503,6 +514,19 @@ class Context:
         h = C.c_void_p()
         self._check(lib().tp_srs_upload(self._h, _buf(g1_xy), C.c_size_t(len(g1_xy) // 96), C.byref(h)))
         return SrsHandle(self, h)
+
+    def srs_contribute(self, srs, s_mont: bytes):
+        """tp_srs_contribute: (new SRS with g1[i] * s^i and g2s * s, pubkey [s]G2 as a 193-byte ABI record)."""
+        h = C.c_void_p()
+        pub = (C.c_char * G2_BYTES)()
+        self._check(lib().tp_srs_contribute(self._h, srs._h, _buf(s_mont), C.byref(h), pub))
+        return SrsHandle(self, h), bytes(pub)
+
+    def srs_verify(self, srs) -> bool:
+        """tp_srs_verify: is the SRS the powers of one secret (randomised pairing check, G1 subgroup checks)?"""
+        ok = C.c_int(0)
+        self._check(lib().tp_srs_verify(self._h, srs._h, C.byref(ok)))
+        return bool(ok.value)
 
     # ---- KZG / NTT / permutation ---------------------------------------------------------
     def commit(self, srs, coeffs_mont: bytes) -> bytes:

@@ -2,6 +2,8 @@
 over the CUDA library: same names, argument meaning and error behaviour, so the parity tests
 read like the reference's own tests.  Scalars/points at this level are canonical Python ints /
 affine (x, y) tuples (None = infinity)."""
+import secrets
+
 from . import field as F
 from . import ffi
 from .ffi import Context, TyplonkError  # noqa: F401
@@ -35,6 +37,25 @@ class Srs:
         if compressed:
             return cls(ctx, ctx.srs_deserialize_compressed(raw, check))
         return cls(ctx, ctx.srs_deserialize(raw, check))
+
+    def contribute(self, s=None):
+        """One powers-of-tau contribution (tp_srs_contribute) -> (new Srs, pubkey [s]G2 in the g2_ref() shape).  With
+        s = None the secret is drawn from the operating system's CSPRNG and never returned.  This Srs is unchanged."""
+        if s is None:
+            s = secrets.randbelow(F.R_MOD - 1) + 1
+        handle, pub = self.ctx.srs_contribute(self.handle, F.fr_to_bytes(s))
+        return Srs(self.ctx, handle), F.g2_from_abi(pub)
+
+    def verify(self) -> bool:
+        """tp_srs_verify: g1[i] = [t^i]G for the t with g2s = [t]G2, g2 = the G2 generator, every point in its group."""
+        return self.ctx.srs_verify(self.handle)
+
+    def verify_update(self, prev: "Srs", pubkey) -> bool:
+        """tp_srs_update_check on g1[1] of `prev` and of this SRS: was this SRS made from `prev` by the contribution
+        whose pubkey ([s]G2, g2_ref() shape) is given?"""
+        def tau_g1(srs):
+            return F.g1_to_abi(F.g1_from_packed(srs.handle.download(1, 1)))
+        return ffi.srs_update_check(tau_g1(prev), tau_g1(self), F.g2_to_abi(pubkey))
 
     def g1_ref(self, offset=0, count=None):
         raw = self.handle.download(offset, count)
