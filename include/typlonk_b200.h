@@ -308,10 +308,11 @@ int tp_verify(tp_ctx* ctx, tp_circuit* c, const uint8_t* proof, size_t proof_len
  * verdict except with probability about 2^-250.  Device groups: as tp_verify (the MSMs are sharded by bucket). */
 int tp_verify_batch(tp_ctx* ctx, tp_circuit* c, const uint8_t* proofs, size_t count,
                     const uint64_t* const* public_inputs, const size_t* n_public, int* all_ok, int* each_ok);
-/* The host half of tp_verify with every circuit-dependent value supplied by the caller, for verifiers that hold a
- * verification key instead of the circuit: the eight commitments, the domain size n (power of two), the coset
- * representatives k_i, sigma_1(zeta), sigma_2(zeta) and PI(zeta) for THIS proof's challenge point, [1]G (srs[0]) and
- * the two G2 points.  No device involved. */
+/* The host half of tp_verify with every circuit-dependent value supplied by the caller, for callers that compute
+ * sigma_1(zeta), sigma_2(zeta) and PI(zeta) themselves: the eight commitments, the domain size n (power of two), the
+ * coset representatives k_i, those three evaluations for THIS proof's challenge point, [1]G (srs[0]) and the two G2
+ * points.  No device involved.  The proof does not carry sigma_1(zeta) and sigma_2(zeta) (verify() evaluates them
+ * from the circuit, proof.rs:458-459): a verifier without the circuit uses a verification key (tp_vk_*) instead. */
 typedef struct tp_verifier_inputs {
   uint8_t fixed_commitments[5][TP_G1_BYTES];
   uint8_t sigma_commitments[3][TP_G1_BYTES];
@@ -323,6 +324,48 @@ typedef struct tp_verifier_inputs {
   uint64_t n;
 } tp_verifier_inputs;
 int tp_verify_prepared(const tp_verifier_inputs* in, const uint8_t* proof, size_t proof_len, int* ok);
+/* ---- verification keys ----------------------------------------------------------------------------------------
+ * A tp_vk holds exactly what verify() reads of a compiled circuit: n, the coset representatives k_i, the five selector
+ * and three sigma commitments, identity = srs[0], the SRS's G2 and tau G2, and sigma_1, sigma_2 in coefficient form on
+ * the device (n Fr each).  The proof does not carry sigma_1(zeta), sigma_2(zeta), so the key must hold both
+ * polynomials: it is O(n), 64n bytes (64 MiB at 2^20, 1 GiB at 2^24); sigma_3 enters only through its commitment.
+ * A key does not hold the prover's state (about 99n Fr of caches and per-proof buffers for a tp_circuit).
+ * Made on a device group, a key holds one part per rank; serialisation reads rank 0's part. */
+typedef struct tp_vk tp_vk;
+/* Export from a compiled circuit: the commitments come from the circuit's cache (one MSM on first use, as
+ * tp_verify), sigma_1 and sigma_2 are copied on the device.  The key owns its copies and outlives the circuit.
+ * An SRS without G2 points -> TP_ERR_INVALID_ARG. */
+int tp_vk_from_circuit(tp_ctx* ctx, tp_circuit* c, tp_vk** out);
+int tp_vk_destroy(tp_ctx* ctx, tp_vk* vk);
+/* Wire form, ark-serialize 0.3 uncompressed items: "TPVK" | u32 LE version = 1 | u64 n | 3 x Fr k |
+ * 9 x G1 (q_l q_r q_o q_m q_c sigma_1 sigma_2 sigma_3 identity) | G2 g2 | G2 g2s | Vec<Fr> sigma_1 | Vec<Fr> sigma_2:
+ * 1376 + 64n bytes.  The scalars are converted on the device.  Buffer too small -> TP_ERR_BUFFER_TOO_SMALL. */
+int tp_vk_serialized_size(const tp_vk* vk, size_t* bytes);
+int tp_vk_serialize(tp_ctx* ctx, const tp_vk* vk, uint8_t* out, size_t cap, size_t* written);
+/* check 0: exact length, tag and version, n a power of two in [2, 2^28], both Vec lengths == n, every scalar < r,
+ * every coordinate < q, valid flags (and both G2 points on the twist, which the pairings need); 1: + every point on
+ * its curve; 2: + the nine G1 points in the prime-order subgroup and g2, g2s in G2.  A rejected record ->
+ * TP_ERR_MALFORMED naming the field (or the sigma index) in tp_last_error.  Device groups: every rank decodes its own
+ * part. */
+int tp_vk_deserialize(tp_ctx* ctx, const uint8_t* bytes, size_t len, int check, tp_vk** out);
+/* tp_verify against a key: the same checks, the same code and the same verdict as tp_verify on the circuit the key
+ * came from, malformed-input errors included.  PI(zeta) takes two n-Fr device buffers, allocated with the key on the
+ * first non-zero public-input vector; all-zero public inputs need no device work.  A key made on another context ->
+ * TP_ERR_INVALID_ARG. */
+int tp_vk_verify(tp_ctx* ctx, tp_vk* vk, const uint8_t* proof, size_t proof_len, const uint64_t* public_inputs,
+                 size_t n_public, int* ok);
+/* tp_verify_batch over proofs of several circuits: proof k (block k of `proofs`) is checked against keys[key_of[k]].
+ * Keys may differ in n and in SRS.  sigma_1, sigma_2 of every key are evaluated at all of its proofs' points in one
+ * launch; the proofs are grouped by their key's (g2, g2s) and every group g gets its own L_g, R_g, all in one batched
+ * MSM (up to eight groups per MSM call), checked by one pairing product of 2G pairs.  The weights rho are drawn from
+ * a Blake2b-512 hash of every key (n, k, the nine G1 points, g2, g2s) and of every proof with its key index and public
+ * inputs.  Localisation, each_ok and the subgroup check as tp_verify_batch.
+ * count == 0 -> *all_ok = 1.  count > 65536, n_keys not in [1, 4096], key_of[k] >= n_keys, null pointers,
+ * n_public[k] > that key's n, an unreduced public input, a key made on another context -> TP_ERR_INVALID_ARG.
+ * Device groups: every rank runs, the MSMs are sharded by bucket, the verdict is rank 0's. */
+int tp_vk_verify_batch(tp_ctx* ctx, tp_vk* const* keys, size_t n_keys, const uint32_t* key_of, const uint8_t* proofs,
+                       size_t count, const uint64_t* const* public_inputs, const size_t* n_public, int* all_ok,
+                       int* each_ok);
 /* The challenges verify() derives from a proof (proof.rs:235-244): alpha, beta, gamma, evaluation point. */
 int tp_proof_challenges(const uint8_t* proof, size_t proof_len, uint64_t alpha[4], uint64_t beta[4], uint64_t gamma[4],
                         uint64_t point[4]);

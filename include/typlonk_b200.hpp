@@ -517,6 +517,74 @@ struct Proof {
   }
 };
 
+/// Additive API: what verify() reads of a compiled circuit (tp_vk_*): n, the cosets, the eight commitments, srs[0], the
+/// SRS's G2 points and sigma_1, sigma_2 in coefficient form, so 1376 + 64n bytes on the wire.
+class VerifyingKey {
+ public:
+  /// tp_vk_deserialize; check 0 / 1 / 2 as Srs::from_bytes.  A rejected key throws Malformed naming the field.
+  static VerifyingKey from_bytes(const Context& ctx, const std::vector<uint8_t>& raw, int check = 2) {
+    tp_vk* h = nullptr;
+    detail::check(tp_vk_deserialize(ctx.get(), raw.data(), raw.size(), check, &h), "tp_vk_deserialize", ctx.get());
+    return VerifyingKey(ctx, h);
+  }
+  std::vector<uint8_t> to_bytes() const {
+    size_t need = 0;
+    tp_vk_serialized_size(get(), &need);
+    std::vector<uint8_t> out(need);
+    detail::check(tp_vk_serialize(ctx_.get(), get(), out.data(), out.size(), nullptr), "tp_vk_serialize", ctx_.get());
+    return out;
+  }
+  /// CompiledCircuit::verify against the key (tp_vk_verify): the same verdict, and the same throws.
+  bool verify(const Proof& proof) const {
+    int ok = 0;
+    detail::check(tp_vk_verify(ctx_.get(), get(), proof.fixed.data(), proof.fixed.size(),
+                               proof.public_inputs.empty() ? nullptr : proof.public_inputs[0].limbs, proof.public_inputs.size(), &ok),
+                  "tp_vk_verify", ctx_.get());
+    return ok != 0;
+  }
+  tp_vk* get() const { return h_.get(); }
+  const Context& context() const { return ctx_; }
+
+ private:
+  template <class D>
+  friend class CompiledCircuit;
+  VerifyingKey(const Context& ctx, tp_vk* h) : ctx_(ctx) {
+    Context keep = ctx;
+    h_ = std::shared_ptr<tp_vk>(h, [keep](tp_vk* p) { tp_vk_destroy(keep.get(), p); });
+  }
+  Context ctx_;
+  std::shared_ptr<tp_vk> h_;
+};
+
+/// Additive API: proofs of several circuits in one folded check (tp_vk_verify_batch) -> per-proof verdicts.  The keys
+/// must share one context; they may differ in size and SRS.
+inline std::vector<bool> verify_batch(const std::vector<std::pair<const VerifyingKey*, const Proof*>>& pairs) {
+  if (pairs.empty()) return {};
+  std::vector<tp_vk*> keys;
+  std::vector<uint32_t> key_of(pairs.size());
+  std::vector<uint8_t> blob(pairs.size() * TP_PROOF_FIXED_BYTES);
+  std::vector<const uint64_t*> pis(pairs.size());
+  std::vector<size_t> npub(pairs.size());
+  for (size_t k = 0; k < pairs.size(); k++) {
+    tp_vk* h = pairs[k].first->get();
+    size_t j = 0;
+    while (j < keys.size() && keys[j] != h) j++;
+    if (j == keys.size()) keys.push_back(h);
+    key_of[k] = (uint32_t)j;
+    const Proof& p = *pairs[k].second;
+    std::memcpy(blob.data() + k * TP_PROOF_FIXED_BYTES, p.fixed.data(), TP_PROOF_FIXED_BYTES);
+    pis[k] = p.public_inputs.empty() ? nullptr : p.public_inputs[0].limbs;
+    npub[k] = p.public_inputs.size();
+  }
+  tp_ctx* ctx = pairs[0].first->context().get();
+  int all_ok = 0;
+  std::vector<int> each(pairs.size());
+  detail::check(tp_vk_verify_batch(ctx, keys.data(), keys.size(), key_of.data(), blob.data(), pairs.size(), pis.data(),
+                                   npub.data(), &all_ok, each.data()),
+                "tp_vk_verify_batch", ctx);
+  return std::vector<bool>(each.begin(), each.end());
+}
+
 /// plonk/src/lib.rs:18-35.  DESC provides `static constexpr size_t INPUTS` and
 /// `template <class V> static void run(std::array<V, INPUTS>)` (description.rs:4-9).
 template <class DESC>
@@ -614,6 +682,12 @@ class CompiledCircuit {
                                   each.data()),
                   "tp_verify_batch", ctx_.get());
     return std::vector<bool>(each.begin(), each.end());
+  }
+  /// Additive API: the circuit's verification key (tp_vk_from_circuit); it outlives the circuit.
+  VerifyingKey verifying_key() const {
+    tp_vk* h = nullptr;
+    detail::check(tp_vk_from_circuit(ctx_.get(), circuit_.get(), &h), "tp_vk_from_circuit", ctx_.get());
+    return VerifyingKey(ctx_, h);
   }
   const Srs& srs() const { return *srs_; }
   tp_circuit* get() const { return circuit_.get(); }

@@ -15,7 +15,7 @@ ROOT = Path(__file__).resolve().parent
 CSRC = ROOT / "csrc"
 LIBDIR = ROOT / "lib"
 LIB = LIBDIR / "libtyplonk_b200.so"
-SOURCES = ["api.cu", "comm.cu", "ntt.cu", "msm.cu", "poly.cu", "prove_batch.cu", "srs.cu", "srs_ceremony.cu", "selftest.cu", "verify.cu", "verify_batch.cu", "wire.cu", "trace.cpp"]
+SOURCES = ["api.cu", "comm.cu", "ntt.cu", "msm.cu", "poly.cu", "prove_batch.cu", "srs.cu", "srs_ceremony.cu", "selftest.cu", "verify.cu", "verify_batch.cu", "verify_key.cu", "wire.cu", "trace.cpp"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

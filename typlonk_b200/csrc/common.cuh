@@ -314,6 +314,9 @@ int srs_group_new(tp_ctx* group, tp_srs** out, const std::function<int(tp_ctx*, 
 int g1_to_wire_dev(tp_ctx* ctx, const G1Affine* in, size_t len, void* out_dev);
 int g1_from_wire_dev(tp_ctx* ctx, const void* in_dev, size_t len, int check, G1Affine* out, size_t* rejected,
                      size_t* first_rejected);
+// wire.cu: Montgomery Fr <-> 32-byte canonical records (in_dev / out_dev 16-byte aligned); a record >= r is rejected
+int fr_to_wire_dev(tp_ctx* ctx, const Fr* in, size_t len, void* out_dev);
+int fr_from_wire_dev(tp_ctx* ctx, const void* in_dev, size_t len, Fr* out, size_t* rejected, size_t* first_rejected);
 // srs.cu
 int srs_generate_dev(tp_ctx* ctx, const tph::HFr& tau, size_t len, G1Affine* out);
 int srs_build_levels_dev(tp_ctx* ctx, tp_srs* srs);

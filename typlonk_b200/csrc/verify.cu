@@ -208,6 +208,68 @@ int circuit_verifier_values(tp_ctx* ctx, tp_circuit* c, VerifierValues* v) {
   return TP_OK;
 }
 
+int circuit_view(tp_ctx* ctx, tp_circuit* c, VerifierView* view) {
+  TP_TRY(circuit_verifier_values(ctx, c, &view->v));
+  view->log_n = c->log_n;
+  memcpy(view->com, c->fixed_com, sizeof(c->fixed_com));
+  memcpy(view->com + 5, c->sigma_com, sizeof(c->sigma_com));
+  view->sig_coef[0] = c->sig_coef[0];
+  view->sig_coef[1] = c->sig_coef[1];
+  view->sp = (const SrsPairing*)c->srs->pairing;
+  // the prover's public-input buffers
+  view->pi_scratch = [c](Fr** eval, Fr** coef) -> int {
+    c->pi_buffers_zero = false;
+    *eval = c->pi_eval;
+    *coef = c->pi_coef;
+    return TP_OK;
+  };
+  return TP_OK;
+}
+
+int verify_single(tp_ctx* ctx, size_t n, bool have_g2, const std::function<int(VerifierView*)>& make_view,
+                  const uint8_t* proof, size_t proof_len, const uint64_t* public_inputs, size_t n_public, int* ok) {
+  if (proof_len < TP_PROOF_FIXED_BYTES) return fail(ctx, TP_ERR_INVALID_ARG, "verify: proof shorter than the fixed block");
+  if (!have_g2) return fail(ctx, TP_ERR_INVALID_ARG, "verify: the SRS has no G2 points (tp_srs_set_g2)");
+  *ok = 0;
+  // the same bound the prover enforces (prove_from_host); Montgomery limbs must be reduced
+  if (n_public > n) return fail(ctx, TP_ERR_INVALID_ARG, "verify: more public inputs than rows");
+  bool pi_zero = true;
+  for (size_t i = 0; i < n_public; i++) {
+    if (ge<4>(public_inputs + 4 * i, FR_PARAMS.mod)) return fail(ctx, TP_ERR_INVALID_ARG, "verify: public input not reduced modulo r");
+    for (int j = 0; j < 4; j++) pi_zero &= public_inputs[4 * i + j] == 0;
+  }
+  ParsedProof p;
+  if (!parse_proof(proof, &p)) return fail(ctx, TP_ERR_INVALID_ARG, "verify: non-canonical field element in the proof");
+  if (!points_on_curve(p)) return TP_OK;
+  VerifierView view;
+  TP_TRY(make_view(&view));
+  VerifierValues& v = view.v;
+  // sigma_1, sigma_2 and the public inputs resized to n (proof.rs:204-205), interpolated, at the proof's point (the
+  // point is checked against the re-derived challenge on the host side; a mismatch rejects before these are used).
+  // All-zero public inputs give PI = 0 without device work.
+  {
+    const Fr* polys[3] = {view.sig_coef[0], view.sig_coef[1], nullptr};
+    Fr* quots[3] = {nullptr, nullptr, nullptr};
+    Fr points[3] = {to_dev(p.point), to_dev(p.point), to_dev(p.point)};
+    HFr ys[3];
+    v.public_eval = HFr::zero();
+    if (!pi_zero) {
+      Fr *eval, *coef;
+      TP_TRY(view.pi_scratch(&eval, &coef));
+      TP_CUDA_OK(ctx, cudaMemsetAsync(eval, 0, n * sizeof(Fr), ctx->stream));
+      TP_CUDA_OK(ctx, cudaMemcpyAsync(eval, public_inputs, n_public * sizeof(Fr), cudaMemcpyHostToDevice, ctx->stream));
+      TP_TRY(ntt_dev(ctx, eval, coef, view.log_n, true, nullptr));
+      polys[2] = coef;
+    }
+    TP_TRY(poly_open_batch_dev(ctx, polys, n, points, quots, pi_zero ? 2 : 3, ys));
+    v.sigma_bar[0] = ys[0];
+    v.sigma_bar[1] = ys[1];
+    if (!pi_zero) v.public_eval = ys[2];
+  }
+  *ok = verify_host(*view.sp, v, p) ? 1 : 0;
+  return TP_OK;
+}
+
 }  // namespace tpv
 
 namespace {
@@ -352,38 +414,8 @@ int tp_verify(tp_ctx* ctx, tp_circuit* c, const uint8_t* proof, size_t proof_len
     *ok = oks[0];
     return TP_OK;
   }
-  if (proof_len < TP_PROOF_FIXED_BYTES) return fail(ctx, TP_ERR_INVALID_ARG, "verify: proof shorter than the fixed block");
-  if (!c->srs->pairing) return fail(ctx, TP_ERR_INVALID_ARG, "verify: the SRS has no G2 points (tp_srs_set_g2)");
-  *ok = 0;
-  // the same bound the prover enforces (prove_from_host); Montgomery limbs must be reduced
-  if (n_public > c->n) return fail(ctx, TP_ERR_INVALID_ARG, "verify: more public inputs than rows");
-  for (size_t i = 0; i < n_public; i++)
-    if (ge<4>(public_inputs + 4 * i, FR_PARAMS.mod)) return fail(ctx, TP_ERR_INVALID_ARG, "verify: public input not reduced modulo r");
-  ParsedProof p;
-  if (!parse_proof(proof, &p)) return fail(ctx, TP_ERR_INVALID_ARG, "verify: non-canonical field element in the proof");
-  if (!points_on_curve(p)) return TP_OK;
-  const size_t n = c->n;
-  VerifierValues v;
-  TP_TRY(circuit_verifier_values(ctx, c, &v));
-  // public inputs resized to n (proof.rs:204-205), interpolated, evaluated at the proof's point together with sigma_1, sigma_2
-  // (the point is checked against the re-derived challenge on the host side; a mismatch rejects before these are used)
-  {
-    size_t take = n_public < n ? n_public : n;
-    TP_CUDA_OK(ctx, cudaMemsetAsync(c->pi_eval, 0, n * sizeof(Fr), ctx->stream));
-    if (take) TP_CUDA_OK(ctx, cudaMemcpyAsync(c->pi_eval, public_inputs, take * sizeof(Fr), cudaMemcpyHostToDevice, ctx->stream));
-    c->pi_buffers_zero = false;
-    TP_TRY(ntt_dev(ctx, c->pi_eval, c->pi_coef, c->log_n, true, nullptr));
-    const Fr* polys[3] = {c->pi_coef, c->sig_coef[0], c->sig_coef[1]};
-    Fr* quots[3] = {nullptr, nullptr, nullptr};
-    Fr points[3] = {to_dev(p.point), to_dev(p.point), to_dev(p.point)};
-    HFr ys[3];
-    TP_TRY(poly_open_batch_dev(ctx, polys, n, points, quots, 3, ys));
-    v.public_eval = ys[0];
-    v.sigma_bar[0] = ys[1];
-    v.sigma_bar[1] = ys[2];
-  }
-  *ok = verify_host(*(const SrsPairing*)c->srs->pairing, v, p) ? 1 : 0;
-  return TP_OK;
+  return verify_single(ctx, c->n, c->srs->pairing != nullptr, [&](VerifierView* view) { return circuit_view(ctx, c, view); },
+                       proof, proof_len, public_inputs, n_public, ok);
 }
 
 }  // extern "C"

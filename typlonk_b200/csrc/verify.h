@@ -2,6 +2,8 @@
 // Fiat-Shamir challenges, the circuit's verifier values, the scalars of the linearisation commitment and the host half
 // of one proof's check.
 #pragma once
+#include <functional>
+
 #include "circuit.h"
 #include "pairing.h"
 
@@ -48,4 +50,34 @@ HFr l0_denominator(uint64_t n, const HFr& zeta);
 // proof.rs:195-233 after the device work (sigma_bar and public_eval of v are this proof's)
 bool verify_host(const SrsPairing& sp, const VerifierValues& v, const ParsedProof& p);
 
+// Everything the device half of the verifier reads, built from a circuit (circuit_view) or from a verification key
+// (verify_key.cu), so that both run the same code.
+struct VerifierView {
+  VerifierValues v;                 // fixed / sigma / identity / k / n (sigma_bar and public_eval are per proof)
+  unsigned log_n;
+  uint8_t com[8][TP_G1_BYTES];      // q_l q_r q_o q_m q_c sigma_1 sigma_2 sigma_3 as ABI records
+  const tp::Fr* sig_coef[2];        // sigma_1, sigma_2 coefficients on the device, n each
+  const SrsPairing* sp;
+  // two n-Fr device buffers for PI(zeta) (pad, interpolate, evaluate); asked for only when a public input is non-zero
+  std::function<int(tp::Fr** eval, tp::Fr** coef)> pi_scratch;
+};
+int circuit_view(tp_ctx* ctx, tp_circuit* c, VerifierView* view);
+
+// tp_verify after a device group's fan-out: argument checks, parsing, then the device evaluations and verify_host over
+// the view (made only once the proof has parsed and its points are on the curve).
+int verify_single(tp_ctx* ctx, size_t n, bool have_g2, const std::function<int(VerifierView*)>& make_view,
+                  const uint8_t* proof, size_t proof_len, const uint64_t* public_inputs, size_t n_public, int* ok);
+
+// tp_verify_batch over several views: proof k is checked against views[view_of[k]] (view_of NULL: every proof against
+// views[0]).  keys_hash: the rho of tp_vk_verify_batch (keys-v1 tag, every key bound) instead of tp_verify_batch's.
+int verify_batch_views(tp_ctx* ctx, const VerifierView* views, size_t n_views, const uint32_t* view_of, bool keys_hash,
+                       const uint8_t* proofs, size_t count, const uint64_t* const* public_inputs, const size_t* n_public,
+                       int* all_ok, int* each_ok);
+
 }  // namespace tpv
+
+namespace tp {
+// wire.cu: G2 records of the ark-serialize 0.3 uncompressed encoding (check as tp_srs_deserialize)
+void g2_to_wire(const tph::G2Aff& p, uint8_t out[TP_WIRE_G2_BYTES]);
+bool g2_from_wire(const uint8_t in[TP_WIRE_G2_BYTES], int check, tph::G2Aff* out);
+}  // namespace tp

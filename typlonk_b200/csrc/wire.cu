@@ -213,10 +213,64 @@ __global__ void __launch_bounds__(128) k_g1_from_wire_compressed(const uint4* __
   }
 }
 
+// ---- Fr records (32 B little-endian canonical) ---------------------------------------------------------------------
+// Montgomery scalars -> wire records, one scalar per thread as two 16-byte loads and stores.
+__global__ void __launch_bounds__(128) k_fr_to_wire(const Fr* __restrict__ in, size_t len, Fr* __restrict__ out) {
+  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < len; i += (size_t)gridDim.x * blockDim.x)
+    fr_store(out + i, fr_from_mont(fr_load(in + i)));
+}
+
+// Wire records -> Montgomery scalars; a record >= r is rejected (its slot gets zero).  bad[] as in k_g1_from_wire.
+__global__ void __launch_bounds__(128) k_fr_from_wire(const Fr* __restrict__ in, size_t len, Fr* __restrict__ out,
+                                                      unsigned long long* __restrict__ bad) {
+  const uint32_t m[8] = TP_FR_MOD, r2c[8] = TP_FR_R2;
+  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < len; i += (size_t)gridDim.x * blockDim.x) {
+    const Fr a = fr_load(in + i);
+    bool lt = false;
+    for (int k = 7; k >= 0; k--) {
+      if (a.v[k] != m[k]) {
+        lt = a.v[k] < m[k];
+        break;
+      }
+    }
+    Fr r2;
+#pragma unroll
+    for (int k = 0; k < 8; k++) r2.v[k] = r2c[k];
+    fr_store(out + i, lt ? fr_mul(a, r2) : fr_zero());
+    if (!lt) {
+      atomicAdd(bad, 1ull);
+      atomicMin(bad + 1, (unsigned long long)i + 1);
+    }
+  }
+}
+
 static unsigned wire_grid(tp_ctx* ctx, size_t len) {
   size_t blocks = (len + 127) / 128;
   size_t cap = (size_t)ctx->sm_count * 16;
   return (unsigned)(blocks < cap ? (blocks ? blocks : 1) : cap);
+}
+
+int fr_to_wire_dev(tp_ctx* ctx, const Fr* in, size_t len, void* out_dev) {
+  if (!len) return TP_OK;
+  k_fr_to_wire<<<wire_grid(ctx, len), 128, 0, ctx->stream>>>(in, len, (Fr*)out_dev);
+  TP_LAUNCH(ctx, "k_fr_to_wire");
+  return TP_OK;
+}
+
+int fr_from_wire_dev(tp_ctx* ctx, const void* in_dev, size_t len, Fr* out, size_t* rejected, size_t* first_rejected) {
+  *rejected = 0;
+  *first_rejected = 0;
+  if (!len) return TP_OK;
+  TP_TRY(ensure(ctx, ctx->flag, 16));
+  unsigned long long init[2] = {0, ~0ull}, got[2];
+  TP_CUDA_OK(ctx, cudaMemcpyAsync(ctx->flag.p, init, 16, cudaMemcpyHostToDevice, ctx->stream));
+  k_fr_from_wire<<<wire_grid(ctx, len), 128, 0, ctx->stream>>>((const Fr*)in_dev, len, out, (unsigned long long*)ctx->flag.p);
+  TP_LAUNCH(ctx, "k_fr_from_wire");
+  TP_CUDA_OK(ctx, cudaMemcpyAsync(got, ctx->flag.p, 16, cudaMemcpyDeviceToHost, ctx->stream));
+  TP_CUDA_OK(ctx, cudaStreamSynchronize(ctx->stream));
+  *rejected = (size_t)got[0];
+  *first_rejected = got[0] ? (size_t)(got[1] - 1) : 0;
+  return TP_OK;
 }
 
 int g1_to_wire_dev(tp_ctx* ctx, const G1Affine* in, size_t len, void* out_dev) {

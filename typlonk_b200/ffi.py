@@ -44,6 +44,8 @@ SYMBOLS = [
     "tp_proof_decode_compressed", "tp_proofs_decompress",
     "tp_srs_serialized_size_compressed", "tp_srs_serialize_compressed", "tp_srs_deserialize_compressed",
     "tp_srs_contribute", "tp_srs_verify", "tp_srs_update_check",
+    "tp_vk_from_circuit", "tp_vk_destroy", "tp_vk_serialized_size", "tp_vk_serialize", "tp_vk_deserialize",
+    "tp_vk_verify", "tp_vk_verify_batch",
 ]
 
 COMM_ID_BYTES = 128
@@ -609,6 +611,35 @@ class Context:
         self._check(rc)
         return SrsHandle(self, h)
 
+    def vk_deserialize(self, raw, check=2):
+        """tp_vk_deserialize: a verification key's bytes (1376 + 64n) -> device key.  check: 0 canonical encoding and
+        framing, 1 + points on their curves, 2 + prime-order subgroups.  Raises Malformed naming the field."""
+        h = C.c_void_p()
+        rc = lib().tp_vk_deserialize(self._h, _buf(raw), C.c_size_t(len(raw)), C.c_int(check), C.byref(h))
+        if rc == 12:
+            raise Malformed(rc, lib().tp_last_error(self._h).decode())
+        self._check(rc)
+        return VerifyingKeyHandle(self, h)
+
+    def vk_verify_batch(self, keys, key_of, proofs_fixed, public_inputs):
+        """tp_vk_verify_batch: proof k (a 1472-byte block) against keys[key_of[k]], public_inputs[k] its Montgomery
+        public-input bytes (b"" = none).  Returns (every proof accepted, per-proof verdicts)."""
+        count = len(proofs_fixed)
+        assert len(public_inputs) == count and len(key_of) == count
+        if any(len(p) != PROOF_FIXED_BYTES for p in proofs_fixed):
+            raise TyplonkError(1, "vk_verify_batch: every proof must be a %d-byte block" % PROOF_FIXED_BYTES)
+        hs = (C.c_void_p * max(len(keys), 1))(*[k._h for k in keys])
+        kof = (C.c_uint32 * max(count, 1))(*key_of)
+        blob = b"".join(proofs_fixed)
+        keep = [(C.c_char * len(b)).from_buffer_copy(b) if b else None for b in public_inputs]
+        pis = (C.c_void_p * max(count, 1))(*[C.cast(b, C.c_void_p) if b is not None else None for b in keep])
+        npub = (C.c_size_t * max(count, 1))(*[len(b) // 32 for b in public_inputs])
+        each = (C.c_int * max(count, 1))()
+        all_ok = C.c_int(0)
+        self._check(lib().tp_vk_verify_batch(self._h, hs, C.c_size_t(len(keys)), kof, _buf(blob) if count else None,
+                                             C.c_size_t(count), pis, npub, C.byref(all_ok), each))
+        return bool(all_ok.value), [bool(each[k]) for k in range(count)]
+
     def proofs_decompress(self, blocks: bytes, count: int):
         """tp_proofs_decompress: `count` contiguous 848-byte blocks -> (count x 1472-byte blocks as one bytes object,
         per-block statuses: 0 = TP_OK, 12 = TP_ERR_MALFORMED with the block zero-filled)."""
@@ -754,6 +785,12 @@ class CircuitHandle:
                                               pis, npub, C.byref(all_ok), each))
         return bool(all_ok.value), [bool(each[k]) for k in range(count)]
 
+    def verifying_key(self):
+        """tp_vk_from_circuit: the circuit's verification key (owns its copies; outlives the circuit)."""
+        h = C.c_void_p()
+        self.ctx._check(lib().tp_vk_from_circuit(self.ctx._h, self._h, C.byref(h)))
+        return VerifyingKeyHandle(self.ctx, h)
+
     POLY_QUOTIENT, POLY_LINEARISATION, POLY_Z_EVALS, POLY_Z, POLY_A, POLY_B, POLY_C = range(7)
 
     def read_poly(self, which: int) -> bytes:
@@ -774,3 +811,42 @@ class CircuitHandle:
         if self._h:
             lib().tp_circuit_destroy(self.ctx._h, self._h)
             self._h = C.c_void_p()
+
+
+class VerifyingKeyHandle:
+    """A tp_vk: what verify() reads of a compiled circuit (include/typlonk_b200.h, "verification keys")."""
+
+    def __init__(self, ctx, h):
+        self.ctx = ctx
+        self._h = h
+
+    def serialized_size(self) -> int:
+        need = C.c_size_t(0)
+        lib().tp_vk_serialized_size(self._h, C.byref(need))
+        return need.value
+
+    def serialize(self) -> bytearray:
+        """tp_vk_serialize: "TPVK" | u32 1 | u64 n | 3 Fr | 9 G1 | 2 G2 | Vec<Fr> sigma_1 | Vec<Fr> sigma_2."""
+        out = bytearray(self.serialized_size())
+        self.ctx._check(lib().tp_vk_serialize(self.ctx._h, self._h, _buf(out), C.c_size_t(len(out)), None))
+        return out
+
+    def verify(self, proof_fixed: bytes, public_inputs_mont: bytes) -> bool:
+        """tp_vk_verify: tp_verify's verdict (and errors) for the circuit the key came from."""
+        ok = C.c_int(0)
+        self.ctx._check(lib().tp_vk_verify(self.ctx._h, self._h, _buf(proof_fixed), C.c_size_t(len(proof_fixed)),
+                                           _buf(public_inputs_mont) if public_inputs_mont else None,
+                                           C.c_size_t(len(public_inputs_mont) // 32), C.byref(ok)))
+        return bool(ok.value)
+
+    def destroy(self):
+        if self._h:
+            lib().tp_vk_destroy(self.ctx._h, self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            if self._h and self.ctx._h:
+                self.destroy()
+        except Exception:
+            pass

@@ -25,7 +25,7 @@ its circuit-sized parts on the device and the pairings on the host inside the li
 """
 import struct
 from dataclasses import dataclass
-from typing import List
+from typing import List, Tuple
 
 from . import field as F
 from .ffi import (Context, GateUnsatisfied, TyplonkError, PROOF_FIXED_BYTES, GATE_ADD, GATE_MUL, Trace,  # noqa: F401
@@ -139,6 +139,54 @@ class CompiledCircuit:
         """Every proof of this circuit checked at once (tp_verify_batch): (all accepted, per-proof verdicts).  Stricter
         than `verify` on points outside the prime-order subgroup, which it rejects."""
         return self.handle.verify_batch([p.fixed for p in proofs], [F.fr_vec_to_bytes(p.public_inputs) for p in proofs])
+
+    def verifying_key(self) -> "VerifyingKey":
+        """What `verify` reads of this circuit, without the prover's state (tp_vk_from_circuit); it stays valid after
+        the circuit is destroyed."""
+        return VerifyingKey(self.handle.verifying_key())
+
+
+class VerifyingKey:
+    """A verification key: n, the coset representatives, the eight circuit commitments, srs[0], the SRS's two G2
+    points and sigma_1, sigma_2 in coefficient form (the proof does not carry their values at the challenge point), so
+    1376 + 64n bytes on the wire."""
+
+    def __init__(self, handle):
+        self.handle = handle
+
+    @property
+    def ctx(self):
+        return self.handle.ctx
+
+    def to_bytes(self) -> bytes:
+        """tp_vk_serialize."""
+        return bytes(self.handle.serialize())
+
+    @classmethod
+    def from_bytes(cls, ctx: Context, raw: bytes, check=2) -> "VerifyingKey":
+        """tp_vk_deserialize (check 0: encoding and framing, 1: + on the curve, 2: + prime-order subgroups); raises
+        ffi.Malformed naming the rejected field."""
+        return cls(ctx.vk_deserialize(raw, check))
+
+    def verify(self, proof: Proof) -> bool:
+        """CompiledCircuit::verify against the key (tp_vk_verify): the verdict `CompiledCircuit.verify` gives."""
+        return self.handle.verify(proof.fixed, F.fr_vec_to_bytes(proof.public_inputs))
+
+
+def verify_batch(pairs: List[Tuple[VerifyingKey, Proof]]) -> Tuple[bool, List[bool]]:
+    """Proofs of several circuits in one folded check (tp_vk_verify_batch): (all accepted, per-proof verdicts).  Every
+    key must belong to one context; keys of different sizes and SRSes may be mixed."""
+    if not pairs:
+        return True, []
+    keys, key_of, index = [], [], {}
+    for vk, _ in pairs:
+        if id(vk.handle) not in index:
+            index[id(vk.handle)] = len(keys)
+            keys.append(vk.handle)
+        key_of.append(index[id(vk.handle)])
+    ctx = keys[0].ctx
+    return ctx.vk_verify_batch(keys, key_of, [p.fixed for _, p in pairs],
+                               [F.fr_vec_to_bytes(p.public_inputs) for _, p in pairs])
 
 
 class CircuitDescription:
