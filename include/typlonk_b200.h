@@ -51,7 +51,8 @@ enum {
   TP_ERR_BUFFER_TOO_SMALL = 9,
   TP_ERR_INVALID_TAG = 10,       /* add_constrain(..) -> Err(()) .unwrap()   permutation/src/lib.rs:48-51, plonk/src/builder.rs:155-159 */
   TP_ERR_UNPLACED_VARIABLE = 11, /* assert!(inner.pending_eq.is_empty())     plonk/src/builder.rs:177 */
-  TP_ERR_MALFORMED = 12          /* a wire encoding that is not canonical / not on the curve */
+  TP_ERR_MALFORMED = 12,         /* a wire encoding that is not canonical / not on the curve */
+  TP_ERR_INTERNAL = 13           /* a result the library's own invariants rule out (a defect of the library, not of the input) */
 };
 
 #define TP_G1_BYTES 97
@@ -366,6 +367,58 @@ int tp_vk_verify(tp_ctx* ctx, tp_vk* vk, const uint8_t* proof, size_t proof_len,
 int tp_vk_verify_batch(tp_ctx* ctx, tp_vk* const* keys, size_t n_keys, const uint32_t* key_of, const uint8_t* proofs,
                        size_t count, const uint64_t* const* public_inputs, const size_t* n_public, int* all_ok,
                        int* each_ok);
+/* ---- proof format v2 -------------------------------------------------------------------------------------------
+ * The format above (v1) matches the reference's prove() and verify() byte for byte, and it is NOT SOUND: its
+ * challenge zeta is drawn from [a], [b], [c], [z] alone, and the quotient commitments [t0], [t1], [t2] are made after
+ * zeta is known and never hashed.  A prover who knows zeta can take t = Lin(zeta) / Z_H(zeta) as a constant, so that
+ * r(zeta) = 0 for ANY witness, and tp_verify accepts.  v1 also has no working public inputs (no gate reads them; only
+ * all-zero vectors prove).  v1 is kept for reference parity; new users should use v2 (DESIGN.md, "Proof format v2").
+ *
+ * v2: the first l inputs of a circuit are public (tp_trace_create_public puts them in public gates, rows 0..l-1,
+ * q_l = 1, PI_i = -x_i); a Blake2b-512 transcript binds the key, the public values and every commitment before each
+ * challenge; one batched KZG opening at zeta and one at zeta * omega; a 1056-byte block
+ *   [a] [b] [c] [z] [t0] [t1] [t2] [W_zeta] [W_zeta_omega] | a(zeta) b(zeta) c(zeta) s1(zeta) s2(zeta) z(zeta omega)
+ * and a constant-size key (1368 B).  Verification is host only: no context, no device. */
+#define TP_PROOF_V2_FIXED_BYTES 1056 /* 9 G1 x 96 + 6 Fr x 32 */
+#define TP_VK2_BYTES 1368
+typedef struct tp_vk2 tp_vk2;
+/* The key of circuit c with its first n_public rows public: n, l, the cosets, the five selector and three sigma
+ * commitments (the circuit's cache: one MSM on first use), srs[0], g2 and g2s (prepared for the pairing).  Host
+ * memory only; it outlives the circuit and the context.  An SRS without G2, n_public > n - 3, or rows 0..n_public-1
+ * not all public gates (q_l = 1, other selectors 0) or row n_public one too -> TP_ERR_INVALID_ARG: the key's l must be
+ * the number of public gates the circuit was traced with. */
+int tp_vk2_from_circuit(tp_ctx* ctx, tp_circuit* c, size_t n_public, tp_vk2** out);
+int tp_vk2_destroy(tp_vk2* vk);
+/* "TPK2" | u32 LE version = 1 | u64 n | u64 l | 3 x Fr k | 9 x G1 (q_l q_r q_o q_m q_c sigma_1 sigma_2 sigma_3 srs[0])
+ * | G2 g2 | G2 g2s, ark-serialize 0.3 uncompressed items: TP_VK2_BYTES.  cap < TP_VK2_BYTES -> TP_ERR_BUFFER_TOO_SMALL. */
+int tp_vk2_serialize(const tp_vk2* vk, uint8_t* out, size_t cap);
+/* check 0: exact length, tag, version, n a power of two in [4, 2^28], l <= n - 3, every scalar < r, every coordinate
+ * < q, valid flags, both G2 points on the twist; 1: + the nine G1 points on the curve; 2: + in the prime-order
+ * subgroup, g2 and g2s in G2.  A rejected field -> TP_ERR_MALFORMED; tp_vk2_last_error names it.  Host only. */
+int tp_vk2_deserialize(const uint8_t* bytes, size_t len, int check, tp_vk2** out);
+/* The reason of the last failed tp_vk2_deserialize / tp_proof_v2_decode of the calling thread. */
+const char* tp_vk2_last_error(void);
+/* Proves with c: advice = three host columns (n Montgomery Fr each, as tp_prove).  The public values are column a,
+ * rows 0..l-1 (l = the key's); they are written to public_out (l x 4 limbs, may be NULL when l = 0).  A key whose n,
+ * cosets, commitments or srs[0] are not c's -> TP_ERR_INVALID_ARG; proof_cap < TP_PROOF_V2_FIXED_BYTES ->
+ * TP_ERR_BUFFER_TOO_SMALL; a gate that fails -> TP_ERR_GATE_UNSATISFIED.  A witness that breaks a copy constraint
+ * gives a proof that tp_verify_v2 rejects; r(zeta) != 0 for a witness that meets its constraints (which the protocol
+ * rules out) -> TP_ERR_INTERNAL.  Device groups: every rank proves, rank 0's bytes go out. */
+int tp_prove_v2(tp_ctx* ctx, tp_circuit* c, const tp_vk2* vk, const uint64_t* const advice[3], uint8_t* proof_out,
+                size_t proof_cap, uint64_t* public_out);
+/* Host only.  *ok = 1 iff the TP_PROOF_V2_FIXED_BYTES block is canonical, its nine points are on the curve and in G1,
+ * n_public equals the key's l, and the pairing check holds for these public values (Montgomery limbs).
+ * proof_len != TP_PROOF_V2_FIXED_BYTES -> *ok = 0.  An unreduced public input -> TP_ERR_INVALID_ARG. */
+int tp_verify_v2(const tp_vk2* vk, const uint8_t* proof, size_t proof_len, const uint64_t* public_inputs,
+                 size_t n_public, int* ok);
+/* Wire form: the block | u64 LE l | l x Fr (32 B canonical LE).  encode: cap < 1064 + 32 l -> TP_ERR_BUFFER_TOO_SMALL
+ * (*written, if not NULL, gets the size either way).  decode: exact length, canonical scalars and coordinates, points
+ * on the curve, else TP_ERR_MALFORMED; fixed_out and public_out may be NULL (ask for *n_public first; public_cap: the
+ * values public_out holds).  Host only. */
+int tp_proof_v2_encode(const uint8_t fixed[TP_PROOF_V2_FIXED_BYTES], const uint64_t* public_inputs, size_t n_public,
+                       uint8_t* out, size_t cap, size_t* written);
+int tp_proof_v2_decode(const uint8_t* bytes, size_t len, uint8_t fixed_out[TP_PROOF_V2_FIXED_BYTES],
+                       uint64_t* public_out, size_t public_cap, size_t* n_public);
 /* The challenges verify() derives from a proof (proof.rs:235-244): alpha, beta, gamma, evaluation point. */
 int tp_proof_challenges(const uint8_t* proof, size_t proof_len, uint64_t alpha[4], uint64_t beta[4], uint64_t gamma[4],
                         uint64_t point[4]);
@@ -377,10 +430,15 @@ int tp_proof_challenges(const uint8_t* proof, size_t proof_len, uint64_t alpha[4
  * flat gate list); padding, selector columns, the copy-constraint permutation and every
  * witness are derived from it natively.  No device involved; feeds tp_circuit_compile and
  * tp_prove.  Variables are dense ids: the n_inputs inputs are 0..n_inputs-1 in order. */
-enum { TP_GATE_MUL = 0, TP_GATE_ADD = 1, TP_GATE_DUMMY = 2 }; /* plonk/src/builder.rs:30-36 */
+enum { TP_GATE_MUL = 0, TP_GATE_ADD = 1, TP_GATE_DUMMY = 2, TP_GATE_PUBLIC = 3 }; /* plonk/src/builder.rs:30-36; PUBLIC: proof format v2 */
 
 /* Context::default + BuildVar::input per input (plonk/src/builder.rs:371-377, 95-99). */
 int tp_trace_create(size_t n_inputs, tp_trace** out);
+/* tp_trace_create with the first n_public inputs public (proof format v2): public gate i (row i, i < n_public,
+ * kind TP_GATE_PUBLIC, q_l = 1, all other selectors 0) places input i at (0, i); a later use of input i gets a copy
+ * constraint like any already-placed operand.  The witness has a = x_i, b = c = 0 there.  tp_trace_gate(s) refuse the
+ * kind.  n_public > n_inputs -> TP_ERR_INVALID_ARG. */
+int tp_trace_create_public(size_t n_inputs, size_t n_public, tp_trace** out);
 int tp_trace_destroy(tp_trace* t);
 /* BuildVar::binary_operation (plonk/src/builder.rs:339-370): appends a gate row j, gives the
  * output a new id placed at (2, j), and places each operand at (0, j) / (1, j) -- an operand

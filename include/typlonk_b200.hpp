@@ -13,6 +13,8 @@
 //   plonk        CircuitDescription (run / build), Var (+, *, clone, assert_eq),
 //                CompiledCircuit::{prove, verify, rows}, Proof                  plonk/src/description.rs:4-16, lib.rs:18-35,
 //                                                                               proof.rs:26-63, 85-95
+//                (additive, proof format v2: CircuitDescription::PUBLIC, CompiledCircuit::{verifying_key_v2,
+//                prove_v2}, ProofV2, VerifyingKeyV2 -- v1 keeps reference parity and is not sound; use v2)
 //
 //   struct Pythagoras {                                   // README.md:16-27
 //     static constexpr size_t INPUTS = 3;
@@ -40,6 +42,7 @@
 #include <cstdio>
 #include <stdexcept>
 #include <string>
+#include <type_traits>
 #include <utility>
 #include <vector>
 
@@ -77,6 +80,19 @@ inline void check(int rc, const char* what, tp_ctx* ctx = nullptr) {
   throw Error(rc, msg);
 }
 /// 64 bits from the operating system's CSPRNG: getrandom(2) where it exists, else /dev/urandom.
+/// DESC::PUBLIC if the description declares it (proof format v2: its first PUBLIC inputs are public), else 0.
+template <class D, class = void>
+struct public_count : std::integral_constant<size_t, 0> {};
+template <class D>
+struct public_count<D, std::void_t<decltype(D::PUBLIC)>> : std::integral_constant<size_t, (size_t)D::PUBLIC> {};
+/// A failed host-only v2 call (no context): tp_vk2_last_error names the rejected field.
+inline void check_v2(int rc, const char* what) {
+  if (rc == TP_OK) return;
+  const char* e = tp_vk2_last_error();
+  std::string msg = std::string(what) + (e && *e ? std::string(": ") + e : std::string());
+  if (rc == TP_ERR_MALFORMED) throw Malformed(rc, msg);
+  throw Error(rc, msg);
+}
 inline uint64_t os_random_u64() {
   uint64_t v = 0;
   size_t got = 0;
@@ -556,6 +572,65 @@ class VerifyingKey {
   std::shared_ptr<tp_vk> h_;
 };
 
+/// Proof format v2 (sound; DESIGN.md, "Proof format v2"): the 1056-byte block ([a] [b] [c] [z] [t0] [t1] [t2] [W_zeta]
+/// [W_zeta_omega] | six evaluations) and the public values it proves.
+struct ProofV2 {
+  std::array<uint8_t, TP_PROOF_V2_FIXED_BYTES> fixed{};
+  std::vector<Fr> public_inputs;
+  /// tp_proof_v2_encode: the block | Vec<Fr> of the public values.
+  std::vector<uint8_t> to_bytes() const {
+    size_t need = 0;
+    const uint64_t* pis = public_inputs.empty() ? nullptr : public_inputs[0].limbs;
+    tp_proof_v2_encode(fixed.data(), pis, public_inputs.size(), nullptr, 0, &need);
+    std::vector<uint8_t> out(need);
+    detail::check(tp_proof_v2_encode(fixed.data(), pis, public_inputs.size(), out.data(), out.size(), nullptr),
+                  "tp_proof_v2_encode");
+    return out;
+  }
+  /// tp_proof_v2_decode (checked): throws Malformed naming the rejected field.
+  static ProofV2 from_bytes(const std::vector<uint8_t>& raw) {
+    ProofV2 p;
+    size_t n = 0;
+    detail::check_v2(tp_proof_v2_decode(raw.data(), raw.size(), nullptr, nullptr, 0, &n), "tp_proof_v2_decode");
+    p.public_inputs.resize(n);
+    detail::check_v2(tp_proof_v2_decode(raw.data(), raw.size(), p.fixed.data(), n ? p.public_inputs[0].limbs : nullptr, n, &n),
+                     "tp_proof_v2_decode");
+    return p;
+  }
+};
+
+/// The key of proof format v2 (tp_vk2_*): 1368 bytes in host memory; verification needs no Context and no device.
+class VerifyingKeyV2 {
+ public:
+  /// tp_vk2_deserialize; check 0 / 1 / 2 as VerifyingKey::from_bytes.  A rejected key throws Malformed naming the field.
+  static VerifyingKeyV2 from_bytes(const std::vector<uint8_t>& raw, int check = 2) {
+    tp_vk2* h = nullptr;
+    detail::check_v2(tp_vk2_deserialize(raw.data(), raw.size(), check, &h), "tp_vk2_deserialize");
+    return VerifyingKeyV2(h);
+  }
+  std::vector<uint8_t> to_bytes() const {
+    std::vector<uint8_t> out(TP_VK2_BYTES);
+    detail::check(tp_vk2_serialize(get(), out.data(), out.size()), "tp_vk2_serialize");
+    return out;
+  }
+  /// tp_verify_v2 for these public values (those the proof carries by default).
+  bool verify(const ProofV2& proof, const std::vector<Fr>* public_inputs = nullptr) const {
+    const std::vector<Fr>& pub = public_inputs ? *public_inputs : proof.public_inputs;
+    int ok = 0;
+    detail::check(tp_verify_v2(get(), proof.fixed.data(), proof.fixed.size(), pub.empty() ? nullptr : pub[0].limbs,
+                               pub.size(), &ok),
+                  "tp_verify_v2");
+    return ok != 0;
+  }
+  tp_vk2* get() const { return h_.get(); }
+
+ private:
+  template <class D>
+  friend class CompiledCircuit;
+  explicit VerifyingKeyV2(tp_vk2* h) : h_(h, [](tp_vk2* p) { tp_vk2_destroy(p); }) {}
+  std::shared_ptr<tp_vk2> h_;
+};
+
 /// Additive API: proofs of several circuits in one folded check (tp_vk_verify_batch) -> per-proof verdicts.  The keys
 /// must share one context; they may differ in size and SRS.
 inline std::vector<bool> verify_batch(const std::vector<std::pair<const VerifyingKey*, const Proof*>>& pairs) {
@@ -586,11 +661,14 @@ inline std::vector<bool> verify_batch(const std::vector<std::pair<const Verifyin
 }
 
 /// plonk/src/lib.rs:18-35.  DESC provides `static constexpr size_t INPUTS` and
-/// `template <class V> static void run(std::array<V, INPUTS>)` (description.rs:4-9).
+/// `template <class V> static void run(std::array<V, INPUTS>)` (description.rs:4-9).  It may declare
+/// `static constexpr size_t PUBLIC` (proof format v2): its first PUBLIC inputs are then public.
 template <class DESC>
 class CompiledCircuit {
  public:
   static constexpr size_t INPUTS = DESC::INPUTS;
+  static constexpr size_t PUBLIC = detail::public_count<DESC>::value;
+  static_assert(PUBLIC <= INPUTS, "PUBLIC must not exceed INPUTS");
   size_t rows = 0;
   std::array<KzgCommitment, 5> fixed_commitments;
 
@@ -689,6 +767,35 @@ class CompiledCircuit {
     detail::check(tp_vk_from_circuit(ctx_.get(), circuit_.get(), &h), "tp_vk_from_circuit", ctx_.get());
     return VerifyingKey(ctx_, h);
   }
+  /// Proof format v2: the constant-size key (tp_vk2_from_circuit), made once and shared; it outlives the circuit.
+  const VerifyingKeyV2& verifying_key_v2() const {
+    if (!vk2_) {
+      tp_vk2* h = nullptr;
+      detail::check(tp_vk2_from_circuit(ctx_.get(), circuit_.get(), PUBLIC, &h), "tp_vk2_from_circuit", ctx_.get());
+      vk2_ = std::make_shared<VerifyingKeyV2>(VerifyingKeyV2(h));
+    }
+    return *vk2_;
+  }
+  /// Proof format v2 (tp_prove_v2): sound, and bound to the first PUBLIC inputs, which it carries.  Throws
+  /// GateUnsatisfied where prove() does.
+  ProofV2 prove_v2(const std::array<Fr, INPUTS>& inputs, const std::array<Fr, 9>& blinders) const {
+    std::vector<Fr> a(rows), b(rows), c(rows);
+    uint64_t* adv[3] = {a[0].limbs, b[0].limbs, c[0].limbs};
+    detail::check(tp_trace_witness(trace_.get(), INPUTS ? inputs[0].limbs : nullptr, INPUTS, blinders[0].limbs, adv), "tp_trace_witness");
+    const uint64_t* cadv[3] = {adv[0], adv[1], adv[2]};
+    ProofV2 p;
+    p.public_inputs.resize(PUBLIC);
+    detail::check(tp_prove_v2(ctx_.get(), circuit_.get(), verifying_key_v2().get(), cadv, p.fixed.data(), p.fixed.size(),
+                              PUBLIC ? p.public_inputs[0].limbs : nullptr),
+                  "tp_prove_v2", ctx_.get());
+    return p;
+  }
+  /// ... with the blinders drawn like `Fr::rand(&mut thread_rng())`.
+  ProofV2 prove_v2(const std::array<Fr, INPUTS>& inputs) const {
+    std::array<Fr, 9> blinders;
+    for (auto& x : blinders) x = Fr::random();
+    return prove_v2(inputs, blinders);
+  }
   const Srs& srs() const { return *srs_; }
   tp_circuit* get() const { return circuit_.get(); }
 
@@ -699,7 +806,7 @@ class CompiledCircuit {
   }
   void trace() {
     tp_trace* t = nullptr;
-    detail::check(tp_trace_create(INPUTS, &t), "tp_trace_create");
+    detail::check(PUBLIC ? tp_trace_create_public(INPUTS, PUBLIC, &t) : tp_trace_create(INPUTS, &t), "tp_trace_create");
     trace_ = std::shared_ptr<tp_trace>(t, [](tp_trace* p) { tp_trace_destroy(p); });
     DESC::template run<Var>(make_inputs(std::make_index_sequence<INPUTS>{}));
     size_t gates = 0;
@@ -724,6 +831,7 @@ class CompiledCircuit {
   std::shared_ptr<tp_trace> trace_;
   std::unique_ptr<Srs> srs_;
   std::shared_ptr<tp_circuit> circuit_;
+  mutable std::shared_ptr<VerifyingKeyV2> vk2_;
 };
 
 /// `Circuit::build()` (description.rs:6-8): tau from the thread's random generator like Srs::random (builder.rs:71) ...

@@ -719,7 +719,12 @@ static int coset_owner(const tp_ctx* ctx, bool shard, unsigned first, unsigned k
 // `col_ready` (may be null): three events on another stream, one per witness column, recorded when that column's
 // upload has landed.  The prover then interpolates column k as soon as it is there -- while the next one is still
 // crossing PCIe -- instead of waiting for all three and running the batched transform.
-static int prove_resident(tp_ctx* ctx, tp_circuit* c, uint8_t* proof_out, const cudaEvent_t* col_ready = nullptr) {
+extern "C++" {
+// The stages every proof format shares, up to the quotient t: gate check, interpolation, [a], [b], [c], grand product,
+// [z], quotient (proof.rs:96-131, 292-375).  `ch` draws beta, gamma after [a] [b] [c] and alpha after [z].
+// pi_from_a > 0 (format v2): the public-input column is -a[i] for rows i < pi_from_a, zero elsewhere, built here.
+int tpp::prove_to_quotient(tp_ctx* ctx, tp_circuit* c, const cudaEvent_t* col_ready, size_t pi_from_a,
+                           ChallengeSource& ch, Round3* out) {
   const size_t n = c->n;
   const tp_srs* srs = c->srs;
   // Quotient cosets of a, b, c on the side stream, under the round-1 MSMs.  Which cosets this rank owns depends on
@@ -773,6 +778,7 @@ static int prove_resident(tp_ctx* ctx, tp_circuit* c, uint8_t* proof_out, const 
       if (side) TP_TRY(side_cosets(k, k + 1, first_guess, 0));
     }
   }
+  if (pi_from_a) TP_TRY(pi_from_column_dev(ctx, c->adv_eval[0], pi_from_a, n, c->pi_eval));
   // gate equation on every row (the reference asserts it via vanishes(line1), proof.rs:317-321) -- first, because it
   // needs nothing but the uploaded columns and also tells whether the public inputs are all zero.
   bool pi_zero = false;
@@ -829,7 +835,7 @@ static int prove_resident(tp_ctx* ctx, tp_circuit* c, uint8_t* proof_out, const 
     TP_TRY(msm_batch_dev(ctx, srs, sets, 3, n, com));
   }
   HFr beta, gamma;
-  tph::challenges2({com[0], com[1], com[2]}, &beta, &gamma);
+  ch.after_abc(com, &beta, &gamma);
   // grand product z (proof.rs:117-131); z_closes: the last value, which the reference pops (proof.rs:120), is 1
   bool z_closes = false;
   {
@@ -843,8 +849,8 @@ static int prove_resident(tp_ctx* ctx, tp_circuit* c, uint8_t* proof_out, const 
   const unsigned first = skip0 ? 1u : 0u;
   if (side) TP_TRY(side_cosets(0, 4, first, 2));   // z on this rank's cosets; a, b, c only where the guess above missed
   TP_TRY(msm_dev(ctx, srs, c->z_coef, n, com[3]));
-  HFr alpha, zeta;
-  tph::challenges2({com[0], com[1], com[2], com[3]}, &alpha, &zeta);
+  HFr alpha;
+  ch.after_z(com, &alpha);
 
   // quotient (proof.rs:292-375) on the 4n domain, coset by coset: four coset NTTs, the pointwise numerator, one
   // inverse coset NTT each.  Coset 0 is H itself, where the numerator is zero whenever the witness satisfies the gates
@@ -909,6 +915,38 @@ static int prove_resident(tp_ctx* ctx, tp_circuit* c, uint8_t* proof_out, const 
     }
     TP_TRY(quotient_combine_dev(ctx, c->buf4[0], n, 0, 1, &skip0, c->t));
   }
+  memcpy(out->com, com, sizeof(com));
+  out->alpha = alpha;
+  out->beta = beta;
+  out->gamma = gamma;
+  out->pi_zero = pi_zero;
+  out->z_closes = z_closes;
+  return TP_OK;
+}
+}  // extern "C++"
+
+namespace {
+// v1's challenges (proof.rs:235-244): beta, gamma from [a] [b] [c]; alpha and zeta together from [a] [b] [c] [z]
+struct ChallengesV1 : tpp::ChallengeSource {
+  HFr zeta;
+  void after_abc(const uint8_t com[4][TP_G1_BYTES], HFr* beta, HFr* gamma) override {
+    tph::challenges2({com[0], com[1], com[2]}, beta, gamma);
+  }
+  void after_z(const uint8_t com[4][TP_G1_BYTES], HFr* alpha) override {
+    tph::challenges2({com[0], com[1], com[2], com[3]}, alpha, &zeta);
+  }
+};
+}  // namespace
+
+static int prove_resident(tp_ctx* ctx, tp_circuit* c, uint8_t* proof_out, const cudaEvent_t* col_ready = nullptr) {
+  const size_t n = c->n;
+  const tp_srs* srs = c->srs;
+  ChallengesV1 ch;
+  tpp::Round3 st;
+  TP_TRY(tpp::prove_to_quotient(ctx, c, col_ready, 0, ch, &st));
+  const HFr alpha = st.alpha, beta = st.beta, gamma = st.gamma, zeta = ch.zeta;
+  const bool pi_zero = st.pi_zero;
+  const uint8_t(*com)[TP_G1_BYTES] = st.com;
 
   // The three t commitments (proof.rs:175,181) need nothing that follows: with the MSM pipe they are queued now and
   // accumulate while this stream computes the opening polynomials; the opening witnesses follow as two more sub-batches
@@ -1005,6 +1043,15 @@ static int prove_from_host(tp_ctx* ctx, tp_circuit* c, const uint64_t* const adv
   if (n_public > c->n) return fail(ctx, TP_ERR_INVALID_ARG, "prove: more public inputs than rows");
   if (!advice || !advice[0] || !advice[1] || !advice[2] || (n_public && !public_inputs))
     return fail(ctx, TP_ERR_INVALID_ARG, "prove: null argument");
+  return tpp::upload_and_prove(ctx, c, advice, public_inputs, n_public, [&](const cudaEvent_t* col_ready) {
+    return prove_resident(ctx, c, proof_out, col_ready);
+  });
+}
+extern "C++" {
+// The three witness columns (and the first n_public public inputs, the rest zero-filled) to the device, then
+// prove(col_ready): col_ready is null when the columns are already in place on the compute stream.
+int tpp::upload_and_prove(tp_ctx* ctx, tp_circuit* c, const uint64_t* const advice[3], const uint64_t* public_inputs,
+                          size_t n_public, const std::function<int(const cudaEvent_t*)>& prove) {
   size_t bytes = c->n * sizeof(Fr);
   const uint64_t* cols[4] = {advice[0], advice[1], advice[2], public_inputs};
   Fr* dst[4] = {c->adv_eval[0], c->adv_eval[1], c->adv_eval[2], c->pi_eval};
@@ -1041,10 +1088,11 @@ static int prove_from_host(tp_ctx* ctx, tp_circuit* c, const uint64_t* const adv
       TP_CUDA_OK(ctx, cudaEventRecord(ctx->copy_ev[j], ctx->copy_stream));
     }
     if (ncols == 4) TP_TRY(h2d(ctx, dst[3], cols[3], bytes));   // the full-length public-input column, compute stream
-    return prove_resident(ctx, c, proof_out, ctx->copy_ev);
+    return prove(ctx->copy_ev);
   }
-  return prove_resident(ctx, c, proof_out);
+  return prove(nullptr);
 }
+}  // extern "C++"
 int tp_prove(tp_ctx* ctx, tp_circuit* c, const uint64_t* const advice[3], const uint64_t* public_inputs,
              uint8_t* proof_out, size_t proof_cap) {
   return prove_from_host(ctx, c, advice, public_inputs, c ? c->n : 0, proof_out, proof_cap);

@@ -41,4 +41,7 @@ struct tp_circuit {
   bool have_fixed_com = false, have_sigma_com = false;
   uint8_t fixed_com[5][TP_G1_BYTES];
   uint8_t sigma_com[3][TP_G1_BYTES];
+  // tp_prove_v2 (prove_v2.cu): digest of the last v2 key found to be this circuit's, so the check runs once per key
+  bool have_v2_key = false;
+  uint8_t v2_key_digest[64];
 };

@@ -5,6 +5,8 @@
 #include "circuit.h"
 #include "transcript.h"
 
+#include <functional>
+
 namespace tpp {
 
 using tph::HFr;
@@ -51,6 +53,26 @@ inline void lin_scalars(const HFr k[3], const ProofEvals& e, const HFr& alpha, c
   s[R_T2] = (zh * zn * zn).neg();
   s[R_TERMS] = e.pi_bar - ab_zw * (gamma + cc) - alpha2 * l0;
 }
+
+// The driver's stages up to the quotient t (api.cu), shared by tp_prove and tp_prove_v2.  The challenge source is
+// the format's transcript: it sees [a] [b] [c] (then draws beta, gamma) and [a] [b] [c] [z] (then draws alpha).
+struct ChallengeSource {
+  virtual void after_abc(const uint8_t com[4][TP_G1_BYTES], HFr* beta, HFr* gamma) = 0;
+  virtual void after_z(const uint8_t com[4][TP_G1_BYTES], HFr* alpha) = 0;
+  virtual ~ChallengeSource() {}
+};
+struct Round3 {
+  uint8_t com[4][TP_G1_BYTES];   // a b c z
+  HFr alpha, beta, gamma;
+  bool pi_zero;                  // the public-input column is zero (pi_coef and its cosets were skipped)
+  bool z_closes;                 // the grand product closes: the witness meets the copy constraints
+};
+int prove_to_quotient(tp_ctx* ctx, tp_circuit* c, const cudaEvent_t* col_ready, size_t pi_from_a, ChallengeSource& ch,
+                      Round3* out);
+int upload_and_prove(tp_ctx* ctx, tp_circuit* c, const uint64_t* const advice[3], const uint64_t* public_inputs,
+                     size_t n_public, const std::function<int(const cudaEvent_t*)>& prove);
+// prove_v2.cu: pi[i] = -a[i] for i < ell, 0 for ell <= i < n
+int pi_from_column_dev(tp_ctx* ctx, const tp::Fr* a, size_t ell, size_t n, tp::Fr* pi);
 
 inline void put_g1(uint8_t*& w, const uint8_t pt[TP_G1_BYTES]) {
   tph::serialize_g1_unchecked(pt, w);

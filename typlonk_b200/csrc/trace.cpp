@@ -150,6 +150,12 @@ struct tp_trace {
     return TP_ERR_INVALID_ARG;      \
   }
 
+#define TP_TRY_OK(stmt)             \
+  do {                              \
+    int rc__ = (stmt);              \
+    if (rc__ != TP_OK) return rc__; \
+  } while (0)
+
 extern "C" {
 
 // ---- Fr conversions for host languages without a big-integer type (the C++ mirror, include/typlonk_b200.hpp) -------
@@ -223,6 +229,21 @@ int tp_trace_create(size_t n_inputs, tp_trace** out) {
   t->n_inputs = n_inputs;
   TP_TRY_ALLOC(for (size_t k = 0; k < n_inputs; k++) t->new_id(k))  // BuildVar::input, builder.rs:371-377
   *out = t;
+  return TP_OK;
+}
+
+int tp_trace_create_public(size_t n_inputs, size_t n_public, tp_trace** out) {
+  if (!out || n_public > n_inputs) return TP_ERR_INVALID_ARG;
+  TP_TRY_OK(tp_trace_create(n_inputs, out));
+  tp_trace* t = *out;
+  // public gate j = input j at (0, j); its output slot n_inputs + j exists but no variable refers to it
+  TP_TRY_ALLOC(for (size_t j = 0; j < n_public; j++) {
+    t->kind.push_back(TP_GATE_PUBLIC);
+    t->lhs.push_back(j);
+    t->rhs.push_back(j);
+    t->cc.rows++;
+    t->tag_of[j] = pack_tag(0, j);
+  })
   return TP_OK;
 }
 
@@ -311,13 +332,18 @@ int tp_trace_gate_kinds(const tp_trace* t, uint8_t* out) {
 }
 
 // Selector columns as evaluations over the domain, [q_l | q_r | q_o | q_m | q_c], each `rows` Fr in Montgomery form
-// (builder.rs:73-84 transposes Gate::to_row the same way): Mul = [0,0,1,1,0], Add = [1,1,1,0,0], Dummy = 0.
+// (builder.rs:73-84 transposes Gate::to_row the same way): Mul = [0,0,1,1,0], Add = [1,1,1,0,0], Dummy = 0,
+// Public = [1,0,0,0,0].
 int tp_trace_selectors(const tp_trace* t, uint64_t* out) {
   if (!t || !t->finished || !out) return TP_ERR_INVALID_ARG;
   const size_t n = t->rows;
   memset(out, 0, 5 * n * 32);
   const HFr one = HFr::one();
   for (size_t j = 0; j < t->kind.size(); j++) {
+    if (t->kind[j] == TP_GATE_PUBLIC) {   // q_l = 1 only: x_i + PI_i = 0
+      memcpy(out + j * 4, one.v, 32);
+      continue;
+    }
     const bool mul = t->kind[j] == TP_GATE_MUL;
     memcpy(out + (2 * n + j) * 4, one.v, 32);
     if (mul) {
@@ -359,6 +385,11 @@ int tp_trace_witness(const tp_trace* t, const uint64_t* inputs, size_t n_inputs,
   HFr* c = reinterpret_cast<HFr*>(advice[2]);
   for (size_t j = 0; j < g; j++) {
     const HFr l = val[t->lhs[j]], r = val[t->rhs[j]];
+    if (t->kind[j] == TP_GATE_PUBLIC) {   // a = x_i, b = c = 0
+      a[j] = l;
+      b[j] = c[j] = val[n_inputs + j] = HFr::zero();
+      continue;
+    }
     const HFr v = t->kind[j] == TP_GATE_MUL ? l * r : l + r;
     val[n_inputs + j] = v;
     a[j] = l;

@@ -211,4 +211,59 @@ static inline void challenges2(const std::vector<const uint8_t*>& commitments, H
   *c1 = fr_rand(rng);
 }
 
+// Proof format v2 (DESIGN.md, "Proof format v2"): H = Blake2b-512, s = H("typlonk-plonk-v2" | H(key bytes) | u64 LE l
+// | public values), absorb: s = H(s | label | data), squeeze(i) = LE-int(H(s | "challenge" | u8 i)) mod r.
+// G1 as serialize_g1_unchecked (96 B), Fr as 32 B canonical LE.
+struct TranscriptV2 {
+  uint8_t s[64];
+
+  static void put_fr(Blake2b& b, const HFr& x) {
+    HFr c = x.from_mont();
+    b.update((const uint8_t*)c.v, 32);
+  }
+  void init(const uint8_t vk_digest[64], const HFr* publics, size_t count) {
+    Blake2b b;
+    b.init();
+    b.update((const uint8_t*)"typlonk-plonk-v2", 16);
+    b.update(vk_digest, 64);
+    uint8_t l[8];
+    for (int i = 0; i < 8; i++) l[i] = (uint8_t)((uint64_t)count >> (8 * i));
+    b.update(l, 8);
+    for (size_t i = 0; i < count; i++) put_fr(b, publics[i]);
+    b.finalize(s);
+  }
+  // points: 97-byte ABI records
+  void absorb(const char* label, const std::vector<const uint8_t*>& points, const HFr* frs = nullptr, int nfr = 0) {
+    Blake2b b;
+    b.init();
+    b.update(s, 64);
+    b.update((const uint8_t*)label, strlen(label));
+    for (const uint8_t* p : points) {
+      uint8_t ser[96];
+      serialize_g1_unchecked(p, ser);
+      b.update(ser, 96);
+    }
+    for (int i = 0; i < nfr; i++) put_fr(b, frs[i]);
+    b.finalize(s);
+  }
+  HFr squeeze(uint8_t i) const {
+    Blake2b b;
+    b.init();
+    b.update(s, 64);
+    b.update((const uint8_t*)"challenge", 9);
+    b.update(&i, 1);
+    uint8_t d[64];
+    b.finalize(d);
+    // 512-bit little-endian integer mod r, Horner over 64-bit limbs from the top
+    const HFr two32 = HFr::from_u64((uint64_t)1 << 32), two64 = two32 * two32;
+    HFr acc = HFr::zero();
+    for (int k = 7; k >= 0; k--) {
+      uint64_t limb = 0;
+      for (int j = 7; j >= 0; j--) limb = (limb << 8) | d[8 * k + j];
+      acc = acc * two64 + HFr::from_u64(limb);
+    }
+    return acc;
+  }
+};
+
 }  // namespace tph

@@ -14,13 +14,15 @@ G1_BYTES = 97
 G2_BYTES = 193
 PROOF_FIXED_BYTES = 1472
 PROOF_COMPRESSED_FIXED_BYTES = 848
+PROOF_V2_FIXED_BYTES = 1056
+VK2_BYTES = 1368
 PHASES = ["msm_total", "msm_sort", "msm_accum", "msm_reduce", "ntt", "quotient", "perm", "scan"]
 
 ERRORS = {
     1: "TP_ERR_INVALID_ARG", 2: "TP_ERR_CUDA", 3: "TP_ERR_SRS_TOO_SHORT", 4: "TP_ERR_EMPTY_POLY",
     5: "TP_ERR_ZERO_DENOMINATOR", 6: "TP_ERR_GATE_UNSATISFIED", 7: "TP_ERR_NO_DEVICE",
     8: "TP_ERR_COLLECTIVE", 9: "TP_ERR_BUFFER_TOO_SMALL", 10: "TP_ERR_INVALID_TAG",
-    11: "TP_ERR_UNPLACED_VARIABLE", 12: "TP_ERR_MALFORMED",
+    11: "TP_ERR_UNPLACED_VARIABLE", 12: "TP_ERR_MALFORMED", 13: "TP_ERR_INTERNAL",
 }
 
 # every symbol include/typlonk_b200.h declares
@@ -46,6 +48,8 @@ SYMBOLS = [
     "tp_srs_contribute", "tp_srs_verify", "tp_srs_update_check",
     "tp_vk_from_circuit", "tp_vk_destroy", "tp_vk_serialized_size", "tp_vk_serialize", "tp_vk_deserialize",
     "tp_vk_verify", "tp_vk_verify_batch",
+    "tp_trace_create_public", "tp_vk2_from_circuit", "tp_vk2_destroy", "tp_vk2_serialize", "tp_vk2_deserialize",
+    "tp_vk2_last_error", "tp_prove_v2", "tp_verify_v2", "tp_proof_v2_encode", "tp_proof_v2_decode",
 ]
 
 COMM_ID_BYTES = 128
@@ -93,6 +97,7 @@ def lib():
         _lib = C.CDLL(str(_LIB_PATH))
         _lib.tp_last_error.restype = C.c_char_p
         _lib.tp_last_error.argtypes = [C.c_void_p]
+        _lib.tp_vk2_last_error.restype = C.c_char_p
         for name in SYMBOLS:
             getattr(_lib, name)  # AttributeError if the header and the library diverge
     return _lib
@@ -266,17 +271,98 @@ def proof_points_in_subgroup(fixed: bytes) -> bool:
 GATE_MUL, GATE_ADD, GATE_DUMMY = 0, 1, 2
 
 
+# ---- proof format v2 (host only) ------------------------------------------------------------------------------
+def _vk2_error() -> str:
+    return lib().tp_vk2_last_error().decode()
+
+
+def vk2_deserialize(raw: bytes, check=2):
+    """tp_vk2_deserialize -> VerifyingKeyV2Handle.  Raises Malformed naming the rejected field."""
+    h = C.c_void_p()
+    rc = lib().tp_vk2_deserialize(_buf(bytes(raw)), C.c_size_t(len(raw)), C.c_int(check), C.byref(h))
+    if rc == 12:
+        raise Malformed(rc, _vk2_error())
+    if rc != 0:
+        raise TyplonkError(rc, "tp_vk2_deserialize: " + _vk2_error())
+    return VerifyingKeyV2Handle(h)
+
+
+def proof_v2_encode(fixed: bytes, public_mont: bytes) -> bytes:
+    """tp_proof_v2_encode: the 1056-byte block | u64 LE l | l canonical Fr.  Host only."""
+    n = len(public_mont) // 32
+    need = PROOF_V2_FIXED_BYTES + 8 + 32 * n
+    out = (C.c_char * need)()
+    rc = lib().tp_proof_v2_encode(_buf(fixed), _buf(public_mont) if n else None, C.c_size_t(n), out, C.c_size_t(need), None)
+    if rc != 0:
+        raise TyplonkError(rc, "tp_proof_v2_encode")
+    return bytes(out)
+
+
+def proof_v2_decode(raw: bytes):
+    """tp_proof_v2_decode (checked) -> (fixed block, public values as Montgomery bytes).  Raises Malformed."""
+    n = C.c_size_t(0)
+    rc = lib().tp_proof_v2_decode(_buf(bytes(raw)), C.c_size_t(len(raw)), None, None, C.c_size_t(0), C.byref(n))
+    if rc == 12:
+        raise Malformed(rc, _vk2_error())
+    if rc != 0:
+        raise TyplonkError(rc, "tp_proof_v2_decode")
+    fixed = (C.c_char * PROOF_V2_FIXED_BYTES)()
+    pis = (C.c_char * (32 * n.value or 1))()
+    rc = lib().tp_proof_v2_decode(_buf(bytes(raw)), C.c_size_t(len(raw)), fixed, pis, C.c_size_t(n.value), C.byref(n))
+    if rc != 0:
+        raise TyplonkError(rc, "tp_proof_v2_decode")
+    return bytes(fixed), bytes(pis)[: 32 * n.value]
+
+
+class VerifyingKeyV2Handle:
+    """A tp_vk2: the constant-size key of proof format v2 (host memory; no context)."""
+
+    def __init__(self, h):
+        self._h = h
+
+    def serialize(self) -> bytes:
+        out = (C.c_char * VK2_BYTES)()
+        rc = lib().tp_vk2_serialize(self._h, out, C.c_size_t(VK2_BYTES))
+        if rc != 0:
+            raise TyplonkError(rc, "tp_vk2_serialize")
+        return bytes(out)
+
+    def verify(self, proof_fixed: bytes, public_mont: bytes) -> bool:
+        """tp_verify_v2 (host only)."""
+        ok = C.c_int(0)
+        rc = lib().tp_verify_v2(self._h, _buf(bytes(proof_fixed)), C.c_size_t(len(proof_fixed)),
+                                _buf(public_mont) if public_mont else None, C.c_size_t(len(public_mont) // 32),
+                                C.byref(ok))
+        if rc != 0:
+            raise TyplonkError(rc, "tp_verify_v2: public input not reduced modulo r")
+        return bool(ok.value)
+
+    def destroy(self):
+        if self._h:
+            lib().tp_vk2_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.destroy()
+        except Exception:
+            pass
+
+
 class Trace:
     """tp_trace: a circuit recorded once as a flat gate list; padding, selectors, the copy-constraint permutation
     and witnesses come from it natively (plonk/src/builder.rs:119-188, 339-397; permutation/src/lib.rs:62-93;
     plonk/src/proof.rs:33-49).  Host only."""
 
-    def __init__(self, n_inputs: int):
+    def __init__(self, n_inputs: int, n_public: int = 0):
         self._h = C.c_void_p()
         self.n_inputs = n_inputs
         self.rows = None
         self.gate_count = None
-        rc = lib().tp_trace_create(C.c_size_t(n_inputs), C.byref(self._h))
+        if n_public:   # proof format v2: the first n_public inputs in public gates
+            rc = lib().tp_trace_create_public(C.c_size_t(n_inputs), C.c_size_t(n_public), C.byref(self._h))
+        else:
+            rc = lib().tp_trace_create(C.c_size_t(n_inputs), C.byref(self._h))
         if rc != 0:
             raise TyplonkError(rc, "tp_trace_create")
 
@@ -790,6 +876,22 @@ class CircuitHandle:
         h = C.c_void_p()
         self.ctx._check(lib().tp_vk_from_circuit(self.ctx._h, self._h, C.byref(h)))
         return VerifyingKeyHandle(self.ctx, h)
+
+    def verifying_key_v2(self, n_public: int):
+        """tp_vk2_from_circuit: the v2 key with the first n_public rows public (host memory)."""
+        h = C.c_void_p()
+        self.ctx._check(lib().tp_vk2_from_circuit(self.ctx._h, self._h, C.c_size_t(n_public), C.byref(h)))
+        return VerifyingKeyV2Handle(h)
+
+    def prove_v2(self, vk, advice_mont, n_public: int):
+        """tp_prove_v2 -> (1056-byte block, public values as Montgomery bytes)."""
+        keep = [_buf(b) for b in advice_mont]
+        adv = (C.c_void_p * 3)(*[C.cast(x, C.c_void_p) for x in keep])
+        out = (C.c_char * PROOF_V2_FIXED_BYTES)()
+        pub = (C.c_char * (32 * n_public or 1))()
+        self.ctx._check(lib().tp_prove_v2(self.ctx._h, self._h, vk._h, adv, out, C.c_size_t(PROOF_V2_FIXED_BYTES),
+                                          pub if n_public else None))
+        return bytes(out), bytes(pub)[: 32 * n_public]
 
     POLY_QUOTIENT, POLY_LINEARISATION, POLY_Z_EVALS, POLY_Z, POLY_A, POLY_B, POLY_C = range(7)
 

@@ -29,7 +29,8 @@ from typing import List, Tuple
 
 from . import field as F
 from .ffi import (Context, GateUnsatisfied, TyplonkError, PROOF_FIXED_BYTES, GATE_ADD, GATE_MUL, Trace,  # noqa: F401
-                  proof_decode, proof_decode_compressed, proof_encode, proof_encode_compressed)
+                  proof_decode, proof_decode_compressed, proof_encode, proof_encode_compressed, proof_v2_decode,
+                  proof_v2_encode, vk2_deserialize)
 from .kzg import Srs
 from .permutation import Permutation
 
@@ -65,7 +66,7 @@ class TraceVar(Var):
         self.trace.assert_eq(self.id, other.id)
 
 
-KIND_NAMES = {0: "Mul", 1: "Add", 2: "Dummy"}
+KIND_NAMES = {0: "Mul", 1: "Add", 2: "Dummy", 3: "Public"}
 
 
 @dataclass
@@ -140,6 +141,19 @@ class CompiledCircuit:
         than `verify` on points outside the prime-order subgroup, which it rejects."""
         return self.handle.verify_batch([p.fixed for p in proofs], [F.fr_vec_to_bytes(p.public_inputs) for p in proofs])
 
+    def verifying_key_v2(self) -> "VerifyingKeyV2":
+        """The constant-size key of proof format v2 (tp_vk2_from_circuit), with the description's PUBLIC inputs public.
+        Host memory: it outlives the circuit and its context."""
+        if getattr(self, "_vk2", None) is None:
+            self._vk2 = VerifyingKeyV2(self.handle.verifying_key_v2(self.desc.PUBLIC))
+        return self._vk2
+
+    def prove_v2(self, inputs, blinders) -> "ProofV2":
+        """A proof in format v2 (tp_prove_v2): sound, and bound to the first PUBLIC inputs, which it carries."""
+        cols = self.witness_bytes(inputs, blinders)
+        fixed, pub = self.handle.prove_v2(self.verifying_key_v2().handle, cols, self.desc.PUBLIC)
+        return ProofV2(fixed, F.fr_vec_from_bytes(pub))
+
     def verifying_key(self) -> "VerifyingKey":
         """What `verify` reads of this circuit, without the prover's state (tp_vk_from_circuit); it stays valid after
         the circuit is destroyed."""
@@ -173,6 +187,45 @@ class VerifyingKey:
         return self.handle.verify(proof.fixed, F.fr_vec_to_bytes(proof.public_inputs))
 
 
+@dataclass
+class ProofV2:
+    """A proof in format v2: the 1056-byte block ([a] [b] [c] [z] [t0] [t1] [t2] [W_zeta] [W_zeta_omega] | six
+    evaluations) and the public values it proves."""
+    fixed: bytes
+    public_inputs: List[int]
+
+    def to_bytes(self) -> bytes:
+        """tp_proof_v2_encode: the block | Vec<Fr> of the public values."""
+        return proof_v2_encode(self.fixed, F.fr_vec_to_bytes(self.public_inputs))
+
+    @classmethod
+    def from_bytes(cls, raw: bytes) -> "ProofV2":
+        """tp_proof_v2_decode (checked); raises ffi.Malformed."""
+        fixed, pub = proof_v2_decode(raw)
+        return cls(fixed, F.fr_vec_from_bytes(pub))
+
+
+class VerifyingKeyV2:
+    """The key of proof format v2: 1368 bytes, verification on the host with no Context."""
+
+    def __init__(self, handle):
+        self.handle = handle
+
+    def to_bytes(self) -> bytes:
+        return self.handle.serialize()
+
+    @classmethod
+    def from_bytes(cls, raw: bytes, check=2) -> "VerifyingKeyV2":
+        """tp_vk2_deserialize (check 0: encoding and framing, 1: + on the curve, 2: + subgroups); raises
+        ffi.Malformed naming the rejected field."""
+        return cls(vk2_deserialize(raw, check))
+
+    def verify(self, proof: ProofV2, public_inputs=None) -> bool:
+        """tp_verify_v2 for these public values (default: the ones the proof carries)."""
+        pub = proof.public_inputs if public_inputs is None else public_inputs
+        return self.handle.verify(proof.fixed, F.fr_vec_to_bytes([v % F.R_MOD for v in pub]))
+
+
 def verify_batch(pairs: List[Tuple[VerifyingKey, Proof]]) -> Tuple[bool, List[bool]]:
     """Proofs of several circuits in one folded check (tp_vk_verify_batch): (all accepted, per-proof verdicts).  Every
     key must belong to one context; keys of different sizes and SRSes may be mixed."""
@@ -190,8 +243,9 @@ def verify_batch(pairs: List[Tuple[VerifyingKey, Proof]]) -> Tuple[bool, List[bo
 
 
 class CircuitDescription:
-    """description.rs:4-9."""
+    """description.rs:4-9.  PUBLIC (proof format v2): the first PUBLIC inputs are public."""
     INPUTS = 0
+    PUBLIC = 0
 
     @staticmethod
     def run(inputs):
@@ -200,7 +254,7 @@ class CircuitDescription:
     @classmethod
     def trace_native(cls) -> Trace:
         """The closure recorded once by the library's tracer (finished: padded, equalities resolved)."""
-        t = Trace(cls.INPUTS)
+        t = Trace(cls.INPUTS, cls.PUBLIC)
         cls.run([TraceVar(t, k) for k in range(cls.INPUTS)])
         t.finish()
         return t
